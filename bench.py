@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- SBS equirect output Mpix/s of the reprojection hot path (BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic stereo pairs.  Default workload (the
 configuration BASELINE.json's target is quoted on -- "bit-exact INTER_LINEAR SBS equirectangular output ... on
@@ -19,6 +19,11 @@ Euclidean3DRotator + PolynomialScaler chain (configs[2]), fused analytic warp, I
 N > 1: one process per GPU (torchrun or self-spawned), frames sharded statically, no data-path collective
 (weak scaling: every rank warps its own B pairs); torch.distributed is used only for the barrier and the
 max-over-ranks of the device time.
+
+--dump-outputs DIR: after the timed steps, rank 0 writes the SBS frames its last timed step produced, as a seeded
+sample of whole output rows (DIR/sbs_rows.npy, float32 (rows, 2n, 3)) and the (frame, row) of each sampled row
+(DIR/sbs_rows_index.npy, float64).  The input frames are generated from fixed seeds, so two builds run with the same
+arguments can be compared array for array.
 """
 from __future__ import annotations
 
@@ -211,6 +216,20 @@ def touched_fraction(torch, maps, n_in: int, taps: int) -> float:
     return float(touched.float().mean().item())
 
 
+DUMP_BYTES = 48 << 20  # float32 row sample written by --dump-outputs: all rows of a small step, a sample of a batch
+
+
+def dump_outputs(torch, sbs, out_dir: Path) -> None:
+    """Seeded sample of whole rows of `sbs` (frames, rows, cols, channels uint8, one step's output) -> out_dir."""
+    f, h, w, c = sbs.shape
+    n_rows = max(1, min(f * h, DUMP_BYTES // (w * c * 4)))
+    pick = np.sort(np.random.default_rng(0).choice(f * h, n_rows, replace=False))
+    rows = sbs.reshape(f * h, w, c).index_select(0, torch.from_numpy(pick).to(sbs.device))
+    out_dir.mkdir(parents=True, exist_ok=True)
+    np.save(out_dir / "sbs_rows.npy", rows.cpu().numpy().astype(np.float32))
+    np.save(out_dir / "sbs_rows_index.npy", np.stack([pick // h, pick % h], axis=1).astype(np.float64))
+
+
 # ---------------------------------------------------------------------------------------------------------
 # CPU reference path (oracle port: NumPy chain restatement + the real cv2.remap + concatenate)
 # ---------------------------------------------------------------------------------------------------------
@@ -339,7 +358,7 @@ def time_device(torch, fn, steps: int, warmup: int, dist):
 
 
 def run_workload(torch, V, wl_name: str, wl: dict, steps: int, warmup: int, dist, pairs: int | None = None,
-                 want_e2e: bool = True, device=None, check_frames=()):
+                 want_e2e: bool = True, device=None, check_frames=(), dump_dir: Path | None = None):
     n = wl["n"]
     pairs = pairs or wl["pairs"]
     ring = 1
@@ -387,6 +406,9 @@ def run_workload(torch, V, wl_name: str, wl: dict, steps: int, warmup: int, dist
             graphs[k].replay()
 
     ms = time_device(torch, step, steps, warmup, dist)
+    if dump_dir is not None:
+        k = (state["i"] - 1) % ring  # the ring slot the last timed step wrote
+        dump_outputs(torch, out[k * pairs:(k + 1) * pairs], dump_dir)
     mpix_step = pairs * n * 2 * n / 1e6
 
     # algorithmic bytes (DESIGN.md "roofline"): output written once + unique source pixels touched, per eye
@@ -583,7 +605,8 @@ def run_gpu(args) -> dict:
     n_pairs = args.pairs or wl["pairs"]
     main = run_workload(torch, V, args.workload, wl, args.steps, args.warmup, dist, pairs=args.pairs, device=device,
                         want_e2e=not args.no_e2e,
-                        check_frames=(0, n_pairs // 2 - 1, n_pairs - 1) if want_parity else ())
+                        check_frames=(0, n_pairs // 2 - 1, n_pairs - 1) if want_parity else (),
+                        dump_dir=args.dump_outputs if rank == 0 else None)
     clocks = sampler.stop() if rank == 0 else {}
     # total shards = world * pairs (weak scaling)
     value = main["value"] * world
@@ -726,7 +749,13 @@ def main() -> None:
     ap.add_argument("--no-e2e", action="store_true", help="skip the host-buffer leg (profiling runs)")
     ap.add_argument("--debug-set", default="", help="experiments: comma list of what=value for vr180_debug_set "
                                                     "(0 frames per CTA, 1 tiled flags, 2 frames-per-CTA cap)")
+    ap.add_argument("--dump-outputs", type=Path, default=None, metavar="DIR",
+                    help="write a seeded sample of the last timed step's SBS frames to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl b200)")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     # stdout carries exactly ONE line, the JSON result: whatever libraries print there while the bench runs (NCCL's

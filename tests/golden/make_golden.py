@@ -1,9 +1,9 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (/root/reference/src) in the build
-container.  Run from the repo root:   python tests/golden/make_golden.py
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference (a checkout of the original vr180-convert
+project).  Run from the repo root:   VR180_CONVERT_REF=/path/to/vr180-convert python tests/golden/make_golden.py
 
-The reference is pure Python; `quaternion` (numpy-quaternion) and `strenum` are absent from the image, so the
-test-only stand-ins in tests/refshim/ are put on sys.path first (SURVEY.md Appendix D).  /root/reference does
-not exist on the GPU box, which is why the vectors are committed.
+The reference is pure Python; its `quaternion` (numpy-quaternion) and `strenum` dependencies are served by the
+test-only stand-ins in tests/refshim/, which are put on sys.path first (SURVEY.md Appendix D).  The tests never need
+the reference itself, which is why the vectors are committed.
 
 Every case stores (a) the Python expression that builds the transformer (evaluated both against the
 reference and, in the tests, against the product package), (b) the op-tuple lowering fed to the oracle, and
@@ -12,6 +12,7 @@ reference and, in the tests, against the product package), (b) the op-tuple lowe
 from __future__ import annotations
 
 import json
+import os
 import sys
 import tempfile
 from pathlib import Path
@@ -19,8 +20,9 @@ from pathlib import Path
 import numpy as np
 
 HERE = Path(__file__).resolve().parent
+REF = Path(os.environ["VR180_CONVERT_REF"])  # checkout of the original vr180-convert project
 sys.path.insert(0, str(HERE.parent / "refshim"))
-sys.path.insert(0, "/root/reference/src")
+sys.path.insert(0, str(REF / "src"))
 
 import cv2  # noqa: E402
 import quaternion as Q  # noqa: E402  (the shim)
@@ -245,7 +247,7 @@ def make_cfg1():
     import hashlib
     import shutil
 
-    src = Path("/root/reference/docs/_static/test.jpg")
+    src = REF / "docs" / "_static" / "test.jpg"
     shutil.copyfile(src, HERE / "cfg1_test.jpg")
     (HERE / "cfg1_test.jpg").chmod(0o644)
     img = cv2.imread(str(src))
@@ -259,7 +261,7 @@ def make_cfg1():
         out = cv2.imread(str(p))
     assert out.shape == (4096, 8192, 3)
     rng = np.random.default_rng(2024)
-    idx = np.stack([rng.integers(0, 4096, 200_000), rng.integers(0, 8192, 200_000)], axis=1).astype(np.int32)
+    idx = np.stack([rng.integers(0, 4096, 200_000), rng.integers(0, 8192, 200_000)], axis=1).astype(np.int16)  # keeps the file < 1 MB
     rows = np.array([0, 1, 1023, 2047, 2048, 3000, 4094, 4095], np.int32)
     np.savez_compressed(HERE / "cfg1.npz", idx=idx, px=out[idx[:, 0], idx[:, 1]], rows=rows, row_px=out[rows],
                         meta=np.array(json.dumps({

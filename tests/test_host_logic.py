@@ -283,3 +283,22 @@ def test_host_copy_moves_every_byte_at_every_alignment():
             assert rc == 0
             assert np.array_equal(dst[do:do + n], src[so:so + n]), (n, so, do)
             assert (dst[:do] == 0xA5).all() and (dst[do + n:] == 0xA5).all(), (n, so, do)
+
+
+def test_bench_dump_outputs_is_a_seeded_row_sample(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: whole rows of one step's SBS frames as float32 with their (frame, row), within the byte
+    budget, and the same rows on every run."""
+    import torch
+
+    import bench
+
+    sbs = torch.from_numpy(np.random.default_rng(4).integers(0, 256, (5, 40, 64, 3), dtype=np.uint8))
+    monkeypatch.setattr(bench, "DUMP_BYTES", 50 * 64 * 3 * 4)
+    for d in ("a", "b"):
+        bench.dump_outputs(torch, sbs, tmp_path / d)
+    rows, index = np.load(tmp_path / "a" / "sbs_rows.npy"), np.load(tmp_path / "a" / "sbs_rows_index.npy")
+    assert rows.dtype == np.float32 and index.dtype == np.float64 and rows.shape == (50, 64, 3)
+    assert len({tuple(i) for i in index}) == 50
+    assert np.array_equal(rows, sbs.numpy()[index[:, 0].astype(int), index[:, 1].astype(int)])
+    for name in ("sbs_rows.npy", "sbs_rows_index.npy"):
+        assert np.array_equal(np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name))
