@@ -353,13 +353,10 @@ int vr180_ctx_run(vr180_ctx_t* ctx, const vr180_host_job_t* job);
 int vr180_debug_weight_table(int K, int16_t* out);
 /* what 0: frames per CTA of the tiled kernel (0 = automatic) -- lets tests drive long frame loops (stage-ring
    refills, mbarrier phase flips) with small outputs; what 1: tiled-kernel experiment flags (-1 = environment
-   variable VR180_TILED_DEBUG; bit 0: legacy row pitches, bit 1: take the tile-streaming kernel whenever the request
-   is eligible, bit 2: never, bit 3: 4 CTAs per SM for the tile-streaming kernel, bits 4-5: TMA L2 promotion none /
-   64 B / 256 B instead of 128 B -- read when a descriptor set is first encoded, bit 8: the standard chain through the
-   op-by-op interpreter of chain.cuh instead of its folded form, chain_fast.cuh); what 2: cap of the automatic
-   frames-per-CTA choice (0 = default 64); what 3: CTAs of
-   the tile-streaming kernel (0 = 3 per SM) -- lets tests push hundreds of tiles through one CTA.  Returns the
-   previous value. */
+   variable VR180_TILED_DEBUG; bit 1: take the tile-streaming kernel whenever the request is eligible, bit 2: never,
+   bit 8: the standard chain through the op-by-op interpreter of chain.cuh instead of its folded form, chain_fast.cuh);
+   what 2: cap of the automatic frames-per-CTA choice (0 = default 64); what 3: CTAs of the tile-streaming kernel
+   (0 = 3 per SM) -- lets tests push hundreds of tiles through one CTA.  Returns the previous value. */
 int vr180_debug_set(int what, int value);
 /* The byte mover of the pipeline's copy threads (packs pageable frames into the page-locked ring: streaming stores for
    copies of 8 KB and more on CPUs with AVX2, memcpy otherwise; VR180_NT_COPY=0 forces memcpy) applied to caller buffers. */

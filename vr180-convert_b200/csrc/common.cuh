@@ -16,7 +16,7 @@ extern std::atomic<uint64_t> g_launches;
 extern std::atomic<int> g_debug_frames_per_cta;  // frames per CTA of the tiled kernel (tests force long frame loops on small outputs)
 extern std::atomic<int> g_debug_tiled_flags;     // -1 = take VR180_TILED_DEBUG from the environment
 extern std::atomic<int> g_debug_max_frames_per_cta;  // cap of the automatic choice (0 = default)
-extern std::atomic<int> g_debug_stream_grid;  // CTAs of the streaming kernel (0 = 4 per SM): tests force many tiles per CTA
+extern std::atomic<int> g_debug_stream_grid;  // CTAs of the streaming kernel (0 = 3 per SM): tests force many tiles per CTA
 void set_cuda_error(cudaError_t e, const char* where);
 
 #define VR180_CUDA(call)                                  \

@@ -31,14 +31,14 @@ namespace tiled {
 
 constexpr int kSlots = 3;       // stage ring: slots of Lay<M>::kStageArea / 3 bytes (13.5 KB; a bilinear 8K tile needs <= 10.5 KB)
 constexpr int kSlowCap = 128;   // non-staged tiles a CTA notes before it stops streaming to gather them
-constexpr int kStreamCtas = 3;  // CTAs per SM: 72 registers (4 CTAs / 56 registers spill and measure 1-2 % slower: VR180_TILED_DEBUG bit 3)
+constexpr int kStreamCtas = 3;  // CTAs per SM: 72 registers (4 CTAs / 56 registers spill and measure 1-2 % slower)
 
-template <class M, int CTAS = kStreamCtas>
+template <class M>
 struct SLay {
     static constexpr int kSlotBytes = kStreamSlotBytes<M>;
     static_assert(kSlots == 3, "kStreamSlotBytes (tiled.cuh) is a third of the staging area");
     static constexpr int kOutTileBytes = M::kTileH * kTileW * 3;
-    static constexpr int kOB = CTAS >= 4 ? 2 : kOutBufs;  // out buffers of one item each: the tile of one eye or of both
+    static constexpr int kOB = kOutBufs;  // out buffers of one item each: the tile of one eye or of both
     static constexpr int kOutItemBytes = 2 * kOutTileBytes;
     static constexpr int kOffOut = kSlots * kSlotBytes;
     static constexpr int kOffBar = kOffOut + kOB * kOutItemBytes;  // full[kSlots], ofull[kOB], oempty[kOB]
@@ -60,9 +60,6 @@ struct StreamParams {
 
 // Source rectangle of a packed tile from its header alone (both the producer and the sampling warps evaluate it): the
 // box sizes were chosen by k_pack_tiles, only the origin and the border test are left.
-__device__ __forceinline__ int4 raw_header(const void* packed, int tile) {
-    return __ldg(reinterpret_cast<const int4*>(packed) + tile);
-}
 struct UnitGeom {
     int fast, bx0, ry0, pitch, rsel, rect_bytes, org;
     int eye_pitch;  // distance of the two eyes' rectangles inside a slot (TMA destinations are 128-byte aligned)
@@ -70,11 +67,11 @@ struct UnitGeom {
 template <class M>
 __device__ __forceinline__ UnitGeom unit_geom(const int4& raw, int zero_border, int src_cols, int src_rows) {
     UnitGeom g;
-    struct { int mnx, mxx, mny, mxy, flags; } h = {(short)(raw.x & 0xffff), raw.x >> 16, (short)(raw.y & 0xffff), raw.y >> 16, raw.z};
-    const int c0 = 3 * ((int)h.mnx - M::kLo);  // byte column of the tile's first tap column
-    g.bx0 = c0 & ~15;
-    g.org = c0 & 15;
-    g.ry0 = (int)h.mny - M::kLo;
+    const TileHdr h = decode_header(raw);
+    const TileRect rc = tile_rect<M>(h.mnx, h.mxx, h.mny, h.mxy);
+    g.bx0 = rc.bx0;
+    g.org = 3 * (h.mnx - M::kLo) - rc.bx0;  // byte offset of the tile's first tap column in the box
+    g.ry0 = rc.ry0;
     g.pitch = kPitchMin + kPitchStep * ((h.flags >> 8) & 15);
     g.rsel = (h.flags >> 12) & 15;
     g.rect_bytes = (M::kRowsMin + g.rsel * kRowsStep) * g.pitch;
@@ -106,56 +103,36 @@ __device__ __forceinline__ void gather_tile(const RemapArgs& a, const StreamPara
     for (int k = 0; k < kPx; ++k) {
         const int i = x0 + lane, j = y0 + kPx * sw + k;
         if (i >= a.W || j >= a.H) continue;
-        int qx, qy;
+        int2 q;
         if (packed) {
-            qx = ((mnx + (int)(ev.e[k] & 255u)) << M::kShift) | (int)((ev.e[k] >> 16) & 31u);
-            qy = ((mny + (int)((ev.e[k] >> 8) & 255u)) << M::kShift) | (int)((ev.e[k] >> 21) & 31u);
+            q = unpack_entry<M>(mnx, mny, ev.e[k]);
         } else {
-            qx = M::quant(__ldg(mv.xmap + (long long)j * mv.map_pitch + i));
-            qy = M::quant(__ldg(mv.ymap + (long long)j * mv.map_pitch + i));
+            q.x = M::quant(__ldg(mv.xmap + (long long)j * mv.map_pitch + i));
+            q.y = M::quant(__ldg(mv.ymap + (long long)j * mv.map_pitch + i));
         }
-        for (int f = 0; f < a.n_frames; ++f) {
-            uint8_t* drow = a.dst + (long long)f * a.dst_frame_stride + (long long)j * a.dst_pitch;
-            for (int v = grp; v < grp + nv; ++v) {
-                const ViewArgs& vw = a.view[v];
-                Src s{vw.src + (long long)f * vw.frame_stride, vw.rows, vw.cols, vw.pitch};
-                int px[3];
-                if (M::kInterp == VR180_INTER_NEAREST)
-                    fetch_tap<3>(s, sat16(qx), sat16(qy), a.border_mode, a.bv, px);
-                else if (M::kInterp == VR180_INTER_LINEAR)
-                    sample_linear<3>(s, qx, qy, a.border_mode, a.bv, px);
-                else if (M::kInterp == VR180_INTER_CUBIC)
-                    sample_tab<3, 4>(s, qx, qy, sp.tab, a.border_mode, a.bv, px);
-                else
-                    sample_tab<3, 8>(s, qx, qy, sp.tab, a.border_mode, a.bv, px);
-                uint8_t* o = drow + (long long)(vw.dst_x_offset + i) * 3;
-                o[0] = (uint8_t)px[0];
-                o[1] = (uint8_t)px[1];
-                o[2] = (uint8_t)px[2];
-            }
-        }
+        for (int f = 0; f < a.n_frames; ++f) gather_pixel<M>(a, f, i, j, grp, grp + nv, q.x, q.y, sp.tab);
     }
 }
 
-template <class M, int CTAS>
-__global__ void __launch_bounds__(kThreads, CTAS)
+template <class M>
+__global__ void __launch_bounds__(kThreads, kStreamCtas)
 k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ StreamParams sp,
               const __grid_constant__ TmaMaps tm) {
     constexpr int kPx = M::kPx;
-    constexpr int kOB = SLay<M, CTAS>::kOB, kOutTileBytes = SLay<M, CTAS>::kOutTileBytes, kSlotBytes = SLay<M, CTAS>::kSlotBytes;
-    constexpr int kOutItemBytes = SLay<M, CTAS>::kOutItemBytes;
+    constexpr int kOB = SLay<M>::kOB, kOutTileBytes = SLay<M>::kOutTileBytes, kSlotBytes = SLay<M>::kSlotBytes;
+    constexpr int kOutItemBytes = SLay<M>::kOutItemBytes;
     extern __shared__ __align__(1024) uint8_t smem[];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint32_t s_stage = smem_u32(smem), s_full = s_stage + SLay<M, CTAS>::kOffBar;
-    const uint32_t s_ofull = s_full + kSlots * 8, s_oempty = s_ofull + kOB * 8, s_out = s_stage + SLay<M, CTAS>::kOffOut;
-    int4* const s_q = reinterpret_cast<int4*>(smem + SLay<M, CTAS>::kOffQ);
+    const uint32_t s_stage = smem_u32(smem), s_full = s_stage + SLay<M>::kOffBar;
+    const uint32_t s_ofull = s_full + kSlots * 8, s_oempty = s_ofull + kOB * 8, s_out = s_stage + SLay<M>::kOffOut;
+    int4* const s_q = reinterpret_cast<int4*>(smem + SLay<M>::kOffQ);
     if (tid < kSlots + 2 * kOB) {
         const bool by_warps = tid >= kSlots && tid < kSlots + kOB;  // ofull: one arrive per sampling warp
         mbar_init(s_full + tid * 8, by_warps ? kSamplers / 32 : 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if constexpr (SLay<M, CTAS>::kWeightTab != 0) {
-        uint2* const wt = reinterpret_cast<uint2*>(smem + SLay<M, CTAS>::kOffTab);
+    if constexpr (SLay<M>::kWeightTab != 0) {
+        uint2* const wt = reinterpret_cast<uint2*>(smem + SLay<M>::kOffTab);
         for (int i = tid; i < 1024; i += kThreads) {
             typename M::Pixel p;
             M::weights(p, i & 31, i >> 5, nullptr);
@@ -184,13 +161,13 @@ k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ Strea
         };
         int grp_n = 0, tile_n = blockIdx.x;  // unit = (map group, tile); blockIdx.x < n_units
         while (tile_n >= sp.n_tiles) { tile_n -= sp.n_tiles; ++grp_n; }
-        int4 hn = raw_header(a.view[grp_n].packed, tile_n);  // kept as loaded: three registers
+        int4 hn = packed_header_raw(a.view[grp_n].packed, tile_n);  // kept as loaded: three registers
         for (int u = blockIdx.x; u < sp.n_units; u += stride) {
             const int4 hdr = hn;
             const int grp = grp_n, tile = tile_n;
             tile_n += stride;
             while (tile_n >= sp.n_tiles) { tile_n -= sp.n_tiles; ++grp_n; }
-            if (u + stride < sp.n_units) hn = raw_header(a.view[grp_n].packed, tile_n);
+            if (u + stride < sp.n_units) hn = packed_header_raw(a.view[grp_n].packed, tile_n);
             const UnitGeom g = unit_geom<M>(hdr, sp.zero_border, src_cols, src_rows);
             if (!g.fast) continue;
             const int ty = tile / sp.tiles_x, tx = tile - ty * sp.tiles_x;
@@ -228,23 +205,10 @@ k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ Strea
     uint32_t flags = (sub != 3 ? 1u : 0u) | (lane == 0 ? 2u : 0u);
     asm volatile("" : "+r"(outp), "+r"(flags));
 
-    auto load_entries = [&](int grp, int tile, uint32_t (&e)[kPx]) {
-        const uint32_t* ent = packed_entries(a.view[grp].packed, sp.n_tiles) + ((size_t)tile * kSamplers + tid) * kPx;
-        if constexpr (kPx == 4) {
-            const uint4 v = __ldg(reinterpret_cast<const uint4*>(ent));
-            e[0] = v.x; e[1] = v.y; e[2] = v.z; e[3] = v.w;
-        } else if constexpr (kPx == 2) {
-            const uint2 v = __ldg(reinterpret_cast<const uint2*>(ent));
-            e[0] = v.x; e[1] = v.y;
-        } else {
-            e[0] = __ldg(ent);
-        }
-    };
-
     // Tiles that are not staged are only noted (s_slow) while the CTA streams; they are gathered per pixel afterwards,
     // outside the streaming loop, whose registers the gather code would otherwise claim (the prefetched header and entries
     // ended up in local memory).  A full list ends the streaming phase early; the outer loop resumes it after the drain.
-    int2* const s_slow = reinterpret_cast<int2*>(smem + SLay<M, CTAS>::kOffSlow);
+    int2* const s_slow = reinterpret_cast<int2*>(smem + SLay<M>::kOffSlow);
     int n = 0, st = 0;
     uint32_t ph = 0;
     int grp_n = 0, tile_n = blockIdx.x;  // unit = (map group, tile); blockIdx.x < n_units
@@ -252,9 +216,9 @@ k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ Strea
     int u = blockIdx.x;
   for (;;) {
     int n_slow = 0;
-    int4 hn = raw_header(a.view[grp_n].packed, tile_n);  // kept as loaded: three registers
+    int4 hn = packed_header_raw(a.view[grp_n].packed, tile_n);  // kept as loaded: three registers
     uint32_t en[kPx];
-    load_entries(grp_n, tile_n, en);
+    load_packed_entries<M>(a.view[grp_n].packed, sp.n_tiles, tile_n, tid, en);
     for (; u < sp.n_units && n_slow < kSlowCap; u += stride) {
         const int4 hdr = hn;
         uint32_t e[kPx];
@@ -264,8 +228,8 @@ k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ Strea
         tile_n += stride;
         while (tile_n >= sp.n_tiles) { tile_n -= sp.n_tiles; ++grp_n; }
         if (u + stride < sp.n_units) {  // the next tile's header and entries travel while this one is sampled
-            hn = raw_header(a.view[grp_n].packed, tile_n);
-            load_entries(grp_n, tile_n, en);
+            hn = packed_header_raw(a.view[grp_n].packed, tile_n);
+            load_packed_entries<M>(a.view[grp_n].packed, sp.n_tiles, tile_n, tid, en);
         }
         const UnitGeom g = unit_geom<M>(hdr, sp.zero_border, src_cols, src_rows);
 
@@ -281,16 +245,16 @@ k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ Strea
         for (int k = 0; k < kPx; ++k) {
             const int dx = (int)(e[k] & 255u), dy = (int)((e[k] >> 8) & 255u);  // iy - kLo - ry0 == dy
             M::set_offset(pc[k], dy * g.pitch + 3 * dx + g.org, true);
-            if constexpr (SLay<M, CTAS>::kWeightTab != 0) {
+            if constexpr (SLay<M>::kWeightTab != 0) {
                 asm("ld.shared.v2.u32 {%0, %1}, [%2];"
                     : "=r"(pc[k].W01), "=r"(pc[k].W23)
-                    : "r"(s_stage + SLay<M, CTAS>::kOffTab + ((e[k] >> 13) & (1023u << 3))));
+                    : "r"(s_stage + SLay<M>::kOffTab + ((e[k] >> 13) & (1023u << 3))));
             } else {
                 M::weights(pc[k], (int)((e[k] >> 16) & 31u), (int)((e[k] >> 21) & 31u), sp.tab);
             }
         }
         if constexpr (M::kWeightSmem != 0) {  // Lanczos4: the pixel's 64 weights, private copy in shared memory
-            uint8_t* slot = smem + SLay<M, CTAS>::kOffW + tid * 16;
+            uint8_t* slot = smem + SLay<M>::kOffW + tid * 16;
 #pragma unroll
             for (int ky = 0; ky < 8; ++ky)
                 *reinterpret_cast<uint4*>(slot + ky * (kSamplers * 16)) = __ldg(reinterpret_cast<const uint4*>(pc[0].w) + ky);
@@ -340,29 +304,26 @@ k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ Strea
     asm volatile("bar.sync 1, %0;" ::"n"(kSamplers) : "memory");
     for (int i = 0; i < n_slow; ++i) {
         const int2 gt = s_slow[i];
-        const int4 hdr = raw_header(a.view[gt.x].packed, gt.y);
+        const int4 hdr = packed_header_raw(a.view[gt.x].packed, gt.y);
         Entries<kPx> ev;
-        load_entries(gt.x, gt.y, ev.e);
-        gather_tile<M>(a, sp, gt.x, gt.y, nv, (hdr.z & kHdrPackable) != 0, (short)(hdr.x & 0xffff), (short)(hdr.y & 0xffff), ev);
+        load_packed_entries<M>(a.view[gt.x].packed, sp.n_tiles, gt.y, tid, ev.e);
+        const TileHdr h = decode_header(hdr);
+        gather_tile<M>(a, sp, gt.x, gt.y, nv, (h.flags & kHdrPackable) != 0, h.mnx, h.mny, ev);
     }
     if (u >= sp.n_units) break;
     asm volatile("bar.sync 1, %0;" ::"n"(kSamplers) : "memory");  // the list is rewritten by the next streaming phase
   }
 }
 
-template <class M, int CTAS>
+template <class M>
 static int launch_stream_mode(const RemapArgs& a, const short* tab, cudaStream_t st) {
     const int n_groups = a.share_map ? 1 : a.n_views;
     if (a.n_frames > 0x7fff) return VR180_ERR_UNSUPPORTED;  // an item's two frame indices travel in one int
     const TmaMaps* tm = tma_maps_for(a, M::kInterp, M::kRowsMin, M::kTileH, 1);
     if (!tm) return VR180_ERR_UNSUPPORTED;
-    static std::atomic<int> attr_done[64];
     int dev = 0;
-    VR180_CUDA(cudaGetDevice(&dev));
-    if (dev < 64 && !attr_done[dev].load(std::memory_order_acquire)) {
-        VR180_CUDA(cudaFuncSetAttribute(k_warp_stream<M, CTAS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SLay<M, CTAS>::kSmemBytes));
-        attr_done[dev].store(1, std::memory_order_release);
-    }
+    const int rc = max_dyn_smem_once<k_warp_stream<M>>(SLay<M>::kSmemBytes, dev);
+    if (rc != VR180_OK) return rc;
     static std::atomic<int> sm_count[64];
     int sms = dev < 64 ? sm_count[dev].load(std::memory_order_acquire) : 0;
     if (!sms) {
@@ -376,12 +337,12 @@ static int launch_stream_mode(const RemapArgs& a, const short* tab, cudaStream_t
     if (tiles * n_groups > 0x7fffffffLL) return VR180_ERR_UNSUPPORTED;
     sp.n_tiles = (int)tiles;
     sp.n_units = (int)(tiles * n_groups);
-    sp.zero_border = (a.border_mode == VR180_BORDER_CONSTANT && !(a.bv[0] | a.bv[1] | a.bv[2])) ? 1 : 0;
+    sp.zero_border = zero_border(a);
     sp.tab = tab;
     const int forced = g_debug_stream_grid.load(std::memory_order_relaxed);  // vr180_debug_set(3, n): tests
-    int grid = forced > 0 ? forced : sms * CTAS;
+    int grid = forced > 0 ? forced : sms * kStreamCtas;
     if (grid > sp.n_units) grid = sp.n_units;
-    k_warp_stream<M, CTAS><<<grid, kThreads, SLay<M, CTAS>::kSmemBytes, st>>>(a, sp, *tm);
+    k_warp_stream<M><<<grid, kThreads, SLay<M>::kSmemBytes, st>>>(a, sp, *tm);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     VR180_CUDA(cudaGetLastError());
     return VR180_OK;
@@ -393,12 +354,10 @@ static int launch_stream_mode(const RemapArgs& a, const short* tab, cudaStream_t
 // of this interpolation, no per-frame radius).
 int launch_remap_stream(const RemapArgs& a, int interp, const short* weight_tab, cudaStream_t st) {
     using namespace tiled;
-    if (interp == VR180_INTER_NEAREST) return launch_stream_mode<Nearest, kStreamCtas>(a, nullptr, st);
-    if (interp == VR180_INTER_LINEAR)
-        return (tiled_debug_flags() & 8) ? launch_stream_mode<LinearP, 4>(a, nullptr, st)
-                                         : launch_stream_mode<LinearP, kStreamCtas>(a, nullptr, st);
-    if (interp == VR180_INTER_CUBIC) return launch_stream_mode<Cubic, kStreamCtas>(a, weight_tab, st);
-    if (interp == VR180_INTER_LANCZOS4) return launch_stream_mode<Lanczos4, kStreamCtas>(a, weight_tab, st);
+    if (interp == VR180_INTER_NEAREST) return launch_stream_mode<Nearest>(a, nullptr, st);
+    if (interp == VR180_INTER_LINEAR) return launch_stream_mode<LinearP>(a, nullptr, st);
+    if (interp == VR180_INTER_CUBIC) return launch_stream_mode<Cubic>(a, weight_tab, st);
+    if (interp == VR180_INTER_LANCZOS4) return launch_stream_mode<Lanczos4>(a, weight_tab, st);
     return VR180_ERR_UNSUPPORTED;
 }
 

@@ -49,7 +49,7 @@ namespace vr180 {
 namespace tiled {
 
 struct TileGeom {
-    int nrows;          // source rows of the tile's rectangle
+    int rsel;           // TMA box rows of the tile's rectangle: M::kRowsMin + kRowsStep * rsel
     int bx0, ry0;       // first source byte column (16-aligned, may be negative) and first source row
     int x0, y0;         // output tile origin
 };
@@ -100,8 +100,7 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
     // host keeps chunks even, so it lies past the end of the batch, where TMA loads zeros and drops the store
     static_assert(!VPAIR || (SPLIT && FR == 2 && NV == 2 && !DYN), "an eye pair is two one-frame boxes of two views");
     const int n_items = VPAIR ? (f1 - f0) : ((f1 - f0 + FR - 1) / FR) * NV;
-    const int rsel = tg.nrows <= M::kRowsMin ? 0 : (tg.nrows - M::kRowsMin + kRowsStep - 1) / kRowsStep;
-    const int rect_bytes = (M::kRowsMin + rsel * kRowsStep) * pitch;  // one frame's box; multiple of 64
+    const int rect_bytes = (M::kRowsMin + tg.rsel * kRowsStep) * pitch;  // one frame's box; multiple of 64
     const int stage_bytes = FR * rect_bytes;                          // bytes the box load(s) of an item deliver
     // distance of an item's frames inside a stage: packed by a box FR frames deep; one-frame boxes land 128-byte aligned
     const int frame_pitch = SPLIT ? (rect_bytes + 127) & ~127 : rect_bytes;
@@ -113,7 +112,7 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
 
     if (warp == kSamplers / 32) {  // ---- producer ----
         if (lane != 0) return;
-        const CUtensorMap* const map0 = &tm.src[v_begin][(pitch - kPitchMin) / kPitchStep][rsel];
+        const CUtensorMap* const map0 = &tm.src[v_begin][(pitch - kPitchMin) / kPitchStep][tg.rsel];
         const int dst_x0 = (a.view[v_begin].dst_x_offset + tg.x0) * 3;
         const int dst_x1 = (a.view[v_begin + NV - 1].dst_x_offset + tg.x0) * 3;
         int p_item = 0, p_stage = 0;  // next item to fetch and its stage
@@ -125,11 +124,12 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
             if (DYN) {  // this frame's rectangle; its origin travels to the samplers next to the stage
                 const double rad = __ldg(dr.radius + f);
                 if (rad == rad) {
-                    int lo, hi;
-                    dyn_range<M>(dr.ext[0], dr.ext[1], rad, dr.cx, lo, hi);
-                    bx0 = (3 * (lo - M::kLo)) & ~15;
-                    dyn_range<M>(dr.ext[2], dr.ext[3], rad, dr.cy, lo, hi);
-                    ry0 = lo - M::kLo;
+                    int xlo, xhi, ylo, yhi;
+                    dyn_range<M>(dr.ext[0], dr.ext[1], rad, dr.cx, xlo, xhi);
+                    dyn_range<M>(dr.ext[2], dr.ext[3], rad, dr.cy, ylo, yhi);
+                    const TileRect rc = tile_rect<M>(xlo, xhi, ylo, yhi);
+                    bx0 = rc.bx0;
+                    ry0 = rc.ry0;
                 } else {  // get_radius found no transition: every coordinate is NaN -> border colour
                     bx0 = ry0 = -(1 << 20);
                 }
@@ -226,7 +226,6 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
             }
         }
         uint32_t word[FR][M::kPx];
-#pragma unroll
         if (!DYN && M::kInterp == VR180_INTER_LANCZOS4) {  // a tap row's weights serve every frame of the item
 #pragma unroll
             for (int k = 0; k < M::kPx; ++k) {
@@ -263,15 +262,10 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
     }
 }
 
-// CTAs per SM the kernel is compiled for: 4 (56 registers) unless the mode asks for fewer, larger CTAs
-template <class M, class = void>
-struct MinCtas { static constexpr int value = 4; };
-template <class M>
-struct MinCtas<M, std::void_t<decltype(M::kMinCtas)>> { static constexpr int value = M::kMinCtas; };
-
-// DYN: per-frame radius from device memory (vr180_mapsrc_t::radius_dev); FR: frames per pipeline item
+// DYN: per-frame radius from device memory (vr180_mapsrc_t::radius_dev); FR: frames per pipeline item.  4 CTAs per SM
+// (56 registers).
 template <class M, bool DYN, int FR>
-__global__ void __launch_bounds__(kThreads, MinCtas<M>::value)
+__global__ void __launch_bounds__(kThreads, 4)
 k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_chain_t chain0,
              const __grid_constant__ vr180_chain_t chain1, const __grid_constant__ TiledParams tp,
              const __grid_constant__ TmaMaps tm) {
@@ -280,7 +274,7 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
     constexpr int kWarpsPerBand = 4 / kPx;  // a band = 4 output rows x 32 columns = 4 / kPx warps of 8 kPx columns
     extern __shared__ __align__(1024) uint8_t smem[];
     double* s_trig = reinterpret_cast<double*>(smem + Lay<M>::kOffTrig);  // [4][32]
-    int* s_red = reinterpret_cast<int*>(smem + Lay<M>::kOffRed);          // [8][4]
+    int4* s_red = reinterpret_cast<int4*>(smem + Lay<M>::kOffRed);        // [8]: box of each sampling warp
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     if (tid < 2 * kMaxStages + 2 * kOutBufs) {  // one barrier per thread: a single-frame launch is latency bound, and one
@@ -312,10 +306,8 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
     const bool full_tile = (x0 + kTileW <= a.W) && (y0 + M::kTileH <= a.H);
 
     // tile-packed LUT: the tile's header (every thread: the producer warp needs the rectangle too)
-    PackedHdr hdr;
-    hdr.mnx = hdr.mxx = hdr.mny = hdr.mxy = 0;
-    hdr.flags = hdr.pad = 0;
-    if (mv.map_kind != VR180_MAPSRC_ANALYTIC && mv.packed) hdr = packed_header(mv.packed, tile);
+    TileHdr hdr = {0, 0, 0, 0, 0};
+    if (mv.map_kind != VR180_MAPSRC_ANALYTIC && mv.packed) hdr = decode_header(packed_header_raw(mv.packed, tile));
     const bool packed_tile = (hdr.flags & 1) != 0;  // CTA-uniform: coordinates and bounding box come from the packed LUT
 
     // ---- coordinates of this thread's pixels --------------------------------------------------------------
@@ -431,26 +423,17 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
             }
         }
     } else if (sampler) {
-        // Tile-packed LUT (vr180_pack_lut_tiles): 16-byte tile header + one uint32 per pixel in thread order, i.e. ONE
-        // 128-bit (bilinear / nearest), 64-bit (bicubic) or 32-bit (Lanczos4) coalesced load per thread.
+        // Tile-packed LUT (vr180_pack_lut_tiles): 16-byte tile header + one uint32 per pixel in thread order
         bool unpacked = false;
         {
             if (packed_tile) {
-                const uint32_t* ent = packed_entries(mv.packed, tp.n_tiles) + ((size_t)tile * kSamplers + tid) * kPx;
                 uint32_t e[kPx];
-                if constexpr (kPx == 4) {
-                    const uint4 v = __ldg(reinterpret_cast<const uint4*>(ent));
-                    e[0] = v.x; e[1] = v.y; e[2] = v.z; e[3] = v.w;
-                } else if constexpr (kPx == 2) {
-                    const uint2 v = __ldg(reinterpret_cast<const uint2*>(ent));
-                    e[0] = v.x; e[1] = v.y;
-                } else {
-                    e[0] = __ldg(ent);
-                }
+                load_packed_entries<M>(mv.packed, tp.n_tiles, tile, tid, e);
 #pragma unroll
                 for (int k = 0; k < kPx; ++k) {
-                    sx[k] = ((hdr.mnx + (int)(e[k] & 255u)) << M::kShift) | (int)((e[k] >> 16) & 31u);
-                    sy[k] = ((hdr.mny + (int)((e[k] >> 8) & 255u)) << M::kShift) | (int)((e[k] >> 21) & 31u);
+                    const int2 q = unpack_entry<M>(hdr.mnx, hdr.mny, e[k]);
+                    sx[k] = q.x;
+                    sy[k] = q.y;
                 }
                 unpacked = true;
             }
@@ -495,27 +478,8 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
     }
 
     // ---- source rectangle of the tile ---------------------------------------------------------------------
-    int mnx = INT_MAX, mxx = INT_MIN, mny = INT_MAX, mxy = INT_MIN;
-    if (!packed_tile) {  // a packed tile carries its bounding box in the header: no reduction
-#pragma unroll
-        for (int k = 0; k < kPx; ++k) {
-            const int ix = sat16(sx[k] >> M::kShift), iy = sat16(sy[k] >> M::kShift);
-            mnx = min(mnx, ix);
-            mxx = max(mxx, ix);
-            mny = min(mny, iy);
-            mxy = max(mxy, iy);
-        }
-        mnx = __reduce_min_sync(0xffffffffu, mnx);
-        mxx = __reduce_max_sync(0xffffffffu, mxx);
-        mny = __reduce_min_sync(0xffffffffu, mny);
-        mxy = __reduce_max_sync(0xffffffffu, mxy);
-        if (lane == 0 && sampler) {
-            s_red[warp * 4 + 0] = mnx;
-            s_red[warp * 4 + 1] = mxx;
-            s_red[warp * 4 + 2] = mny;
-            s_red[warp * 4 + 3] = mxy;
-        }
-    }
+    // a packed tile carries its bounding box in the header: no reduction
+    if (!packed_tile) block_box_store<M>(sx, sy, s_red, warp, lane == 0 && sampler);
     DynRadius dr;
     dr.radius = nullptr;
     dr.cx = dr.cy = 0.0;
@@ -549,38 +513,19 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
         }
     }
     nan_px = __syncthreads_or(nan_px);
-    if (packed_tile) {
-        mnx = hdr.mnx;
-        mxx = hdr.mxx;
-        mny = hdr.mny;
-        mxy = hdr.mxy;
-    } else {
-        // lane w holds the box of sampling warp w: one 128-bit load + four warp reductions (a loop over the 8 records
-        // is 64 instructions per thread, and a one-frame tile has few to amortise them over)
-        static_assert(Lay<M>::kOffRed % 16 == 0, "s_red is read as int4");
-        int4 r = make_int4(INT_MAX, INT_MIN, INT_MAX, INT_MIN);
-        if (lane < kSamplers / 32) r = reinterpret_cast<const int4*>(s_red)[lane];
-        mnx = __reduce_min_sync(0xffffffffu, r.x);
-        mxx = __reduce_max_sync(0xffffffffu, r.y);
-        mny = __reduce_min_sync(0xffffffffu, r.z);
-        mxy = __reduce_max_sync(0xffffffffu, r.w);
-    }
-    // taps cover columns ix - kLo .. ix + kHi and rows iy - kLo .. iy + kHi
-    const int bx0 = (3 * (mnx - M::kLo)) & ~15, bx1 = (3 * (mxx + M::kHi + 1) + 15) & ~15;  // 16-byte granules
-    const int ry0 = mny - M::kLo;
-    const int wbytes = bx1 - bx0, nrows = mxy + M::kHi + 1 - ry0;
+    static_assert(Lay<M>::kOffRed % 16 == 0, "s_red is read as int4");
+    const int4 box = packed_tile ? make_int4(hdr.mnx, hdr.mxx, hdr.mny, hdr.mxy) : block_box_load(s_red, lane);
+    const int mnx = box.x, mxx = box.y, mny = box.z, mxy = box.w;
+    const TileRect rc = tile_rect<M>(mnx, mxx, mny, mxy);
     // Taps outside the source read TMA's zero fill = BORDER_CONSTANT(0); only unbounded footprints (NaN / huge
     // coordinates saturate to +-32768) and partial edge tiles leave the fast path.
     // ... and tiles whose item (FR frames x box rows x pitch) does not fit the staging area
-    auto box_rows_of = [](int rows) {
-        return M::kRowsMin + (rows <= M::kRowsMin ? 0 : (rows - M::kRowsMin + kRowsStep - 1) / kRowsStep) * kRowsStep;
-    };
     // (a chunk with varying radii runs one-frame items; FR-frame items of a DYN launch are FR one-frame boxes, each 128-byte aligned)
     // (a launch that gives its CTAs single frames pairs the two eyes of a shared map in one item: see VPAIR)
     const bool vpair = !DYN && FR == 1 && nv == 2;
     const int fr_item = dynr ? 1 : (vpair ? 2 : FR);
-    auto stage_fits = [&](int rows, int pitch_bytes) {
-        const int rect = box_rows_of(rows) * pitch_bytes;
+    auto stage_fits = [&](int box_rows, int pitch_bytes) {
+        const int rect = box_rows * pitch_bytes;
         return ((fr_item * ((DYN || vpair) ? (rect + 127) & ~127 : rect) + 127) & ~127) <= Lay<M>::kStageArea;
     };
     // Any other border (a colour, REPLICATE, REFLECT, WRAP, REFLECT_101) needs real taps or the border colour where the
@@ -589,10 +534,10 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
     auto inside_src = [&](int x_lo, int x_hi, int y_lo, int y_hi) {  // extreme integer coordinates of the tile
         return x_lo - M::kLo >= 0 && x_hi + M::kHi <= src_cols - 1 && y_lo - M::kLo >= 0 && y_hi + M::kHi <= src_rows - 1;
     };
-    bool fast = full_tile && wbytes <= kPitchMax && nrows <= M::kRowsMin + (kRowSizes - 1) * kRowsStep &&
-                mnx > -32768 && mny > -32768 && mxx < 32767 && mxy < 32767 && stage_fits(nrows, max(wbytes, kPitchMin)) &&
+    bool fast = full_tile && rc.wbytes <= kPitchMax && rc.rsel < kRowSizes && mnx > -32768 && mny > -32768 &&
+                mxx < 32767 && mxy < 32767 && stage_fits(rc.box_rows, max(rc.wbytes, kPitchMin)) &&
                 (tp.zero_border || inside_src(mnx, mxx, mny, mxy));
-    int dyn_wbytes = 0, dyn_nrows = 0;
+    int dyn_wbytes = 0, dyn_nrows = 0;  // the largest rectangle over the frames of the chunk
     if (dynr) {
         const double* s_ext = reinterpret_cast<const double*>(smem + Lay<M>::kOffExt);
         dr.ext[0] = dr.ext[2] = CUDART_INF;
@@ -616,10 +561,11 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
                 int lo, hi, ylo, yhi;
                 dyn_range<M>(dr.ext[0], dr.ext[1], rad, dr.cx, lo, hi);
                 ok &= (lo > -32768) & (hi < 32767);
-                dyn_wbytes = max(dyn_wbytes, ((3 * (hi + M::kHi + 1) + 15) & ~15) - ((3 * (lo - M::kLo)) & ~15));
                 dyn_range<M>(dr.ext[2], dr.ext[3], rad, dr.cy, ylo, yhi);
                 ok &= (ylo > -32768) & (yhi < 32767);
-                dyn_nrows = max(dyn_nrows, yhi + M::kHi + 1 - (ylo - M::kLo));
+                const TileRect rf = tile_rect<M>(lo, hi, ylo, yhi);
+                dyn_wbytes = max(dyn_wbytes, rf.wbytes);
+                dyn_nrows = max(dyn_nrows, rf.nrows);
                 if (!tp.zero_border) ok &= inside_src(lo, hi, ylo, yhi) ? 1 : 0;
             } else if (!tp.zero_border) {
                 ok = 0;  // NaN coordinates: the border colour / the replicated edge pixel -- per-pixel path
@@ -628,8 +574,8 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
         dyn_wbytes = __reduce_max_sync(0xffffffffu, dyn_wbytes);
         dyn_nrows = __reduce_max_sync(0xffffffffu, dyn_nrows);
         ok = __all_sync(0xffffffffu, ok);
-        fast = full_tile && ok && !nan_px && dyn_wbytes <= kPitchMax &&
-               dyn_nrows <= M::kRowsMin + (kRowSizes - 1) * kRowsStep && stage_fits(dyn_nrows, max(dyn_wbytes, kPitchMin));
+        fast = full_tile && ok && !nan_px && dyn_wbytes <= kPitchMax && box_rsel<M>(dyn_nrows) < kRowSizes &&
+               stage_fits(M::kRowsMin + box_rsel<M>(dyn_nrows) * kRowsStep, max(dyn_wbytes, kPitchMin));
     }
 
     if (!fast) {  // per-pixel gather from global memory with full border handling (rare tiles)
@@ -639,30 +585,13 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
                 const int i = x0 + pcol(k), j = y0 + prow(k);
                 if (i < a.W && j < a.H) {
                     for (int f = f0; f < f1; ++f) {
-                        uint8_t* drow = a.dst + (long long)f * a.dst_frame_stride + (long long)j * a.dst_pitch;
                         int qx = sx[k], qy = sy[k];
                         if (dynr) {
                             const double rad = __ldg(dr.radius + f);
                             qx = denorm_q<M>(nx[k], rad, dr.cx);
                             qy = denorm_q<M>(ny[k], rad, dr.cy);
                         }
-                        for (int v = v_begin; v < v_end; ++v) {
-                            const ViewArgs& vw = a.view[v];
-                            Src s{vw.src + (long long)f * vw.frame_stride, vw.rows, vw.cols, vw.pitch};
-                            int px[3];
-                            if (M::kInterp == VR180_INTER_NEAREST)
-                                fetch_tap<3>(s, sat16(qx), sat16(qy), a.border_mode, a.bv, px);
-                            else if (M::kInterp == VR180_INTER_LINEAR)
-                                sample_linear<3>(s, qx, qy, a.border_mode, a.bv, px);
-                            else if (M::kInterp == VR180_INTER_CUBIC)
-                                sample_tab<3, 4>(s, qx, qy, tp.tab, a.border_mode, a.bv, px);
-                            else
-                                sample_tab<3, 8>(s, qx, qy, tp.tab, a.border_mode, a.bv, px);
-                            uint8_t* o = drow + (long long)(vw.dst_x_offset + i) * 3;
-                            o[0] = (uint8_t)px[0];
-                            o[1] = (uint8_t)px[1];
-                            o[2] = (uint8_t)px[2];
-                        }
+                        gather_pixel<M>(a, f, i, j, v_begin, v_end, qx, qy, tp.tab);
                     }
                 }
             }
@@ -670,44 +599,14 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
         return;
     }
 
-    // ---- row pitch of the stages = TMA box width ------------------------------------------------------------
-    // Candidates: the kPitchCands smallest multiples of 16 bytes that hold the rectangle.  Cost of a candidate in
-    // shared-memory wavefronts per (frame, eye) item: the tap loads (every sampling warp measures the wavefronts
-    // = max distinct words per bank, counted with match.any, of the first tap load of its step k = 0; a tile has
-    // 32 steps of ~6 loads with the same address pattern) + the TMA write of the box (64 bytes per wavefront, measured).
-    int pitch = max(dynr ? dyn_wbytes : wbytes, kPitchMin);
-    if (tp.debug & 1) pitch = pitch <= 160 ? 160 : (pitch <= 224 ? 224 : 256);
+    // ---- row pitch of the stages = TMA box width: the kPitchCands smallest multiples of 16 bytes that hold the
+    // rectangle compete (pitch_costs) ----------------------------------------------------------------------------
+    int pitch = max(dynr ? dyn_wbytes : rc.wbytes, kPitchMin);
     // (not worth ~100 instructions per thread when the tile serves only a few frames: tightest box then)
     if (!dynr && (f1 - f0) * nv >= 8) {
-        const int box_rows = box_rows_of(nrows);
-        if (sampler) {
-            const int row = (sy[0] >> M::kShift) - M::kLo - ry0, col = 3 * ((sx[0] >> M::kShift) - M::kLo) - bx0;
-            int cost = 0;
-#pragma unroll
-            for (int e = 0; e < kPitchCands; ++e) {
-                const int w = (row * (pitch + kPitchStep * e) + col) >> 2;
-                const unsigned same = __match_any_sync(0xffffffffu, w);
-                const bool leader = (__ffs(same) - 1) == lane;  // one lane per distinct word
-                const unsigned lm = __ballot_sync(0xffffffffu, leader);
-                int deg = 0;
-                if (leader) deg = __popc(__match_any_sync(lm, w & 31));
-                deg = __reduce_max_sync(0xffffffffu, deg);
-                if (lane == e) cost = deg;
-            }
-            constexpr int kStepsPerWarp = M::kTileH * kTileW / kSamplers;  // warp steps (32 pixels) of a tile, per warp
-            constexpr int kLoadsPerTile = kStepsPerWarp * (M::kInterp == VR180_INTER_NEAREST ? 2 : M::kInterp == VR180_INTER_LINEAR ? 6
-                                                           : M::kInterp == VR180_INTER_CUBIC ? 16 : 56);
-            if (lane < kPitchCands) atomicAdd(&s_cost[lane], cost * kLoadsPerTile);
-        }
+        if (sampler) pitch_costs<M>(sx[0], sy[0], rc, pitch, lane, s_cost);
         __syncthreads();
-        int best = 0, best_cost = INT_MAX;
-#pragma unroll
-        for (int e = 0; e < kPitchCands; ++e) {
-            const int pe = pitch + kPitchStep * e;
-            const int c = s_cost[e] + box_rows * pe / 64;
-            if (pe <= kPitchMax && stage_fits(nrows, pe) && c < best_cost) { best_cost = c; best = e; }
-        }
-        if (!(tp.debug & 1)) pitch += kPitchStep * best;
+        pitch = pick_pitch(s_cost, pitch, rc.box_rows, [&](int pe) { return stage_fits(rc.box_rows, pe); });
     }
 
     // ---- per-pixel constants of the frame loop ------------------------------------------------------------
@@ -715,7 +614,7 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
 #pragma unroll
     for (int k = 0; k < kPx; ++k) {
         const int ix = sx[k] >> M::kShift, iy = sy[k] >> M::kShift;
-        const int off = (iy - M::kLo - ry0) * pitch + 3 * (ix - M::kLo) - bx0;
+        const int off = (iy - M::kLo - rc.ry0) * pitch + 3 * (ix - M::kLo) - rc.bx0;
         M::set_offset(pc[k], off, true);
         if (sampler && !dynr) M::weights(pc[k], sx[k] & 31, sy[k] & 31, tp.tab);
     }
@@ -731,9 +630,9 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
         }
     }
     TileGeom tg;
-    tg.nrows = dynr ? dyn_nrows : nrows;
-    tg.bx0 = bx0;
-    tg.ry0 = ry0;
+    tg.rsel = dynr ? box_rsel<M>(dyn_nrows) : rc.rsel;
+    tg.bx0 = rc.bx0;
+    tg.ry0 = rc.ry0;
     tg.x0 = x0;
     tg.y0 = y0;
     if (DYN && dynr) {
@@ -757,13 +656,14 @@ __global__ void __launch_bounds__(kSamplers) k_pack_tiles(const float* __restric
                                                          long long map_pitch, int W, int H, int tiles_x, int n_tiles,
                                                          void* __restrict__ packed) {
     constexpr int kPx = M::kPx;
-    __shared__ int s_red[kSamplers / 32][4];
+    __shared__ int4 s_red[kSamplers / 32];
+    __shared__ int s_cost[kPitchCands];
     const int tid = threadIdx.x, lane = tid & 31, sw = tid >> 5;
     const int tx = blockIdx.x % tiles_x, ty = blockIdx.x / tiles_x;
     const int x0 = tx * kTileW, y0 = ty * M::kTileH;
     const bool full_tile = (x0 + kTileW <= W) && (y0 + M::kTileH <= H);
+    if (tid < kPitchCands) s_cost[tid] = 0;
     int sx[kPx], sy[kPx];
-    int mnx = INT_MAX, mxx = INT_MIN, mny = INT_MAX, mxy = INT_MIN;
 #pragma unroll
     for (int k = 0; k < kPx; ++k) {
         const int i = x0 + lane, j = y0 + kPx * sw + k;  // row patches: a warp owns rows kPx sw .. kPx sw + kPx - 1
@@ -772,71 +672,30 @@ __global__ void __launch_bounds__(kSamplers) k_pack_tiles(const float* __restric
             sx[k] = M::quant(__ldg(xmap + (long long)j * map_pitch + i));
             sy[k] = M::quant(__ldg(ymap + (long long)j * map_pitch + i));
         }
-        const int ix = sat16(sx[k] >> M::kShift), iy = sat16(sy[k] >> M::kShift);
-        mnx = min(mnx, ix); mxx = max(mxx, ix);
-        mny = min(mny, iy); mxy = max(mxy, iy);
     }
-    mnx = __reduce_min_sync(0xffffffffu, mnx); mxx = __reduce_max_sync(0xffffffffu, mxx);
-    mny = __reduce_min_sync(0xffffffffu, mny); mxy = __reduce_max_sync(0xffffffffu, mxy);
-    if (lane == 0) { s_red[sw][0] = mnx; s_red[sw][1] = mxx; s_red[sw][2] = mny; s_red[sw][3] = mxy; }
+    block_box_store<M>(sx, sy, s_red, sw, lane == 0);
     __syncthreads();
-#pragma unroll
-    for (int w = 0; w < kSamplers / 32; ++w) {
-        mnx = min(mnx, s_red[w][0]); mxx = max(mxx, s_red[w][1]);
-        mny = min(mny, s_red[w][2]); mxy = max(mxy, s_red[w][3]);
-    }
+    const int4 box = block_box_load(s_red, lane);
+    const int mnx = box.x, mxx = box.y, mny = box.z, mxy = box.w;
     const bool ok = full_tile && mnx > -32768 && mny > -32768 && mxx < 32767 && mxy < 32767 && mxx - mnx <= 255 &&
                     mxy - mny <= 255;
     // Geometry of the tile's source rectangle for the tile-streaming kernel (stream.cu), which has no time to derive it
-    // per launch: box rows, and the row pitch (= TMA box width) with the fewest shared-memory wavefronts among the
-    // kPitchCands tightest -- the bank conflicts of the tile's own tap addresses (every warp counts, with match.any, the
-    // distinct words per bank of the first tap load of its first row) + the TMA write of the box, as k_warp_tiled does.
-    __shared__ int s_cost[kPitchCands];
-    if (tid < kPitchCands) s_cost[tid] = 0;
+    // per launch: box rows, and the row pitch (= TMA box width) that k_warp_tiled's choice gives a stage slot.
+    const TileRect rc = tile_rect<M>(mnx, mxx, mny, mxy);
+    const bool stageable = ok && rc.wbytes <= kPitchMax && rc.rsel < kRowSizes;
+    const int pitch0 = max(rc.wbytes, kPitchMin);
+    if (stageable) pitch_costs<M>(sx[0], sy[0], rc, pitch0, lane, s_cost);  // (CTA-uniform)
     __syncthreads();
-    const int bx0 = (3 * (mnx - M::kLo)) & ~15, bx1 = (3 * (mxx + M::kHi + 1) + 15) & ~15, ry0 = mny - M::kLo;
-    const int wbytes = bx1 - bx0, nrows = mxy + M::kHi + 1 - ry0;
-    const int rsel = nrows <= M::kRowsMin ? 0 : (nrows - M::kRowsMin + kRowsStep - 1) / kRowsStep;
-    const int box_rows = M::kRowsMin + rsel * kRowsStep;
-    const int pitch0 = max(wbytes, kPitchMin);
-    const bool stageable = ok && wbytes <= kPitchMax && rsel < kRowSizes;
-    int widx = 0;
-    if (stageable) {  // CTA-uniform
-        const int row = (sy[0] >> M::kShift) - M::kLo - ry0, col = 3 * ((sx[0] >> M::kShift) - M::kLo) - bx0;
-        int cost = 0;
-#pragma unroll
-        for (int e = 0; e < kPitchCands; ++e) {
-            const int w = (row * (pitch0 + kPitchStep * e) + col) >> 2;
-            const unsigned same = __match_any_sync(0xffffffffu, w);
-            const bool leader = (__ffs(same) - 1) == lane;  // one lane per distinct word
-            const unsigned lm = __ballot_sync(0xffffffffu, leader);
-            int deg = 0;
-            if (leader) deg = __popc(__match_any_sync(lm, w & 31));
-            deg = __reduce_max_sync(0xffffffffu, deg);
-            if (lane == e) cost = deg;
-        }
-        constexpr int kStepsPerWarp = M::kTileH * kTileW / kSamplers;
-        constexpr int kLoadsPerTile = kStepsPerWarp * (M::kInterp == VR180_INTER_NEAREST ? 2 : M::kInterp == VR180_INTER_LINEAR ? 6
-                                                       : M::kInterp == VR180_INTER_CUBIC ? 16 : 56);
-        if (lane < kPitchCands) atomicAdd(&s_cost[lane], cost * kLoadsPerTile);
-    }
-    __syncthreads();
-    if (stageable) {
-        int best_cost = INT_MAX;
-#pragma unroll
-        for (int e = 0; e < kPitchCands; ++e) {
-            const int pe = pitch0 + kPitchStep * e;
-            const int c = s_cost[e] + box_rows * pe / 64;
-            if (pe <= kPitchMax && (e == 0 || box_rows * pe <= kStreamSlotBytes<M>) && c < best_cost) { best_cost = c; widx = (pe - kPitchMin) / kPitchStep; }
-        }
-    }
-    const int pitch = kPitchMin + kPitchStep * widx;
+    const int pitch = !stageable ? kPitchMin : pick_pitch(s_cost, pitch0, rc.box_rows, [&](int pe) {
+        return pe == pitch0 || rc.box_rows * pe <= kStreamSlotBytes<M>;
+    });
+    const int widx = (pitch - kPitchMin) / kPitchStep;
     if (tid == 0) {
         int4 h;
         h.x = (mnx & 0xffff) | (mxx << 16);
         h.y = (mny & 0xffff) | (mxy << 16);
         h.z = (ok ? kHdrPackable : 0) | (stageable ? kHdrStageable : 0) |
-              (stageable && box_rows * pitch <= kStreamSlotBytes<M> ? kHdrFitsSlot : 0) | (widx << 8) | (rsel << 12);
+              (stageable && rc.box_rows * pitch <= kStreamSlotBytes<M> ? kHdrFitsSlot : 0) | (widx << 8) | (rc.rsel << 12);
         h.w = 0;
         reinterpret_cast<int4*>(packed)[blockIdx.x] = h;
     }
@@ -853,7 +712,7 @@ __global__ void __launch_bounds__(kSamplers) k_pack_tiles(const float* __restric
 }  // namespace tiled
 
 static int tile_height_of(int interp) {
-    return interp == VR180_INTER_LINEAR || interp == VR180_INTER_NEAREST ? tiled::Linear::kTileH
+    return interp == VR180_INTER_LINEAR || interp == VR180_INTER_NEAREST ? tiled::LinearP::kTileH
            : interp == VR180_INTER_CUBIC                                  ? tiled::Cubic::kTileH
            : interp == VR180_INTER_LANCZOS4                               ? tiled::Lanczos4::kTileH
                                                                           : 0;
@@ -878,7 +737,7 @@ int launch_pack_lut_tiles(const float* xmap, const float* ymap, int64_t map_pitc
     if (interp == VR180_INTER_NEAREST)
         k_pack_tiles<Nearest><<<grid, kSamplers, 0, st>>>(xmap, ymap, (long long)map_pitch, W, H, tiles_x, (int)n_tiles, packed);
     else if (interp == VR180_INTER_LINEAR)
-        k_pack_tiles<Linear><<<grid, kSamplers, 0, st>>>(xmap, ymap, (long long)map_pitch, W, H, tiles_x, (int)n_tiles, packed);
+        k_pack_tiles<LinearP><<<grid, kSamplers, 0, st>>>(xmap, ymap, (long long)map_pitch, W, H, tiles_x, (int)n_tiles, packed);
     else if (interp == VR180_INTER_CUBIC)
         k_pack_tiles<Cubic><<<grid, kSamplers, 0, st>>>(xmap, ymap, (long long)map_pitch, W, H, tiles_x, (int)n_tiles, packed);
     else
@@ -947,7 +806,6 @@ static EncodeTiledFn encode_tiled_fn() {
 
 // uint8 tensor (row_bytes, rows, frames) with byte strides (pitch, frame_stride); box (box_w, box_h, 1).
 // Out-of-bounds box elements are filled with zeros on loads and dropped on stores.
-int tiled_debug_flags();
 static bool encode_u8_3d(CUtensorMap* out, const void* base, long long row_bytes, long long rows, long long frames,
                          long long pitch, long long frame_stride, int box_w, int box_h, int box_d) {
     EncodeTiledFn fn = encode_tiled_fn();
@@ -957,11 +815,8 @@ static bool encode_u8_3d(CUtensorMap* out, const void* base, long long row_bytes
     const cuuint64_t strides[2] = {(cuuint64_t)pitch, (cuuint64_t)frame_stride};
     const cuuint32_t box[3] = {(cuuint32_t)box_w, (cuuint32_t)box_h, (cuuint32_t)box_d};
     const cuuint32_t estr[3] = {1u, 1u, 1u};
-    // VR180_TILED_DEBUG bits 4-5 (experiment): L2 promotion of the boxes' sectors -- 0: 128 B (default), 1: none, 2: 64 B, 3: 256 B
-    static const CUtensorMapL2promotion promo[4] = {CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                                                    CU_TENSOR_MAP_L2_PROMOTION_L2_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B};
     return fn(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(base), dims, strides, box, estr,
-              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, promo[(tiled_debug_flags() >> 4) & 3],
+              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
@@ -1069,13 +924,9 @@ static int launch_mode(const RemapArgs& a0, const vr180_chain_t& c0, const vr180
     if (!tmp) return VR180_ERR_UNSUPPORTED;
     const TmaMaps& tm = *tmp;
 
-    static std::atomic<int> attr_done[64];
     int dev = 0;
-    VR180_CUDA(cudaGetDevice(&dev));
-    if (dev < 64 && !attr_done[dev].load(std::memory_order_acquire)) {
-        VR180_CUDA(cudaFuncSetAttribute(k_warp_tiled<M, DYN, FR>, cudaFuncAttributeMaxDynamicSharedMemorySize, Lay<M>::kSmemBytes));
-        attr_done[dev].store(1, std::memory_order_release);
-    }
+    const int rc = max_dyn_smem_once<k_warp_tiled<M, DYN, FR>>(Lay<M>::kSmemBytes, dev);
+    if (rc != VR180_OK) return rc;
 
     RemapArgs a = a0;
     TiledParams tp;
@@ -1084,7 +935,7 @@ static int launch_mode(const RemapArgs& a0, const vr180_chain_t& c0, const vr180
     tp.tiles_x = tiles_x;
     tp.n_tiles = tiles_x * tiles_y;
     tp.tab = tab;
-    tp.zero_border = (a.border_mode == VR180_BORDER_CONSTANT && !(a.bv[0] | a.bv[1] | a.bv[2])) ? 1 : 0;
+    tp.zero_border = zero_border(a);
     tp.debug = tiled_debug_flags();
     const long long tiles = (long long)tiles_x * tiles_y * n_groups;
     int fpc = frames_per_cta(tiles, a.n_frames, a.share_map ? a.n_views : 1);
@@ -1108,6 +959,17 @@ static int launch_mode(const RemapArgs& a0, const vr180_chain_t& c0, const vr180
     g_launches.fetch_add(1, std::memory_order_relaxed);
     VR180_CUDA(cudaGetLastError());
     return VR180_OK;
+}
+
+// FR = frames per pipeline item for `fpc` frames per CTA: 2 from two frames on, bicubic 4 from eight on
+template <class M>
+static int launch_tiled(const RemapArgs& a0, const vr180_chain_t& c0, const vr180_chain_t& c1, const short* tab, bool dyn,
+                        int fpc, cudaStream_t st) {
+    if constexpr (M::kInterp == VR180_INTER_CUBIC) {
+        if (fpc >= 8) return dyn ? launch_mode<M, true, 4>(a0, c0, c1, tab, st) : launch_mode<M, false, 4>(a0, c0, c1, tab, st);
+    }
+    if (fpc >= 2) return dyn ? launch_mode<M, true, 2>(a0, c0, c1, tab, st) : launch_mode<M, false, 2>(a0, c0, c1, tab, st);
+    return dyn ? launch_mode<M, true, 1>(a0, c0, c1, tab, st) : launch_mode<M, false, 1>(a0, c0, c1, tab, st);
 }
 
 // Host-side eligibility + launch.  Returns VR180_ERR_UNSUPPORTED when the request is outside the fast path (the
@@ -1161,42 +1023,16 @@ int launch_remap_tiled(const RemapArgs& a0, int channels, int interp, const vr18
             if (rc != VR180_ERR_UNSUPPORTED) return rc;
         }
     }
-    // two frames per pipeline item when the frames share their rectangles and every CTA gets at least two of them
-    const int tile_h = interp == VR180_INTER_LINEAR || interp == VR180_INTER_NEAREST ? tiled::Linear::kTileH
-                       : interp == VR180_INTER_CUBIC ? tiled::Cubic::kTileH
-                                                     : tiled::Lanczos4::kTileH;
+    // two frames per pipeline item when the frames share their rectangles (per-frame radii: the chunks whose frames all
+    // share one radius, a static rig) and every CTA gets at least two of them
+    const int tile_h = tile_height_of(interp);
     const long long tiles = (long long)((a0.W + tiled::kTileW - 1) / tiled::kTileW) * ((a0.H + tile_h - 1) / tile_h) * n_groups;
-    const int vpc = a0.share_map ? a0.n_views : 1;
-    const bool pairs = !dyn && frames_per_cta(tiles, a0.n_frames, vpc) >= 2;
-    // per-frame radii: chunks whose frames all share one radius (a static rig) run the same multi-frame items
-    const bool pairs_dyn = dyn && frames_per_cta(tiles, a0.n_frames, vpc) >= 2;
-    if (interp == VR180_INTER_NEAREST) {
-        if (dyn) return pairs_dyn ? launch_mode<tiled::Nearest, true, 2>(a0, c0, c1, nullptr, st)
-                                  : launch_mode<tiled::Nearest, true, 1>(a0, c0, c1, nullptr, st);
-        return pairs ? launch_mode<tiled::Nearest, false, 2>(a0, c0, c1, nullptr, st)
-                     : launch_mode<tiled::Nearest, false, 1>(a0, c0, c1, nullptr, st);
-    }
-    if (interp == VR180_INTER_LINEAR) {  // LinearP: byte alignment by PRMT (5.8 % fewer instructions than Linear's funnel shifts)
-        if (dyn) return pairs_dyn ? launch_mode<tiled::LinearP, true, 2>(a0, c0, c1, nullptr, st)
-                                  : launch_mode<tiled::LinearP, true, 1>(a0, c0, c1, nullptr, st);
-        return pairs ? launch_mode<tiled::LinearP, false, 2>(a0, c0, c1, nullptr, st)
-                     : launch_mode<tiled::LinearP, false, 1>(a0, c0, c1, nullptr, st);
-    }
+    const int fpc = frames_per_cta(tiles, a0.n_frames, a0.share_map ? a0.n_views : 1);
+    if (interp == VR180_INTER_NEAREST) return launch_tiled<tiled::Nearest>(a0, c0, c1, nullptr, dyn, fpc, st);
+    if (interp == VR180_INTER_LINEAR) return launch_tiled<tiled::LinearP>(a0, c0, c1, nullptr, dyn, fpc, st);
     if (!weight_tab) return VR180_ERR_UNSUPPORTED;
-    if (interp == VR180_INTER_LANCZOS4) {
-        if (dyn) return pairs_dyn ? launch_mode<tiled::Lanczos4, true, 2>(a0, c0, c1, weight_tab, st)
-                                  : launch_mode<tiled::Lanczos4, true, 1>(a0, c0, c1, weight_tab, st);
-        return pairs ? launch_mode<tiled::Lanczos4, false, 2>(a0, c0, c1, weight_tab, st)
-                     : launch_mode<tiled::Lanczos4, false, 1>(a0, c0, c1, weight_tab, st);
-    }
-    if (dyn) {
-        if (frames_per_cta(tiles, a0.n_frames, vpc) >= 8) return launch_mode<tiled::Cubic, true, 4>(a0, c0, c1, weight_tab, st);
-        return pairs_dyn ? launch_mode<tiled::Cubic, true, 2>(a0, c0, c1, weight_tab, st)
-                         : launch_mode<tiled::Cubic, true, 1>(a0, c0, c1, weight_tab, st);
-    }
-    if (frames_per_cta(tiles, a0.n_frames, vpc) >= 8) return launch_mode<tiled::Cubic, false, 4>(a0, c0, c1, weight_tab, st);
-    return pairs ? launch_mode<tiled::Cubic, false, 2>(a0, c0, c1, weight_tab, st)
-                 : launch_mode<tiled::Cubic, false, 1>(a0, c0, c1, weight_tab, st);
+    if (interp == VR180_INTER_LANCZOS4) return launch_tiled<tiled::Lanczos4>(a0, c0, c1, weight_tab, dyn, fpc, st);
+    return launch_tiled<tiled::Cubic>(a0, c0, c1, weight_tab, dyn, fpc, st);
 }
 
 }  // namespace vr180

@@ -68,7 +68,7 @@ struct TiledParams {
     int tiles_x;
     int n_tiles;     // tiles of one map (tiles_x * tiles_y): layout of a tile-packed LUT
     int sep_prefix;  // generic chains only: ops[0..1] = Normalize, EquirectangularEncoder
-    int debug;       // VR180_TILED_DEBUG: bit 0 = legacy pitches (160 / 224 bytes, no per-tile choice)
+    int debug;       // VR180_TILED_DEBUG: bit 8 = the standard chain through the op-by-op interpreter (chain.cuh)
     int zero_border; // BORDER_CONSTANT with a zero colour: TMA's out-of-bounds zero fill IS the border, so tiles that
                      // straddle the source edge stay staged; any other border only stages tiles that lie inside the source
     const short* tab;  // bicubic: OpenCV's 1024 x 16 int16 weight table (device)
@@ -95,16 +95,37 @@ constexpr int kHdrFitsSlot = 4;   // ... and one stage slot of the tile-streamin
 // bits 8-11: (row pitch - kPitchMin) / kPitchStep chosen for the tile; bits 12-15: box rows = kRowsMin + kRowsStep * r
 static_assert(sizeof(PackedHdr) == 16, "PackedHdr is one 128-bit load");
 __host__ __device__ inline size_t packed_entries_offset(long long n_tiles) { return ((size_t)n_tiles * 16 + 255) & ~(size_t)255; }
-__device__ __forceinline__ PackedHdr packed_header(const void* packed, unsigned tile) {
-    const int4 v = __ldg(reinterpret_cast<const int4*>(packed) + tile);
-    PackedHdr h;
-    h.mnx = (short)(v.x & 0xffff); h.mxx = (short)(v.x >> 16);
-    h.mny = (short)(v.y & 0xffff); h.mxy = (short)(v.y >> 16);
-    h.flags = v.z; h.pad = v.w;
-    return h;
+// the header as loaded (the streaming kernel keeps the prefetched next header in this form: three live registers)
+__device__ __forceinline__ int4 packed_header_raw(const void* packed, int tile) {
+    return __ldg(reinterpret_cast<const int4*>(packed) + tile);
 }
-__device__ __forceinline__ const uint32_t* packed_entries(const void* packed, long long n_tiles) {
-    return reinterpret_cast<const uint32_t*>(static_cast<const uint8_t*>(packed) + packed_entries_offset(n_tiles));
+struct TileHdr {  // a decoded PackedHdr
+    int mnx, mxx, mny, mxy, flags;
+};
+__device__ __forceinline__ TileHdr decode_header(const int4& v) {
+    return {(short)(v.x & 0xffff), v.x >> 16, (short)(v.y & 0xffff), v.y >> 16, v.z};
+}
+// the tile's kPx entries of thread `tid`: ONE 128-bit (bilinear / nearest), 64-bit (bicubic) or 32-bit (Lanczos4)
+// coalesced load
+template <class M>
+__device__ __forceinline__ void load_packed_entries(const void* packed, int n_tiles, int tile, int tid, uint32_t (&e)[M::kPx]) {
+    const uint32_t* ent = reinterpret_cast<const uint32_t*>(static_cast<const uint8_t*>(packed) + packed_entries_offset(n_tiles)) +
+                          ((size_t)tile * kSamplers + tid) * M::kPx;
+    if constexpr (M::kPx == 4) {
+        const uint4 v = __ldg(reinterpret_cast<const uint4*>(ent));
+        e[0] = v.x; e[1] = v.y; e[2] = v.z; e[3] = v.w;
+    } else if constexpr (M::kPx == 2) {
+        const uint2 v = __ldg(reinterpret_cast<const uint2*>(ent));
+        e[0] = v.x; e[1] = v.y;
+    } else {
+        e[0] = __ldg(ent);
+    }
+}
+// entry -> the mode's quantised coordinates (sx, sy), as M::quant would have produced them
+template <class M>
+__device__ __forceinline__ int2 unpack_entry(int hdr_mnx, int hdr_mny, uint32_t e) {
+    return make_int2(((hdr_mnx + (int)(e & 255u)) << M::kShift) | (int)((e >> 16) & 31u),
+                     ((hdr_mny + (int)((e >> 8) & 255u)) << M::kShift) | (int)((e >> 21) & 31u));
 }
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -152,33 +173,6 @@ __device__ __forceinline__ void bulk_wait_read() {  // all but the N newest bulk
     asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory");
 }
 
-// The 2 x 12-byte tap windows of a bilinear pixel (rows q0 and q1, shared-window addresses), byte-aligned:
-//   lo = [c0 c1 c2 c0'], hi = [c1' c2' . .] of each row (primed = the pixel at ix + 1).
-// Only a byte offset of 3 (sh == 24) reaches into the third word; the other lanes skip that load (fewer active lanes
-// = fewer bank conflicts).  The third word is loaded INTO THE REGISTER OF THE FIRST WORD, which is dead once `lo` has
-// been formed: a predicated load into a register of its own would have to preserve that register's old value for
-// the lanes that skip it, i.e. cost one loop-carried register per load (16 of the 56 registers of the two-frame loop,
-// plus the spills and moves they caused).  For sh < 24 the funnel shift of `hi` never looks at its upper operand.
-// volatile: the same shared address holds another frame after every barrier wait.
-__device__ __forceinline__ void lds_taps_aligned(uint32_t q0, uint32_t q1, int sh, uint32_t& r0lo, uint32_t& r0hi,
-                                                 uint32_t& r1lo, uint32_t& r1hi) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t.reg .b32 a0, a1, b0, b1;\n\t"
-        "setp.eq.s32 p, %6, 24;\n\t"
-        "ld.shared.u32 a0, [%4];\n\t"
-        "ld.shared.u32 a1, [%4+4];\n\t"
-        "ld.shared.u32 b0, [%5];\n\t"
-        "ld.shared.u32 b1, [%5+4];\n\t"
-        "shf.r.wrap.b32 %0, a0, a1, %6;\n\t"
-        "shf.r.wrap.b32 %2, b0, b1, %6;\n\t"
-        "@p ld.shared.u32 a0, [%4+8];\n\t"
-        "@p ld.shared.u32 b0, [%5+8];\n\t"
-        "shf.r.wrap.b32 %1, a1, a0, %6;\n\t"
-        "shf.r.wrap.b32 %3, b1, b0, %6;\n\t}"
-        : "=&r"(r0lo), "=&r"(r0hi), "=&r"(r1lo), "=&r"(r1hi)
-        : "r"(q0), "r"(q1), "r"(sh));
-}
-
 __device__ __forceinline__ void sts32(uint32_t addr, uint32_t v) {
     asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
 }
@@ -207,45 +201,7 @@ __device__ __forceinline__ uint32_t dp2a_hi_su(uint32_t w, uint32_t px, uint32_t
 // A mode fixes: pixels per thread (the per-pixel constants must stay in registers across the frames of the batch),
 // the tile height, the tap footprint (taps start kLo pixels / rows before the integer coordinate and end kHi after
 // it), the per-pixel constants and the sampling of one pixel from the staged rectangle.
-struct Linear {
-    static constexpr int kPx = 4, kTileH = 32, kLo = 0, kHi = 1, kRowsMin = 32, kInterp = VR180_INTER_LINEAR;
-    static constexpr int kShift = kInterBits;  // coordinates are 1/32-pixel fixed point: sx = cvRound(x * 32)
-    __device__ static __forceinline__ int quant(float m) { return quantise(m); }
-    static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 4, kMaxFR = 2;
-    static constexpr bool kRowPatch = true;  // a warp step = 32 pixels of one output row (pixel k of a thread: row 4 band + k)
-    struct Pixel {  // constant over the frames of the batch
-        int boff;          // byte offset (4-aligned) of the 12-byte tap window of row 0 inside a stage buffer
-        int sh;            // 8 * (tap00 byte offset & 3)
-        uint32_t W01, W23; // 16-bit lanes {64 w00, 64 w01}, {64 w10, 64 w11}
-    };
-    __device__ static __forceinline__ void set_offset(Pixel& p, int off, bool valid) {
-        p.boff = valid ? (off & ~3) : 0;
-        p.sh = (off & 3) * 8;
-    }
-    // w00 = 1024 (ax = ay = 0, all other weights 0) is encoded as 65535: (65535 p + 32768) >> 16 is still exactly p.
-    __device__ static __forceinline__ void weights(Pixel& p, int ax, int ay, const short*) {
-        const int w00 = (32 - ax) * (32 - ay), w01 = ax * (32 - ay), w10 = (32 - ax) * ay, w11 = ax * ay;
-        p.W01 = (uint32_t)min(64 * w00, 65535) | ((uint32_t)(64 * w01) << 16);
-        p.W23 = (uint32_t)(64 * w10) | ((uint32_t)(64 * w11) << 16);
-    }
-    // One output pixel from the staged rectangle: the three result bytes [c0 c1 c2 0].
-    // `sbuf`: shared-window address of the stage, `pitch`: its row pitch in bytes
-    __device__ static __forceinline__ uint32_t sample(uint32_t sbuf, const Pixel& p, uint32_t pitch) {
-        uint32_t r0lo, r0hi, r1lo, r1hi;  // byte-aligned: lo = [c0 c1 c2 c0'], hi = [c1' c2' . .]
-        const uint32_t row0 = sbuf + (uint32_t)p.boff;
-        lds_taps_aligned(row0, row0 + pitch, p.sh, r0lo, r0hi, r1lo, r1hi);
-        const uint32_t q0 = __byte_perm(r0lo, r1lo, 0x7430);  // channel 0: [p00 p01 | p10 p11]
-        const uint32_t t0 = __byte_perm(r0lo, r0hi, 0x5241);  // row 0: [c1 c1' | c2 c2']
-        const uint32_t t1 = __byte_perm(r1lo, r1hi, 0x5241);  // row 1
-        // (sum_t w_t p_t + 512) >> 10 == (sum_t 64 w_t p_t + 32768) >> 16: the result is byte 2 of s (s < 2^24)
-        const uint32_t s0 = __dp2a_hi(p.W23, q0, __dp2a_lo(p.W01, q0, 32768u));
-        const uint32_t s1 = __dp2a_lo(p.W23, t1, __dp2a_lo(p.W01, t0, 32768u));
-        const uint32_t s2 = __dp2a_hi(p.W23, t1, __dp2a_hi(p.W01, t0, 32768u));
-        return __byte_perm(__byte_perm(s0, s1, 0x0062), s2, 0x7610);
-    }
-};
-
-// Bilinear as launched: the byte alignment is done by PRMT with per-pixel selectors instead of funnel shifts
+// INTER_LINEAR: the byte alignment of the taps is done by PRMT with per-pixel selectors rather than by funnel shifts
 // (measured on the 64-pair 8K launch: 2.42 G instead of 2.57 G warp instructions, 2.89 instead of 2.95 ms).
 // The window of a row is bytes s .. s + 5 (s = offset & 3) of the words [a0 a1 (a2)]:
 //   u  = PRMT(a0, a1, selA) = [c0 c0' . .]            c0 at s, c0' at s + 3 <= 6: always inside (a0, a1)
@@ -256,14 +212,14 @@ struct Linear {
 // the low 16 bits of its selector; the address is one LEA.HI).
 struct LinearP {
     static constexpr int kPx = 4, kTileH = 32, kLo = 0, kHi = 1, kRowsMin = 32, kInterp = VR180_INTER_LINEAR;
-    static constexpr int kShift = kInterBits;
+    static constexpr int kShift = kInterBits;  // coordinates are 1/32-pixel fixed point: sx = cvRound(x * 32)
     __device__ static __forceinline__ int quant(float m) { return quantise(m); }
-    static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 4, kMaxFR = 2;
-    static constexpr bool kRowPatch = true;
-    struct Pixel {
+    static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 4;
+    static constexpr bool kRowPatch = true;  // a warp step = 32 pixels of one output row (pixel k of a thread: row 4 band + k)
+    struct Pixel {  // constant over the frames of the batch
         uint32_t osel;     // window byte offset (4-aligned) << 16 | selA
         uint32_t selT;
-        uint32_t W01, W23;
+        uint32_t W01, W23; // 16-bit lanes {64 w00, 64 w01}, {64 w10, 64 w11}
     };
     __device__ static __forceinline__ void set_offset(Pixel& p, int off, bool valid) {
         // selA = s | (s + 3) << 4 = 0x30 + 0x11 s;  selT = (s + 1) | (s + 4) << 4 | (s + 2) << 8 | (s + 5) << 12 = 0x5241 +
@@ -272,12 +228,14 @@ struct LinearP {
         p.osel = ((valid ? ((uint32_t)off & ~3u) : 0u) << 16) | (0x30u + 0x11u * s);
         p.selT = (0x5241u + 0x1111u * s) & 0x7fffu;
     }
-    __device__ static __forceinline__ void weights(Pixel& p, int ax, int ay, const short* t) {
-        Linear::Pixel q;
-        Linear::weights(q, ax, ay, t);
-        p.W01 = q.W01;
-        p.W23 = q.W23;
+    // w00 = 1024 (ax = ay = 0, all other weights 0) is encoded as 65535: (65535 p + 32768) >> 16 is still exactly p.
+    __device__ static __forceinline__ void weights(Pixel& p, int ax, int ay, const short*) {
+        const int w00 = (32 - ax) * (32 - ay), w01 = ax * (32 - ay), w10 = (32 - ax) * ay, w11 = ax * ay;
+        p.W01 = (uint32_t)min(64 * w00, 65535) | ((uint32_t)(64 * w01) << 16);
+        p.W23 = (uint32_t)(64 * w10) | ((uint32_t)(64 * w11) << 16);
     }
+    // One output pixel from the staged rectangle: the three result bytes [c0 c1 c2 0].
+    // `sbuf`: shared-window address of the stage, `pitch`: its row pitch in bytes
     __device__ static __forceinline__ uint32_t sample(uint32_t sbuf, const Pixel& p, uint32_t pitch) {
         const uint32_t row0 = sbuf + (p.osel >> 16);
         uint32_t q0, t0, t1;
@@ -297,6 +255,7 @@ struct LinearP {
             "prmt.b32 %2, b0, b1, %6;\n\t}"
             : "=&r"(q0), "=&r"(t0), "=&r"(t1)
             : "r"(row0), "r"(row0 + pitch), "r"(p.osel), "r"(p.selT));
+        // (sum_t w_t p_t + 512) >> 10 == (sum_t 64 w_t p_t + 32768) >> 16: the result is byte 2 of s (s < 2^24)
         const uint32_t s0 = __dp2a_hi(p.W23, q0, __dp2a_lo(p.W01, q0, 32768u));
         const uint32_t s1 = __dp2a_lo(p.W23, t1, __dp2a_lo(p.W01, t0, 32768u));
         const uint32_t s2 = __dp2a_hi(p.W23, t1, __dp2a_hi(p.W01, t0, 32768u));
@@ -309,7 +268,7 @@ struct Nearest {
     static constexpr int kPx = 4, kTileH = 32, kLo = 0, kHi = 0, kRowsMin = 32, kInterp = VR180_INTER_NEAREST;
     static constexpr int kShift = 0;
     __device__ static __forceinline__ int quant(float m) { return cv_round(m); }
-    static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 4, kMaxFR = 2;
+    static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 4;
     static constexpr bool kRowPatch = true;
     struct Pixel {
         int boff;  // byte offset (4-aligned) of the 8-byte window that holds the pixel
@@ -333,7 +292,7 @@ struct Cubic {
     __device__ static __forceinline__ int quant(float m) { return quantise(m); }
     // a thread owns only 2 pixels (their 16 table weights take 16 registers), so an item is FOUR frames: the
     // per-item bookkeeping is paid once per 8 pixels of a thread, as for the bilinear mode
-    static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 8, kMaxFR = 4;
+    static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 8;
     static constexpr bool kRowPatch = true;  // a warp step = 32 pixels of one output row (pixel k of a thread: row 2 warp + k)
     struct Pixel {
         int boff;       // byte offset (4-aligned) of the 16-byte window of tap row 0 (iy - 1), first tap ix - 1
@@ -386,7 +345,7 @@ struct Lanczos4 {
     static constexpr int kShift = kInterBits;  // coordinates are 1/32-pixel fixed point: sx = cvRound(x * 32)
     __device__ static __forceinline__ int quant(float m) { return quantise(m); }
     static constexpr int kStageArea = 16384, kWeightSmem = kSamplers * 128;  // 16 KB of stages + 32 KB of weights
-    static constexpr int kOutTiles = 4, kMaxFR = 2;
+    static constexpr int kOutTiles = 4;
     struct Pixel {
         int boff;        // byte offset (4-aligned) of the 28-byte window of tap row 0 (iy - 3), first tap ix - 3
         int sh;
@@ -474,6 +433,127 @@ __device__ __forceinline__ void dyn_range(double nmin, double nmax, double rad, 
     hi = max(a, b);
 }
 
+// ---- tile geometry: one definition for k_warp_tiled, k_pack_tiles (which stores it in the tile header) and
+// k_warp_stream (which reads it back) ---------------------------------------------------------------------------
+// Block-wide integer bounding box {min ix, max ix, min iy, max iy} of the sampling warps' pixels, in two halves around
+// a barrier of the caller: every warp reduces its own box and lane 0 of a sampling warp stores it as record `warp`;
+// after the barrier lane w reads record w -- one 128-bit load + four REDUX (a loop over the 8 records is 64
+// instructions per thread, and a one-frame tile has few to amortise them over).
+template <class M>
+__device__ __forceinline__ void block_box_store(const int (&sx)[M::kPx], const int (&sy)[M::kPx], int4* s_red, int warp,
+                                                bool store) {
+    int mnx = INT_MAX, mxx = INT_MIN, mny = INT_MAX, mxy = INT_MIN;
+#pragma unroll
+    for (int k = 0; k < M::kPx; ++k) {
+        const int ix = sat16(sx[k] >> M::kShift), iy = sat16(sy[k] >> M::kShift);
+        mnx = min(mnx, ix);
+        mxx = max(mxx, ix);
+        mny = min(mny, iy);
+        mxy = max(mxy, iy);
+    }
+    mnx = __reduce_min_sync(0xffffffffu, mnx);
+    mxx = __reduce_max_sync(0xffffffffu, mxx);
+    mny = __reduce_min_sync(0xffffffffu, mny);
+    mxy = __reduce_max_sync(0xffffffffu, mxy);
+    if (store) s_red[warp] = make_int4(mnx, mxx, mny, mxy);
+}
+__device__ __forceinline__ int4 block_box_load(const int4* s_red, int lane) {
+    int4 r = make_int4(INT_MAX, INT_MIN, INT_MAX, INT_MIN);
+    if (lane < kSamplers / 32) r = s_red[lane];
+    r.x = __reduce_min_sync(0xffffffffu, r.x);
+    r.y = __reduce_max_sync(0xffffffffu, r.y);
+    r.z = __reduce_min_sync(0xffffffffu, r.z);
+    r.w = __reduce_max_sync(0xffffffffu, r.w);
+    return r;
+}
+
+// TMA box rows for a rectangle of `nrows` source rows: M::kRowsMin + kRowsStep * rsel (rsel < kRowSizes to fit a box)
+template <class M>
+__device__ __forceinline__ int box_rsel(int nrows) {
+    return nrows <= M::kRowsMin ? 0 : (nrows - M::kRowsMin + kRowsStep - 1) / kRowsStep;
+}
+// Source rectangle of a tile from the extreme integer coordinates of its pixels: the taps cover columns
+// ix - kLo .. ix + kHi and rows iy - kLo .. iy + kHi; columns in 16-byte granules (a TMA box starts 16-byte aligned)
+struct TileRect {
+    int bx0, wbytes;         // first source byte column (may be negative) and width in bytes
+    int ry0, nrows;          // first source row and row count
+    int rsel, box_rows;      // TMA box rows = M::kRowsMin + kRowsStep * rsel
+};
+template <class M>
+__device__ __forceinline__ TileRect tile_rect(int mnx, int mxx, int mny, int mxy) {
+    TileRect r;
+    r.bx0 = (3 * (mnx - M::kLo)) & ~15;
+    r.wbytes = ((3 * (mxx + M::kHi + 1) + 15) & ~15) - r.bx0;
+    r.ry0 = mny - M::kLo;
+    r.nrows = mxy + M::kHi + 1 - r.ry0;
+    r.rsel = box_rsel<M>(r.nrows);
+    r.box_rows = M::kRowsMin + r.rsel * kRowsStep;
+    return r;
+}
+
+// Row pitch of the staged rectangle (= TMA box width).  Candidates: the kPitchCands widths pitch0 + kPitchStep e.
+// Cost of a candidate in shared-memory wavefronts per (frame, eye) item: the tap loads (every sampling warp measures
+// the wavefronts = max distinct words per bank, counted with match.any, of the first tap load of its step k = 0; a
+// tile has kStepsPerWarp steps of kLoads loads with the same address pattern) + the TMA write of the box (64 bytes per
+// wavefront, measured).  pitch_costs: one sampling warp's share, added into s_cost[kPitchCands] (zeroed by the
+// caller); pick_pitch, after a barrier: the cheapest candidate that is <= kPitchMax and that `fits` admits.
+template <class M>
+__device__ __forceinline__ void pitch_costs(int sx0, int sy0, const TileRect& rc, int pitch0, int lane, int* s_cost) {
+    const int row = (sy0 >> M::kShift) - M::kLo - rc.ry0, col = 3 * ((sx0 >> M::kShift) - M::kLo) - rc.bx0;
+    int cost = 0;
+#pragma unroll
+    for (int e = 0; e < kPitchCands; ++e) {
+        const int w = (row * (pitch0 + kPitchStep * e) + col) >> 2;
+        const unsigned same = __match_any_sync(0xffffffffu, w);
+        const bool leader = (__ffs(same) - 1) == lane;  // one lane per distinct word
+        const unsigned lm = __ballot_sync(0xffffffffu, leader);
+        int deg = 0;
+        if (leader) deg = __popc(__match_any_sync(lm, w & 31));
+        deg = __reduce_max_sync(0xffffffffu, deg);
+        if (lane == e) cost = deg;
+    }
+    constexpr int kStepsPerWarp = M::kTileH * kTileW / kSamplers;  // warp steps (32 pixels) of a tile, per warp
+    constexpr int kLoads = M::kInterp == VR180_INTER_NEAREST ? 2 : M::kInterp == VR180_INTER_LINEAR ? 6
+                         : M::kInterp == VR180_INTER_CUBIC ? 16 : 56;
+    if (lane < kPitchCands) atomicAdd(&s_cost[lane], cost * (kStepsPerWarp * kLoads));
+}
+template <class Fits>
+__device__ __forceinline__ int pick_pitch(const int* s_cost, int pitch0, int box_rows, Fits fits) {
+    int best = 0, best_cost = INT_MAX;
+#pragma unroll
+    for (int e = 0; e < kPitchCands; ++e) {
+        const int pe = pitch0 + kPitchStep * e;
+        const int c = s_cost[e] + box_rows * pe / 64;
+        if (pe <= kPitchMax && fits(pe) && c < best_cost) { best_cost = c; best = e; }
+    }
+    return pitch0 + kPitchStep * best;
+}
+
+// Per-pixel gather from global memory with full border handling (the tiles that are not staged): one output pixel
+// (i, j) of frame f for the views v_begin .. v_end - 1, which share the quantised coordinates (qx, qy).
+template <class M>
+__device__ __forceinline__ void gather_pixel(const RemapArgs& a, int f, int i, int j, int v_begin, int v_end, int qx, int qy,
+                                             const short* tab) {
+    uint8_t* drow = a.dst + (long long)f * a.dst_frame_stride + (long long)j * a.dst_pitch;
+    for (int v = v_begin; v < v_end; ++v) {
+        const ViewArgs& vw = a.view[v];
+        Src s{vw.src + (long long)f * vw.frame_stride, vw.rows, vw.cols, vw.pitch};
+        int px[3];
+        if (M::kInterp == VR180_INTER_NEAREST)
+            fetch_tap<3>(s, sat16(qx), sat16(qy), a.border_mode, a.bv, px);
+        else if (M::kInterp == VR180_INTER_LINEAR)
+            sample_linear<3>(s, qx, qy, a.border_mode, a.bv, px);
+        else if (M::kInterp == VR180_INTER_CUBIC)
+            sample_tab<3, 4>(s, qx, qy, tab, a.border_mode, a.bv, px);
+        else
+            sample_tab<3, 8>(s, qx, qy, tab, a.border_mode, a.bv, px);
+        uint8_t* o = drow + (long long)(vw.dst_x_offset + i) * 3;
+        o[0] = (uint8_t)px[0];
+        o[1] = (uint8_t)px[1];
+        o[2] = (uint8_t)px[2];
+    }
+}
+
 // the FR frames of an item for one pixel; only modes with per-row state worth sharing implement sample_frames
 template <class M, int FR>
 __device__ __forceinline__ void sample_item(uint32_t sbuf, uint32_t frame_bytes, const typename M::Pixel& p, uint32_t pitch,
@@ -484,6 +564,24 @@ __device__ __forceinline__ void sample_item(uint32_t sbuf, uint32_t frame_bytes,
 #pragma unroll
         for (int f = 0; f < FR; ++f) out[f] = M::sample(sbuf + f * frame_bytes, p, pitch);
     }
+}
+
+// ---- host ----------------------------------------------------------------------------------------------------
+// BORDER_CONSTANT with a zero colour: TMA's out-of-bounds zero fill is the border
+inline int zero_border(const RemapArgs& a) {
+    return (a.border_mode == VR180_BORDER_CONSTANT && !(a.bv[0] | a.bv[1] | a.bv[2])) ? 1 : 0;
+}
+// The kernel's dynamic shared-memory limit, raised once per device; `dev` = the current device
+template <auto Kernel>
+int max_dyn_smem_once(int bytes, int& dev) {
+    static std::atomic<int> done[64];
+    dev = 0;
+    VR180_CUDA(cudaGetDevice(&dev));
+    if (dev < 64 && !done[dev].load(std::memory_order_acquire)) {
+        VR180_CUDA(cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes));
+        done[dev].store(1, std::memory_order_release);
+    }
+    return VR180_OK;
 }
 
 }  // namespace tiled
