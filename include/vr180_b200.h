@@ -99,13 +99,16 @@ typedef struct vr180_chain {
 } vr180_chain_t;
 
 /* ------------------------------------------------------------------------------------------------------
- * Images.  uint8, interleaved channels (HWC), rows may be strided (remapper.py:455-456 passes views).
- * A batch is `n_frames` images `frame_stride` bytes apart.
+ * Images.  uint8 or uint16 elements, interleaved channels (HWC), rows may be strided (remapper.py:455-456 passes
+ * views).  A batch is `n_frames` images `frame_stride` bytes apart.  `depth` uses OpenCV's depth codes; a zeroed field
+ * is 8-bit.  Pitches and strides stay in bytes for every depth.
  * ---------------------------------------------------------------------------------------------------- */
+enum { VR180_DEPTH_8U = 0, VR180_DEPTH_16U = 2 };
+
 typedef struct vr180_image {
     const uint8_t* data; /* device pointer to frame 0, row 0 */
     int32_t rows, cols, channels;
-    int32_t reserved;
+    int32_t depth;        /* VR180_DEPTH_8U or VR180_DEPTH_16U */
     int64_t pitch;        /* bytes between rows   */
     int64_t frame_stride; /* bytes between frames */
 } vr180_image_t;
@@ -154,8 +157,9 @@ typedef struct vr180_remap_params {
     int32_t out_w, out_h; /* per-view output size: size_output=(W,H), remapper.py:50 */
     int32_t interpolation; /* VR180_INTER_*  */
     int32_t border_mode;   /* VR180_BORDER_* */
-    uint8_t border_value[4]; /* per channel; a Python scalar v becomes {v,0,0,0} exactly like cv2 */
-    uint8_t* dst;            /* device, uint8 HWC, same channel count as the sources */
+    uint8_t border_value[4]; /* per channel; a Python scalar v becomes {v,0,0,0} exactly like cv2 (8-bit colours; see
+                                vr180_remap_ex for a full-range colour) */
+    uint8_t* dst;            /* device, HWC, same channel count and depth (view[0].src.depth) as the sources */
     int64_t dst_pitch;        /* bytes between destination rows (SBS: >= 2*W*C) */
     int64_t dst_frame_stride; /* bytes between destination frames */
 } vr180_remap_params_t;
@@ -214,7 +218,8 @@ int vr180_pack_lut_tiles(const float* xmap_dev, const float* ymap_dev, int64_t m
 /* ------------------------------------------------------------------------------------------------------
  * (2b) remap / fused warp + SBS packing -- replaces cv.remap per image (remapper.py:388-398) and
  *      np.concatenate(axis=1) (remapper.py:518): each view is written straight into its column range of the
- *      destination frame.  uint8, 1/3/4 channels.  Bit-exact to cv2.remap for the same float32 maps.
+ *      destination frame.  uint8 (16-bit: vr180_remap_ex), 1/3/4 channels.  Bit-exact to cv2.remap for the same
+ *      float32 maps.
  *      Performance note (results are identical either way): the TMA-tiled kernel serves 3 channels, NEAREST /
  *      LINEAR / CUBIC / LANCZOS4 (NEAREST not with a MAPSRC_FIXED LUT, which stores x * 32) when every base pointer, row
  *      pitch and frame stride is a multiple of 16 bytes and every view's dst_x_offset * 3 is too (a TMA box must start at
@@ -224,13 +229,21 @@ int vr180_pack_lut_tiles(const float* xmap_dev, const float* ymap_dev, int64_t m
  *      other request runs in the generic per-pixel kernel.
  * ---------------------------------------------------------------------------------------------------- */
 int vr180_remap(const vr180_remap_params_t* params, void* stream);
+/* vr180_remap with the border colour given as the cv::Scalar the reference passes (borderValue): the library saturates
+ * each entry to the depth of the images (round half to even, clamp), as cv2 does.  NULL = use params->border_value.
+ * 16-bit images (src.depth = VR180_DEPTH_16U for every view; the destination has the same depth) follow cv::remap's
+ * float-weight arithmetic for non-8-bit depths and are bit-exact to cv2.remap on uint16 images; they run in the generic
+ * per-pixel kernel (base pointers, pitches and strides 2-byte aligned).  Any other depth, or views of different depths,
+ * is VR180_ERR_UNSUPPORTED. */
+int vr180_remap_ex(const vr180_remap_params_t* params, const double border_scalar[4], void* stream);
 
 /* ------------------------------------------------------------------------------------------------------
  * (3) get_radius -- replaces transformer.py:108-140 for a batch.  For frame f and view v it scans the centre
  *     row (cols > rows) or centre column (otherwise) and writes
  *        transitions_dev[(f*n_views+v)*2 + 0] = first k with !black[k] && black[k+1]   (or -1)
  *        transitions_dev[(f*n_views+v)*2 + 1] = last  k with  black[k] && !black[k+1]  (or -1)
- *     with black[k] <=> mean_c px[k][c] < threshold (float64, as np.mean does).  If radius_dev is non-NULL it also writes
+ *     with black[k] <=> mean_c px[k][c] < threshold (float64, as np.mean does; 8- or 16-bit elements per views[v].depth,
+ *     every view of one call with the same depth).  If radius_dev is non-NULL it also writes
  *        radius_dev[f] = max_v (last - first) / 2          (remapper.py:82-84, "auto")
  *     as float64, NaN when any view of the frame lacks a transition (the reference raises IndexError; the
  *     Python layer re-raises it from the -1 sentinels).
@@ -297,7 +310,7 @@ typedef struct vr180_host_job {
     /* host source frames: view v, frame f at src[v] + f*src_frame_stride[v]; same geometry rules as vr180_image_t */
     const uint8_t* src[2];
     int32_t src_rows, src_cols, channels;
-    int32_t reserved0;
+    int32_t depth; /* VR180_DEPTH_8U (0) or VR180_DEPTH_16U, for the sources and the destination alike */
     int64_t src_pitch[2];
     int64_t src_frame_stride[2];
     /* coordinate source per view.  ANALYTIC: chain (host).  FLOAT2: HOST float32 maps, uploaded once per call and
@@ -335,7 +348,7 @@ typedef struct vr180_host_job {
        staging: VR180_STAGE_AUTO = per buffer, decided with cudaPointerGetAttributes; ALWAYS / NEVER force it. */
     int32_t staging;
     int32_t copy_threads;
-    /* merge != 0 (n_views == 2, 3 channels): vr180_anaglyph runs on the device SBS frame and the destination frames
+    /* merge != 0 (n_views == 2, 3 channels, 8-bit): vr180_anaglyph runs on the device SBS frame and the destination frames
        are the merged (out_h, out_w, 3) images -- half the download, no host pass (apply_lr(merge=True)). */
     int32_t merge;
     int32_t reserved2;
@@ -345,6 +358,9 @@ enum { VR180_STAGE_AUTO = 0, VR180_STAGE_ALWAYS = 1, VR180_STAGE_NEVER = 2 };
 
 /* Synchronous: returns when every destination frame is complete in host memory. */
 int vr180_ctx_run(vr180_ctx_t* ctx, const vr180_host_job_t* job);
+/* vr180_ctx_run with the border colour as a cv::Scalar saturated to job->depth (see vr180_remap_ex); NULL = use
+ * job->border_value. */
+int vr180_ctx_run_ex(vr180_ctx_t* ctx, const vr180_host_job_t* job, const double border_scalar[4]);
 
 /* ------------------------------------------------------------------------------------------------------
  * Test / profiling hooks (not part of the drop-in surface; no reference counterpart).

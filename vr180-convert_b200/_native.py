@@ -20,6 +20,7 @@ OP_EQUIRECT_ENC, OP_EQUIRECT_DEC, OP_FISHEYE_ENC, OP_FISHEYE_DEC = 6, 7, 8, 9
 OP_RECTILINEAR_DEC, OP_RECTILINEAR_DEC_INV, OP_POLY, OP_ROT3 = 10, 11, 12, 13
 MAPPING_CODES = {"rectilinear": 0, "stereographic": 1, "equidistant": 2, "equisolid": 3, "orthographic": 4}
 MAPSRC_ANALYTIC, MAPSRC_FLOAT2, MAPSRC_FIXED, MAPSRC_PACKED = 0, 1, 2, 3
+DEPTH_8U, DEPTH_16U = 0, 2  # OpenCV's depth codes (vr180_image_t.depth, vr180_host_job_t.depth)
 
 
 class NativeError(RuntimeError):
@@ -36,7 +37,7 @@ class Chain(C.Structure):
 
 class Image(C.Structure):
     _fields_ = [("data", C.c_void_p), ("rows", C.c_int32), ("cols", C.c_int32), ("channels", C.c_int32),
-                ("reserved", C.c_int32), ("pitch", C.c_int64), ("frame_stride", C.c_int64)]
+                ("depth", C.c_int32), ("pitch", C.c_int64), ("frame_stride", C.c_int64)]
 
 
 class MapSrc(C.Structure):
@@ -58,7 +59,7 @@ class RemapParams(C.Structure):
 
 class HostJob(C.Structure):
     _fields_ = [("n_views", C.c_int32), ("n_frames", C.c_int32), ("src", C.c_void_p * 2), ("src_rows", C.c_int32),
-                ("src_cols", C.c_int32), ("channels", C.c_int32), ("reserved0", C.c_int32),
+                ("src_cols", C.c_int32), ("channels", C.c_int32), ("depth", C.c_int32),
                 ("src_pitch", C.c_int64 * 2), ("src_frame_stride", C.c_int64 * 2), ("map_kind", C.c_int32),
                 ("share_map", C.c_int32), ("chain", C.POINTER(Chain) * 2), ("xmap", C.c_void_p * 2),
                 ("ymap", C.c_void_p * 2), ("maps_cache_key", C.c_uint64), ("radius_mode", C.c_int32),
@@ -85,6 +86,7 @@ SYMBOLS = {
     "vr180_pack_lut_tiles": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                        C.c_void_p]),
     "vr180_remap": (C.c_int, [C.POINTER(RemapParams), C.c_void_p]),
+    "vr180_remap_ex": (C.c_int, [C.POINTER(RemapParams), C.POINTER(C.c_double), C.c_void_p]),
     "vr180_anaglyph": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int64,
                                  C.c_int64, C.c_void_p]),
     "vr180_transform_points": (C.c_int, [C.POINTER(Chain), C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
@@ -104,6 +106,7 @@ SYMBOLS = {
     "vr180_host_register": (C.c_int, [C.c_void_p, C.c_size_t]),
     "vr180_host_unregister": (C.c_int, [C.c_void_p]),
     "vr180_ctx_run": (C.c_int, [C.c_void_p, C.POINTER(HostJob)]),
+    "vr180_ctx_run_ex": (C.c_int, [C.c_void_p, C.POINTER(HostJob), C.POINTER(C.c_double)]),
     "vr180_debug_weight_table": (C.c_int, [C.c_int, C.c_void_p]),
     "vr180_debug_set": (C.c_int, [C.c_int, C.c_int]),
     "vr180_debug_copy_ceiling": (C.c_int, [C.c_int, C.c_size_t, C.c_int, C.POINTER(C.c_double)]),

@@ -124,7 +124,14 @@ int vr180_remap(const vr180_remap_params_t* params, void* stream) {
     if (!params || !params->dst) return VR180_ERR_INVALID_ARG;
     DeviceGuard g(params->dst);
     if (!g.ok) return VR180_ERR_INVALID_ARG;
-    return launch_remap(params, (cudaStream_t)stream);
+    return launch_remap(params, nullptr, (cudaStream_t)stream);
+}
+
+int vr180_remap_ex(const vr180_remap_params_t* params, const double border_scalar[4], void* stream) {
+    if (!params || !params->dst) return VR180_ERR_INVALID_ARG;
+    DeviceGuard g(params->dst);
+    if (!g.ok) return VR180_ERR_INVALID_ARG;
+    return launch_remap(params, border_scalar, (cudaStream_t)stream);
 }
 
 int vr180_anaglyph(const uint8_t* sbs_dev, int64_t sbs_pitch, int64_t sbs_frame_stride, int eye_w, int h, int n_frames,

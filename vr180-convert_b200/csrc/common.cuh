@@ -78,17 +78,28 @@ struct RemapArgs {
     int W, H;
     int border_mode;
     uint8_t bv[4];
+    int depth;  // VR180_DEPTH_8U / VR180_DEPTH_16U, sources and destination alike (fills the padding before dst)
     uint8_t* dst;
     long long dst_pitch, dst_frame_stride;
     int frames_per_cta;
 };
+
+// What 16-bit requests add: a trailing kernel parameter, so that RemapArgs keeps its size and the parameters after it
+// their offsets in the 8-bit kernels.
+struct Remap16 {
+    float cval[4];      // border colour saturated to 16 bits (exact in float)
+    const float* ftab;  // float weight table of CUBIC / LANCZOS4 (generic kernel)
+};
+
+inline int depth_bytes(int depth) { return depth == VR180_DEPTH_16U ? 2 : 1; }
 
 // internal launchers (kernels.cu); the device is already selected by the caller
 int launch_build_map(const vr180_chain_t* chain, int out_w, int out_h, float* xmap, float* ymap, int64_t pitch,
                      cudaStream_t st);
 int launch_pack_lut(const float* xmap, const float* ymap, int64_t map_pitch, int out_w, int out_h, int32_t* fixed,
                     int64_t fixed_pitch, cudaStream_t st);
-int launch_remap(const vr180_remap_params_t* p, cudaStream_t st);
+// border_scalar: the cv::Scalar border colour, saturated to the depth here; nullptr = p->border_value
+int launch_remap(const vr180_remap_params_t* p, const double* border_scalar, cudaStream_t st);
 size_t packed_lut_bytes(int out_w, int out_h, int interp);  // tiled.cu; 0 = interpolation without a tiled mode
 int launch_pack_lut_tiles(const float* xmap, const float* ymap, int64_t map_pitch, int out_w, int out_h, int interp,
                           void* packed, cudaStream_t st);

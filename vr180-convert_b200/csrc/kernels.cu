@@ -6,6 +6,7 @@
 //                 straight into the SBS frame, a batch of frames per launch
 //                                                                (cv.remap remapper.py:388-398 + concatenate :518)
 //   k_get_radius  black-pixel transition scan                    (get_radius, transformer.py:108-140)
+#include <cmath>
 #include <cstdlib>
 #include <mutex>
 #include <vector>
@@ -48,6 +49,32 @@ static int ensure_tables(cudaStream_t st) {
     VR180_CUDA(cudaMemcpyToSymbol(g_tab_cubic, c.data(), c.size() * sizeof(int16_t)));
     VR180_CUDA(cudaMemcpyToSymbol(g_tab_lanczos, l.data(), l.size() * sizeof(int16_t)));
     if (dev < 64) g_tab_on_device[dev] = true;
+    return VR180_OK;
+}
+
+// The float tables of 16-bit CUBIC (1024 x 16) and LANCZOS4 (1024 x 64) in device global memory, built on the host once
+// and uploaded once per device; they live as long as the process.
+static const float* g_ftab_dev[64][2] = {};
+
+static int ensure_float_table(int K, const float** out) {
+    int dev = 0;
+    VR180_CUDA(cudaGetDevice(&dev));
+    if (dev >= 64) return VR180_ERR_UNSUPPORTED;
+    std::lock_guard<std::mutex> lock(g_tab_mutex);
+    const float*& slot = g_ftab_dev[dev][K == 4 ? 0 : 1];
+    if (!slot) {
+        const std::vector<float> t = build_float_table(K);
+        void* p = nullptr;
+        VR180_CUDA(cudaMalloc(&p, t.size() * sizeof(float)));
+        const cudaError_t e = cudaMemcpy(p, t.data(), t.size() * sizeof(float), cudaMemcpyHostToDevice);  // once
+        if (e != cudaSuccess) {
+            cudaFree(p);
+            set_cuda_error(e, "cudaMemcpy(float weight table)");
+            return VR180_ERR_CUDA;
+        }
+        slot = static_cast<const float*>(p);
+    }
+    *out = slot;
     return VR180_OK;
 }
 
@@ -111,12 +138,26 @@ __device__ __forceinline__ void sample_and_store(const Src& s, int sx, int sy, f
     for (int c = 0; c < C; ++c) out[c] = (uint8_t)px[c];
 }
 
+template <int C, int INTERP>
+__device__ __forceinline__ void sample_and_store16(const Src& s, int sx, int sy, float mx, float my, int border_mode,
+                                                   const float* cval, const float* ftab, uint16_t* __restrict__ out) {
+    int px[C];
+    if (INTERP == VR180_INTER_NEAREST) sample16_nearest<C>(s, mx, my, border_mode, cval, px);
+    else if (INTERP == VR180_INTER_LINEAR) sample16_linear<C>(s, sx, sy, border_mode, cval, px);
+    else if (INTERP == VR180_INTER_CUBIC) sample16_tab<C, 4>(s, sx, sy, ftab, border_mode, cval, px);
+    else sample16_tab<C, 8>(s, sx, sy, ftab, border_mode, cval, px);
+#pragma unroll
+    for (int c = 0; c < C; ++c) out[c] = (uint16_t)px[c];
+}
+
 // One thread = one output pixel of the tile; coordinates are evaluated once and reused for every frame of the
 // CTA's frame chunk (and for both eyes when they share a map).  grid = (tiles_x, tiles_y, frame_chunks).
-template <int C, int INTERP>
+// T = uint8_t (OpenCV's fixed-point 8-bit arithmetic) or uint16_t (its float arithmetic for other depths).
+template <typename T, int C, int INTERP>
 __global__ void __launch_bounds__(256) k_remap(const __grid_constant__ RemapArgs a,
                                                const __grid_constant__ vr180_chain_t chain0,
-                                               const __grid_constant__ vr180_chain_t chain1) {
+                                               const __grid_constant__ vr180_chain_t chain1,
+                                               const __grid_constant__ Remap16 x16) {
     const int i = blockIdx.x * blockDim.x + threadIdx.x;
     const int j = blockIdx.y * blockDim.y + threadIdx.y;
     if (i >= a.W || j >= a.H) return;
@@ -169,22 +210,42 @@ __global__ void __launch_bounds__(256) k_remap(const __grid_constant__ RemapArgs
             for (int v = v_begin; v < v_end; ++v) {
                 const ViewArgs& vw = a.view[v];
                 Src s{vw.src + (long long)f * vw.frame_stride, vw.rows, vw.cols, vw.pitch};
-                sample_and_store<C, INTERP>(s, sx, sy, mx, my, a.border_mode, a.bv,
-                                            drow + (long long)(vw.dst_x_offset + i) * C);
+                if constexpr (sizeof(T) == 1) {
+                    sample_and_store<C, INTERP>(s, sx, sy, mx, my, a.border_mode, a.bv,
+                                                drow + (long long)(vw.dst_x_offset + i) * C);
+                } else {
+                    sample_and_store16<C, INTERP>(s, sx, sy, mx, my, a.border_mode, x16.cval, x16.ftab,
+                                                  reinterpret_cast<uint16_t*>(drow) + (long long)(vw.dst_x_offset + i) * C);
+                }
             }
         }
     }
 }
 
-template <int C>
+template <typename T, int C>
 static void dispatch_interp(int interp, dim3 grid, dim3 block, cudaStream_t st, const RemapArgs& a,
-                            const vr180_chain_t& c0, const vr180_chain_t& c1) {
+                            const vr180_chain_t& c0, const vr180_chain_t& c1, const Remap16& x) {
     switch (interp) {
-        case VR180_INTER_NEAREST: k_remap<C, VR180_INTER_NEAREST><<<grid, block, 0, st>>>(a, c0, c1); break;
-        case VR180_INTER_LINEAR: k_remap<C, VR180_INTER_LINEAR><<<grid, block, 0, st>>>(a, c0, c1); break;
-        case VR180_INTER_CUBIC: k_remap<C, VR180_INTER_CUBIC><<<grid, block, 0, st>>>(a, c0, c1); break;
-        default: k_remap<C, VR180_INTER_LANCZOS4><<<grid, block, 0, st>>>(a, c0, c1); break;
+        case VR180_INTER_NEAREST: k_remap<T, C, VR180_INTER_NEAREST><<<grid, block, 0, st>>>(a, c0, c1, x); break;
+        case VR180_INTER_LINEAR: k_remap<T, C, VR180_INTER_LINEAR><<<grid, block, 0, st>>>(a, c0, c1, x); break;
+        case VR180_INTER_CUBIC: k_remap<T, C, VR180_INTER_CUBIC><<<grid, block, 0, st>>>(a, c0, c1, x); break;
+        default: k_remap<T, C, VR180_INTER_LANCZOS4><<<grid, block, 0, st>>>(a, c0, c1, x); break;
     }
+}
+
+template <typename T>
+static void dispatch_channels(int C, int interp, dim3 grid, dim3 block, cudaStream_t st, const RemapArgs& a,
+                              const vr180_chain_t& c0, const vr180_chain_t& c1, const Remap16& x) {
+    if (C == 3) dispatch_interp<T, 3>(interp, grid, block, st, a, c0, c1, x);
+    else if (C == 1) dispatch_interp<T, 1>(interp, grid, block, st, a, c0, c1, x);
+    else dispatch_interp<T, 4>(interp, grid, block, st, a, c0, c1, x);
+}
+
+// saturate_cast<uchar / ushort>(double): round half to even, clamp (NaN -> 0, as cvRound gives INT_MIN)
+static int saturate_scalar(double v, int maxval) {
+    if (!(v == v)) return 0;
+    const double r = std::nearbyint(v);
+    return r <= 0.0 ? 0 : (r >= (double)maxval ? maxval : (int)r);
 }
 
 int validate_chain(const vr180_chain_t* c) {
@@ -200,7 +261,7 @@ int validate_chain(const vr180_chain_t* c) {
     return VR180_OK;
 }
 
-int launch_remap(const vr180_remap_params_t* p, cudaStream_t st) {
+int launch_remap(const vr180_remap_params_t* p, const double* border_scalar, cudaStream_t st) {
     if (p->n_views < 1 || p->n_views > 2 || p->n_frames < 0 || p->out_w <= 0 || p->out_h <= 0 || !p->dst)
         return VR180_ERR_INVALID_ARG;
     if (p->n_frames == 0) return VR180_OK;
@@ -211,6 +272,10 @@ int launch_remap(const vr180_remap_params_t* p, cudaStream_t st) {
     if (p->border_mode < VR180_BORDER_CONSTANT || p->border_mode > VR180_BORDER_REFLECT_101) return VR180_ERR_UNSUPPORTED;
     const int C = p->view[0].src.channels;
     if (C != 1 && C != 3 && C != 4) return VR180_ERR_UNSUPPORTED;
+    const int depth = p->view[0].src.depth;
+    if (depth != VR180_DEPTH_8U && depth != VR180_DEPTH_16U) return VR180_ERR_UNSUPPORTED;
+    if (depth == VR180_DEPTH_16U && (((uintptr_t)p->dst | (uintptr_t)p->dst_pitch | (uintptr_t)p->dst_frame_stride) & 1))
+        return VR180_ERR_INVALID_ARG;  // uint16 elements must be 2-byte aligned
 
     RemapArgs a;
     memset(&a, 0, sizeof(a));
@@ -219,6 +284,10 @@ int launch_remap(const vr180_remap_params_t* p, cudaStream_t st) {
     for (int v = 0; v < p->n_views; ++v) {
         const vr180_view_t& vw = p->view[v];
         if (!vw.src.data || vw.src.rows <= 0 || vw.src.cols <= 0 || vw.src.channels != C) return VR180_ERR_INVALID_ARG;
+        if (vw.src.depth != depth) return VR180_ERR_UNSUPPORTED;
+        if (depth == VR180_DEPTH_16U &&
+            (((uintptr_t)vw.src.data | (uintptr_t)vw.src.pitch | (uintptr_t)vw.src.frame_stride) & 1))
+            return VR180_ERR_INVALID_ARG;
         ViewArgs& o = a.view[v];
         o.src = vw.src.data;
         o.rows = vw.src.rows;
@@ -265,13 +334,20 @@ int launch_remap(const vr180_remap_params_t* p, cudaStream_t st) {
     a.W = p->out_w;
     a.H = p->out_h;
     a.border_mode = p->border_mode;
-    memcpy(a.bv, p->border_value, 4);
+    a.depth = depth;
+    Remap16 x16;
+    memset(&x16, 0, sizeof(x16));
+    for (int c = 0; c < 4; ++c) {
+        a.bv[c] = border_scalar ? (uint8_t)saturate_scalar(border_scalar[c], 255) : p->border_value[c];
+        x16.cval[c] = border_scalar ? (float)saturate_scalar(border_scalar[c], 65535) : (float)p->border_value[c];
+    }
     a.dst = p->dst;
     a.dst_pitch = p->dst_pitch;
     a.dst_frame_stride = p->dst_frame_stride;
 
     if (interp == VR180_INTER_CUBIC || interp == VR180_INTER_LANCZOS4) {
-        const int rc = ensure_tables(st);
+        const int rc = depth == VR180_DEPTH_16U ? ensure_float_table(interp == VR180_INTER_CUBIC ? 4 : 8, &x16.ftab)
+                                                : ensure_tables(st);
         if (rc != VR180_OK) return rc;
     }
 
@@ -294,9 +370,8 @@ int launch_remap(const vr180_remap_params_t* p, cudaStream_t st) {
     dim3 grid((a.W + 31) / 32, (a.H + 7) / 8, (a.n_frames + fpc - 1) / fpc);
     if (grid.z > 65535) return VR180_ERR_UNSUPPORTED;
 
-    if (C == 3) dispatch_interp<3>(interp, grid, block, st, a, *chains[0], *chains[1]);
-    else if (C == 1) dispatch_interp<1>(interp, grid, block, st, a, *chains[0], *chains[1]);
-    else dispatch_interp<4>(interp, grid, block, st, a, *chains[0], *chains[1]);
+    if (depth == VR180_DEPTH_16U) dispatch_channels<uint16_t>(C, interp, grid, block, st, a, *chains[0], *chains[1], x16);
+    else dispatch_channels<uint8_t>(C, interp, grid, block, st, a, *chains[0], *chains[1], x16);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     VR180_CUDA(cudaGetLastError());
     return VR180_OK;
@@ -311,12 +386,16 @@ struct RadiusArgs {
     double threshold;
 };
 
-__device__ __forceinline__ bool is_black(const uint8_t* __restrict__ px, int C, double threshold) {
+template <typename T>
+__device__ __forceinline__ bool is_black(const uint8_t* __restrict__ p, int C, double threshold) {
+    const T* px = reinterpret_cast<const T*>(p);
     int sum = 0;
     for (int c = 0; c < C; ++c) sum += __ldg(px + c);
     return __ddiv_rn((double)sum, (double)C) < threshold;  // np.mean(center_row, axis=-1) < threshold, transformer.py:133
 }
 
+// T: the element type of every view (uint8_t / uint16_t); pixel offsets below are in bytes
+template <typename T>
 __global__ void __launch_bounds__(256) k_get_radius(const __grid_constant__ RadiusArgs a, int* __restrict__ transitions,
                                                     double* __restrict__ radius) {
     __shared__ int s_pos[8], s_neg[8];
@@ -332,17 +411,17 @@ __global__ void __launch_bounds__(256) k_get_radius(const __grid_constant__ Radi
         int n;
         if (im.cols > im.rows) {  // centre row, transformer.py:126-127
             base += (long long)(im.rows / 2) * im.pitch;
-            step = C;
+            step = C * (long long)sizeof(T);
             n = im.cols;
         } else {  // centre column (also for square images), :128-129
-            base += (long long)(im.cols / 2) * C;
+            base += (long long)(im.cols / 2) * C * (long long)sizeof(T);
             step = im.pitch;
             n = im.rows;
         }
         int pos = INT_MAX, neg = -1;
         for (int k = threadIdx.x; k < n - 1; k += blockDim.x) {
-            const bool b0 = is_black(base + (long long)k * step, C, a.threshold);
-            const bool b1 = is_black(base + (long long)(k + 1) * step, C, a.threshold);
+            const bool b0 = is_black<T>(base + (long long)k * step, C, a.threshold);
+            const bool b1 = is_black<T>(base + (long long)(k + 1) * step, C, a.threshold);
             if (!b0 && b1) pos = min(pos, k);  // np.diff(...) == +1, first index (:137)
             if (b0 && !b1) neg = max(neg, k);  // np.diff(...) == -1, last index  (:138)
         }
@@ -385,11 +464,17 @@ int launch_get_radius(const vr180_image_t* views, int n_views, int n_frames, dou
     for (int v = 0; v < n_views; ++v) {
         if (!views[v].data || views[v].rows <= 0 || views[v].cols <= 0 || views[v].channels < 1 || views[v].channels > 4)
             return VR180_ERR_INVALID_ARG;
+        if (views[v].depth != views[0].depth || (views[v].depth != VR180_DEPTH_8U && views[v].depth != VR180_DEPTH_16U))
+            return VR180_ERR_UNSUPPORTED;
+        if (views[v].depth == VR180_DEPTH_16U &&
+            (((uintptr_t)views[v].data | (uintptr_t)views[v].pitch | (uintptr_t)views[v].frame_stride) & 1))
+            return VR180_ERR_INVALID_ARG;
         a.view[v] = views[v];
     }
     a.n_views = n_views;
     a.threshold = threshold;
-    k_get_radius<<<n_frames, 256, 0, st>>>(a, transitions, radius);
+    if (views[0].depth == VR180_DEPTH_16U) k_get_radius<uint16_t><<<n_frames, 256, 0, st>>>(a, transitions, radius);
+    else k_get_radius<uint8_t><<<n_frames, 256, 0, st>>>(a, transitions, radius);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     VR180_CUDA(cudaGetLastError());
     return VR180_OK;

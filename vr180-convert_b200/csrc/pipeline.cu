@@ -374,8 +374,9 @@ int vr180_ctx_device(const vr180_ctx_t* c) { return c ? c->device : -1; }
 
 // The body of vr180_ctx_run after argument validation; every failure after the first enqueue returns through the
 // caller, which drains all three streams and the drain thread before the job's buffers may be released.
-static int ctx_run_locked(vr180_ctx* c, const vr180_host_job_t* job) {
-    const int V = job->n_views, F = job->n_frames, C = job->channels;
+static int ctx_run_locked(vr180_ctx* c, const vr180_host_job_t* job, const double* border_scalar) {
+    // C: bytes per pixel (channels x element size); every size below is in bytes
+    const int V = job->n_views, F = job->n_frames, C = job->channels * depth_bytes(job->depth);
     const bool scattered = job->src_frames[0] != nullptr;
     const size_t src_row = (size_t)job->src_cols * C, src_pitch = align_up(src_row, 16);
     const size_t src_frame = src_pitch * job->src_rows;
@@ -543,7 +544,8 @@ static int ctx_run_locked(vr180_ctx* c, const vr180_host_job_t* job) {
             vw.src.data = (const uint8_t*)sl.src[v].p;
             vw.src.rows = job->src_rows;
             vw.src.cols = job->src_cols;
-            vw.src.channels = C;
+            vw.src.channels = job->channels;
+            vw.src.depth = job->depth;
             vw.src.pitch = (int64_t)src_pitch;
             vw.src.frame_stride = (int64_t)src_frame;
             vw.dst_x_offset = v ? (int)eye1_col : 0;
@@ -563,7 +565,7 @@ static int ctx_run_locked(vr180_ctx* c, const vr180_host_job_t* job) {
             rc = launch_get_radius(im, V, nf, job->threshold, (int32_t*)c->trans.p + (size_t)2 * V * f0, rad, c->s_comp);
             if (rc != VR180_OK) return rc;
         }
-        rc = launch_remap(&p, c->s_comp);
+        rc = launch_remap(&p, border_scalar, c->s_comp);
         if (rc != VR180_OK) return rc;
         if (merge) {
             rc = launch_anaglyph((const uint8_t*)sl.dst.p, (int64_t)dst_pitch, (int64_t)dst_frame, job->out_w, (int)eye1_col,
@@ -622,12 +624,17 @@ static int ctx_run_locked(vr180_ctx* c, const vr180_host_job_t* job) {
     return VR180_OK;
 }
 
-int vr180_ctx_run(vr180_ctx_t* c, const vr180_host_job_t* job) {
+int vr180_ctx_run(vr180_ctx_t* c, const vr180_host_job_t* job) { return vr180_ctx_run_ex(c, job, nullptr); }
+
+int vr180_ctx_run_ex(vr180_ctx_t* c, const vr180_host_job_t* job, const double border_scalar[4]) {
     if (!c || !job || (!job->dst && !job->dst_frames)) return VR180_ERR_INVALID_ARG;
-    const int V = job->n_views, F = job->n_frames, C = job->channels;
+    const int V = job->n_views, F = job->n_frames, ch = job->channels;
     if (V < 1 || V > 2 || F < 0 || job->src_rows <= 0 || job->src_cols <= 0 || job->out_w <= 0 || job->out_h <= 0)
         return VR180_ERR_INVALID_ARG;
-    if (C != 1 && C != 3 && C != 4) return VR180_ERR_UNSUPPORTED;
+    if (ch != 1 && ch != 3 && ch != 4) return VR180_ERR_UNSUPPORTED;
+    if (job->depth != VR180_DEPTH_8U && job->depth != VR180_DEPTH_16U) return VR180_ERR_UNSUPPORTED;
+    if (job->merge && job->depth != VR180_DEPTH_8U) return VR180_ERR_UNSUPPORTED;  // the anaglyph is 8-bit
+    const int C = ch * depth_bytes(job->depth);  // bytes per pixel
     const bool scattered = job->src_frames[0] != nullptr;
     for (int v = 0; v < V; ++v) {
         if (scattered ? !job->src_frames[v] : !job->src[v]) return VR180_ERR_INVALID_ARG;
@@ -637,7 +644,7 @@ int vr180_ctx_run(vr180_ctx_t* c, const vr180_host_job_t* job) {
     }
     for (int f = 0; job->dst_frames && f < F; ++f)
         if (!job->dst_frames[f]) return VR180_ERR_INVALID_ARG;
-    if (job->merge && (V != 2 || C != 3)) return VR180_ERR_INVALID_ARG;
+    if (job->merge && (V != 2 || ch != 3)) return VR180_ERR_INVALID_ARG;
     if ((size_t)job->dst_pitch < (size_t)job->out_w * (job->merge ? 1 : V) * C) return VR180_ERR_INVALID_ARG;
     if (job->map_kind != VR180_MAPSRC_ANALYTIC && job->map_kind != VR180_MAPSRC_FLOAT2) return VR180_ERR_UNSUPPORTED;
     if (job->radius_mode == 1 && job->map_kind != VR180_MAPSRC_ANALYTIC) return VR180_ERR_UNSUPPORTED;
@@ -647,7 +654,7 @@ int vr180_ctx_run(vr180_ctx_t* c, const vr180_host_job_t* job) {
     std::lock_guard<std::mutex> lock(c->mu);
     DeviceGuard g(c->device);
     if (!g.ok) return VR180_ERR_CUDA;
-    const int rc = ctx_run_locked(c, job);
+    const int rc = ctx_run_locked(c, job, border_scalar);
     // One exit for success and failure alike: nothing of this job may still be in flight when the caller gets its
     // buffers back (copies and kernels of earlier chunks read job->src / write job->dst asynchronously).
     const cudaError_t e0 = cudaStreamSynchronize(c->s_h2d), e1 = cudaStreamSynchronize(c->s_comp),

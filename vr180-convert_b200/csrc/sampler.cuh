@@ -1,4 +1,4 @@
-// sampler.cuh -- OpenCV-exact coordinate quantisation and uint8 gather (device side).
+// sampler.cuh -- OpenCV-exact coordinate quantisation and uint8 / uint16 gather (device side).
 //
 // Replaces the inside of cv::remap as called at /root/reference/src/vr180_convert/remapper.py:388-398.
 // OpenCV is a third-party dependency of the reference (opencv-python 4.10.0.82 pinned, poetry.lock:1014-1015);
@@ -212,6 +212,136 @@ __device__ __forceinline__ void sample_tab(const Src& s, int sx, int sy, const s
     }
 #pragma unroll
     for (int c = 0; c < C; ++c) out[c] = max(0, min(255, (acc[c] + 16384) >> 15));
+}
+
+// ---------------------------------------------------------------------------------------------------------
+// 16-bit images: cv::remap's float-weight arithmetic for non-8-bit depths (remapBilinear / remapBicubic /
+// remapLanczos4, restated in oracle/remap_float_np.py).  Src.p / pitch stay in bytes; elements are uint16.  Every
+// product and sum is one float32 operation (__fmul_rn / __fadd_rn: no contraction into FMA), in OpenCV's order, and
+// the result is saturate(cvRound(s)).  `cval` is the border colour as float (a uint16 converts exactly).
+// ---------------------------------------------------------------------------------------------------------
+template <int C>
+__device__ __forceinline__ const uint16_t* px16(const Src& s, int x, int y) {
+    return reinterpret_cast<const uint16_t*>(s.p + (long long)y * s.pitch) + (long long)x * C;
+}
+__device__ __forceinline__ int sat_u16(float v) { return max(0, min(65535, __float2int_rn(v))); }
+
+template <int C>
+__device__ __forceinline__ void sample16_nearest(const Src& s, float mx, float my, int border_mode, const float* cval,
+                                                 int* out) {
+    const int ix = sat16(cv_round(mx)), iy = sat16(cv_round(my));
+    if (border_mode == VR180_BORDER_CONSTANT && !((unsigned)ix < (unsigned)s.cols && (unsigned)iy < (unsigned)s.rows)) {
+#pragma unroll
+        for (int c = 0; c < C; ++c) out[c] = (int)cval[c];
+        return;
+    }
+    const uint16_t* q = px16<C>(s, border_index(ix, s.cols, border_mode), border_index(iy, s.rows, border_mode));
+#pragma unroll
+    for (int c = 0; c < C; ++c) out[c] = __ldg(q + c);
+}
+
+// One bilinear tap as float: the pixel, or under BORDER_CONSTANT the border colour outside the source.
+template <int C>
+__device__ __forceinline__ void tap16(const Src& s, int x, int y, int border_mode, const float* cval, float* v) {
+    if (border_mode == VR180_BORDER_CONSTANT && !((unsigned)x < (unsigned)s.cols && (unsigned)y < (unsigned)s.rows)) {
+#pragma unroll
+        for (int c = 0; c < C; ++c) v[c] = cval[c];
+        return;
+    }
+    const uint16_t* q = px16<C>(s, border_index(x, s.cols, border_mode), border_index(y, s.rows, border_mode));
+#pragma unroll
+    for (int c = 0; c < C; ++c) v[c] = (float)__ldg(q + c);
+}
+
+// INTER_LINEAR: w = float((1 - ty or ty) * (1 - tx or tx)) = (32-ay or ay)(32-ax or ax) / 1024 exactly;
+// s = ((v00 w00 + v01 w01) + v10 w10) + v11 w11.  A footprint entirely outside under BORDER_CONSTANT is cval itself.
+template <int C>
+__device__ __forceinline__ void sample16_linear(const Src& s, int sx, int sy, int border_mode, const float* cval,
+                                                int* out) {
+    const int ix = sat16(sx >> kInterBits), iy = sat16(sy >> kInterBits);
+    const int ax = sx & 31, ay = sy & 31;
+    const float w00 = (float)((32 - ax) * (32 - ay)) * (1.0f / 1024.0f), w01 = (float)(ax * (32 - ay)) * (1.0f / 1024.0f);
+    const float w10 = (float)((32 - ax) * ay) * (1.0f / 1024.0f), w11 = (float)(ax * ay) * (1.0f / 1024.0f);
+    if (border_mode == VR180_BORDER_CONSTANT && (ix >= s.cols || ix + 1 < 0 || iy >= s.rows || iy + 1 < 0)) {
+#pragma unroll
+        for (int c = 0; c < C; ++c) out[c] = (int)cval[c];
+        return;
+    }
+    float v00[C], v01[C], v10[C], v11[C];
+    if ((unsigned)ix < (unsigned)(s.cols - 1) && (unsigned)iy < (unsigned)(s.rows - 1)) {
+        const uint16_t* q0 = px16<C>(s, ix, iy);
+        const uint16_t* q1 = reinterpret_cast<const uint16_t*>(reinterpret_cast<const uint8_t*>(q0) + s.pitch);
+#pragma unroll
+        for (int c = 0; c < C; ++c) {
+            v00[c] = __ldg(q0 + c);
+            v01[c] = __ldg(q0 + C + c);
+            v10[c] = __ldg(q1 + c);
+            v11[c] = __ldg(q1 + C + c);
+        }
+    } else {
+        tap16<C>(s, ix, iy, border_mode, cval, v00);
+        tap16<C>(s, ix + 1, iy, border_mode, cval, v01);
+        tap16<C>(s, ix, iy + 1, border_mode, cval, v10);
+        tap16<C>(s, ix + 1, iy + 1, border_mode, cval, v11);
+    }
+#pragma unroll
+    for (int c = 0; c < C; ++c) {
+        float acc = __fadd_rn(__fmul_rn(v00[c], w00), __fmul_rn(v01[c], w01));
+        acc = __fadd_rn(acc, __fmul_rn(v10[c], w10));
+        acc = __fadd_rn(acc, __fmul_rn(v11[c], w11));
+        out[c] = sat_u16(acc);
+    }
+}
+
+// INTER_CUBIC (K = 4) / INTER_LANCZOS4 (K = 8) with the float table ftab[ay*32+ax][ky][kx].
+//   interior (every tap inside): each row summed left to right, then the rows left to right;
+//   elsewhere, in EVERY border mode: s = cval, then s += (S - cval) * w for each valid tap in row-major order (under
+//   BORDER_CONSTANT a tap outside the source is not valid; other modes remap its index) -- so the border colour
+//   reaches results under REPLICATE / REFLECT / WRAP / REFLECT_101 too, as in OpenCV.
+template <int C, int K>
+__device__ __forceinline__ void sample16_tab(const Src& s, int sx, int sy, const float* __restrict__ ftab, int border_mode,
+                                             const float* cval, int* out) {
+    const int ix = sat16(sx >> kInterBits) - (K / 2 - 1), iy = sat16(sy >> kInterBits) - (K / 2 - 1);
+    const float* w = ftab + (size_t)(((sy & 31) << 5) | (sx & 31)) * (K * K);
+    float acc[C];
+    if ((unsigned)ix < (unsigned)max(s.cols - (K - 1), 0) && (unsigned)iy < (unsigned)max(s.rows - (K - 1), 0)) {
+        const uint16_t* q = px16<C>(s, ix, iy);
+#pragma unroll
+        for (int ky = 0; ky < K; ++ky) {
+            float r[C];
+#pragma unroll
+            for (int kx = 0; kx < K; ++kx) {
+                const float wv = __ldg(w + ky * K + kx);
+#pragma unroll
+                for (int c = 0; c < C; ++c) {
+                    const float p = __fmul_rn((float)__ldg(q + kx * C + c), wv);
+                    r[c] = kx ? __fadd_rn(r[c], p) : p;
+                }
+            }
+#pragma unroll
+            for (int c = 0; c < C; ++c) acc[c] = ky ? __fadd_rn(acc[c], r[c]) : r[c];
+            q = reinterpret_cast<const uint16_t*>(reinterpret_cast<const uint8_t*>(q) + s.pitch);
+        }
+    } else {
+#pragma unroll
+        for (int c = 0; c < C; ++c) acc[c] = cval[c];
+        for (int ky = 0; ky < K; ++ky) {
+            const int y = iy + ky;
+            if (border_mode == VR180_BORDER_CONSTANT && (unsigned)y >= (unsigned)s.rows) continue;
+            const int yy = border_index(y, s.rows, border_mode);
+            for (int kx = 0; kx < K; ++kx) {
+                const int x = ix + kx;
+                if (border_mode == VR180_BORDER_CONSTANT && (unsigned)x >= (unsigned)s.cols) continue;
+                const uint16_t* q = px16<C>(s, border_index(x, s.cols, border_mode), yy);
+                const float wv = __ldg(w + ky * K + kx);
+#pragma unroll
+                for (int c = 0; c < C; ++c)
+                    acc[c] = __fadd_rn(acc[c], __fmul_rn(__fsub_rn((float)__ldg(q + c), cval[c]), wv));
+            }
+        }
+    }
+#pragma unroll
+    for (int c = 0; c < C; ++c) out[c] = sat_u16(acc[c]);
 }
 
 }  // namespace vr180

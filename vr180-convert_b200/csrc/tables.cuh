@@ -1,6 +1,7 @@
-// tables.cuh -- host construction of OpenCV's INTER_CUBIC / INTER_LANCZOS4 fixed-point weight tables
-// (cv::initInterTab2D in imgproc/imgwarp.cpp; third-party to the reference, restated in oracle/remap_np.py and
-// SURVEY.md Appendix B.3).  int16 [ay*32+ax][ky][kx], every K*K block sums to exactly 32768.
+// tables.cuh -- host construction of OpenCV's INTER_CUBIC / INTER_LANCZOS4 weight tables (cv::initInterTab2D in
+// imgproc/imgwarp.cpp; third-party to the reference, restated in oracle/remap_np.py, oracle/remap_float_np.py and
+// SURVEY.md Appendix B.3).  8-bit images: int16 [ay*32+ax][ky][kx], every K*K block sums to exactly 32768.  16-bit
+// images: the float products before that conversion.
 #pragma once
 #include <cfloat>
 #include <cmath>
@@ -63,14 +64,35 @@ inline void coef_lanczos4(float t, float* c) {
     }
 }
 
-inline std::vector<int16_t> build_weight_table(int K) {
-    std::vector<int16_t> tab((size_t)1024 * K * K);
-    float one[32][8];
+// 1-D coefficients of the 32 fractional positions t = i * (1/32) (cv::initInterTab1D)
+inline void one_d_table(int K, float one[32][8]) {
     for (int i = 0; i < 32; ++i) {
         volatile float t = (float)i * (1.0f / 32.0f);
         if (K == 4) coef_cubic(t, one[i]);
         else coef_lanczos4(t, one[i]);
     }
+}
+
+// The float table of the non-8-bit depths: w[ay*32+ax][ky][kx] = float(one[ay][ky] * one[ax][kx]), rounded once and
+// without the sum fix-up of the int16 table (initInterTab2D with fixpt = false).
+inline std::vector<float> build_float_table(int K) {
+    std::vector<float> tab((size_t)1024 * K * K);
+    float one[32][8];
+    one_d_table(K, one);
+    for (int ay = 0; ay < 32; ++ay)
+        for (int ax = 0; ax < 32; ++ax)
+            for (int ky = 0; ky < K; ++ky)
+                for (int kx = 0; kx < K; ++kx) {
+                    volatile float v = one[ay][ky] * one[ax][kx];
+                    tab[((size_t)(ay * 32 + ax) * K + ky) * K + kx] = v;
+                }
+    return tab;
+}
+
+inline std::vector<int16_t> build_weight_table(int K) {
+    std::vector<int16_t> tab((size_t)1024 * K * K);
+    float one[32][8];
+    one_d_table(K, one);
     const int k2 = K / 2;
     for (int ay = 0; ay < 32; ++ay)
         for (int ax = 0; ax < 32; ++ax) {

@@ -977,7 +977,7 @@ static int launch_tiled(const RemapArgs& a0, const vr180_chain_t& c0, const vr18
 // the requested interpolation (1024 x 16 bicubic, 1024 x 64 Lanczos4; unused otherwise).
 int launch_remap_tiled(const RemapArgs& a0, int channels, int interp, const vr180_chain_t& c0, const vr180_chain_t& c1,
                        const short* weight_tab, cudaStream_t st) {
-    if (channels != 3) return VR180_ERR_UNSUPPORTED;
+    if (channels != 3 || a0.depth != VR180_DEPTH_8U) return VR180_ERR_UNSUPPORTED;
     if (interp != VR180_INTER_NEAREST && interp != VR180_INTER_LINEAR && interp != VR180_INTER_CUBIC &&
         interp != VR180_INTER_LANCZOS4)
         return VR180_ERR_UNSUPPORTED;

@@ -75,8 +75,10 @@ class _PinnedPool:
         self._keep = keep_bytes
         self._lock = threading.Lock()
 
-    def empty(self, shape: tuple[int, ...]) -> NDArray[np.uint8]:
-        nbytes = max(1, int(np.prod(shape)))
+    def empty(self, shape: tuple[int, ...], dtype: Any = np.uint8) -> NDArray:
+        dtype = np.dtype(dtype)
+        count = int(np.prod(shape))
+        nbytes = max(1, count * dtype.itemsize)  # the pool recycles byte buffers; the array is a view of any dtype
         with self._lock:
             lst = self._free.get(nbytes)
             ptr = lst.pop() if lst else None
@@ -88,7 +90,7 @@ class _PinnedPool:
             ptr = int(handle.value)
         owner = (C.c_uint8 * nbytes).from_address(ptr)
         weakref.finalize(owner, self._release, ptr, nbytes)
-        return np.frombuffer(owner, dtype=np.uint8, count=int(np.prod(shape))).reshape(shape)
+        return np.frombuffer(owner, dtype=dtype, count=count).reshape(shape)
 
     def _release(self, ptr: int, nbytes: int) -> None:
         with self._lock:
@@ -105,17 +107,17 @@ class _PinnedPool:
 _pinned = _PinnedPool()
 
 
-def pinned_empty(shape: tuple[int, ...]) -> NDArray[np.uint8]:
-    """A uint8 array in page-locked host memory (vr180_host_alloc), recycled when garbage-collected.  Frames a capture
-    or decode loop writes straight into such arrays are uploaded by DMA without the packing copy plain NumPy arrays
+def pinned_empty(shape: tuple[int, ...], dtype: Any = np.uint8) -> NDArray:
+    """A uint8 (or `dtype`) array in page-locked host memory (vr180_host_alloc), recycled when garbage-collected.
+    Frames a capture or decode loop writes straight into such arrays are uploaded by DMA without the packing copy plain NumPy arrays
     need (the host pipeline decides per buffer, include/vr180_b200.h `staging`)."""
-    return _pinned.empty(tuple(int(v) for v in shape))
+    return _pinned.empty(tuple(int(v) for v in shape), dtype)
 
 
-def _result_empty(shape: tuple[int, ...]) -> NDArray[np.uint8]:
+def _result_empty(shape: tuple[int, ...], dtype: Any = np.uint8) -> NDArray:
     if os.environ.get("VR180_PINNED_OUTPUTS", "1") == "0":
-        return np.empty(shape, dtype=np.uint8)
-    return _pinned.empty(shape)
+        return np.empty(shape, dtype=dtype)
+    return _pinned.empty(shape, dtype)
 
 
 # ---------------------------------------------------------------------------------------------------------
@@ -204,7 +206,7 @@ def get_map(
 # radius
 # ---------------------------------------------------------------------------------------------------------
 def _centre_line(img: NDArray) -> NDArray:
-    """The one row / column get_radius reads (transformer.py:125-129), as a (1, n, C) or (n, 1, C) uint8 image
+    """The one row / column get_radius reads (transformer.py:125-129), as a (1, n, C) or (n, 1, C) image
     whose centre line is that row / column again -- so only ~n*C bytes are uploaded."""
     if img.ndim != 3:
         raise IndexError("too many indices for array: get_radius needs an (H, W, C) image")
@@ -219,13 +221,11 @@ def _device_radius(images: Sequence[NDArray], threshold: float = 10) -> list[flo
     ONE upload, are scanned by ONE k_get_radius launch and come back with ONE blocking read."""
     import torch
 
-    dev = torch.device("cuda", _default_device)
-    stream = torch.cuda.current_stream(dev).cuda_stream
     lines = []
     for img in images:
         line = _centre_line(np.asarray(img))
-        if line.dtype != np.uint8:
-            raise TypeError("get_radius kernel takes uint8 images")
+        if line.dtype not in _DEPTHS:
+            raise TypeError(f"get_radius kernel takes uint8 or uint16 images, got {line.dtype}")
         rows, cols, ch = line.shape
         if ch > 4:
             raise ValueError("get_radius kernel supports up to 4 channels")
@@ -233,15 +233,18 @@ def _device_radius(images: Sequence[NDArray], threshold: float = 10) -> list[flo
         if cols <= rows and rows == 1:
             raise IndexError("index 0 is out of bounds for axis 0 with size 0")
         lines.append(line)
+    dev = torch.device("cuda", _default_device)
+    stream = torch.cuda.current_stream(dev).cuda_stream
     out: list[float] = [0.0] * len(lines)
     groups: dict[tuple, list[int]] = {}
     for i, line in enumerate(lines):
-        groups.setdefault(line.shape, []).append(i)
-    for (rows, cols, ch), idx in groups.items():
+        groups.setdefault((line.shape, line.dtype), []).append(i)
+    for ((rows, cols, ch), dtype), idx in groups.items():
         stack = np.stack([lines[i] for i in idx])  # (n, rows, cols, ch), one of rows / cols is 1
         d_lines = torch.from_numpy(stack).to(dev)
         trans = torch.empty((len(idx), 2), dtype=torch.int32, device=dev)
-        im = N.Image(d_lines.data_ptr(), rows, cols, ch, 0, cols * ch, rows * cols * ch)
+        esz = dtype.itemsize
+        im = N.Image(d_lines.data_ptr(), rows, cols, ch, _DEPTHS[dtype], cols * ch * esz, rows * cols * ch * esz)
         N.check(N.lib().vr180_get_radius(C.byref(im), 1, len(idx), float(threshold), trans.data_ptr(), None, stream),
                 "vr180_get_radius")
         for i, (first, last) in zip(idx, trans.cpu().tolist()):
@@ -266,6 +269,13 @@ def get_radius_smart(radius: float | Literal["auto", "max"], images: Sequence[ND
 # ---------------------------------------------------------------------------------------------------------
 # apply / apply_lr
 # ---------------------------------------------------------------------------------------------------------
+def _border_scalar(value: Any) -> "C.Array[C.c_double]":
+    """The cv::Scalar cv2 builds from a border value: a Python scalar v becomes (v, 0, 0, 0), a sequence its first four
+    entries.  The library saturates it to the image depth (vr180_remap_ex / vr180_ctx_run_ex)."""
+    vals = [float(value), 0.0, 0.0, 0.0] if np.isscalar(value) else [*map(float, value), 0.0, 0.0, 0.0, 0.0][:4]
+    return (C.c_double * 4)(*vals)
+
+
 def _border_bytes(value: Any, channels: int) -> tuple[int, int, int, int]:
     """cv2 converts a Python scalar to Scalar(v, 0, 0, 0) and saturates each entry to uint8."""
     vals = [float(value), 0.0, 0.0, 0.0] if np.isscalar(value) else [*map(float, value), 0.0, 0.0, 0.0, 0.0][:4]
@@ -286,17 +296,34 @@ def _check_modes(interpolation: int, border_mode: int) -> tuple[int, int]:
     return interpolation, border_mode
 
 
+# element types of the remap path -> vr180 depth codes
+_DEPTHS = {np.dtype(np.uint8): N.DEPTH_8U, np.dtype(np.uint16): N.DEPTH_16U}
+
+
 def _as_image(a: Any) -> NDArray:
     img = np.asarray(a)
-    if img.dtype != np.uint8:
-        raise TypeError("the B200 remap path takes uint8 images (what cv.imread returns)")
+    if img.dtype not in _DEPTHS:
+        raise TypeError(f"the B200 remap path takes uint8 or uint16 images (what cv.imread returns), got {img.dtype}")
     if img.ndim == 2:
         img = img[:, :, None]
     if img.ndim != 3 or img.shape[2] not in (1, 3, 4):
         raise ValueError(f"unsupported image shape {img.shape}")
-    if img.strides[2] != 1 or img.strides[1] != img.shape[2] or img.strides[0] < img.shape[1] * img.shape[2]:
+    e = img.itemsize
+    if img.strides[2] != e or img.strides[1] != img.shape[2] * e or img.strides[0] < img.shape[1] * img.shape[2] * e:
         img = np.ascontiguousarray(img)  # only pixel-contiguous rows can be described by a pitch
     return img
+
+
+def _run_job(job: "N.HostJob", dtype: np.dtype, border_value: Any) -> None:
+    """vr180_ctx_run with the job's depth and border colour: 8-bit colours as saturated bytes, 16-bit ones as the
+    cv::Scalar the library saturates (a colour above 255 does not fit the job's byte field)."""
+    job.depth = _DEPTHS[np.dtype(dtype)]
+    if job.depth == N.DEPTH_8U:
+        for i, b in enumerate(_border_bytes(border_value, job.channels)):
+            job.border_value[i] = b
+        N.check(N.lib().vr180_ctx_run(_ctx(), C.byref(job)), "vr180_ctx_run")
+    else:
+        N.check(N.lib().vr180_ctx_run_ex(_ctx(), C.byref(job), _border_scalar(border_value)), "vr180_ctx_run_ex")
 
 
 def warp_host(
@@ -334,16 +361,21 @@ def warp_host(
     if n_frames == 0:
         return []
     rows, cols, ch = frames[0][0].shape
+    dtype = frames[0][0].dtype
     for v in frames:
         for im in v:
             if im.shape != (rows, cols, ch):
                 raise ValueError("all frames / eyes of one job must have the same shape")
+            if im.dtype != dtype:
+                raise ValueError("all frames / eyes of one job must have the same dtype")
     w, h = int(size_output[0]), int(size_output[1])
     first = np.asarray(images[0][0] if batched else images[0])
     squeeze = first.ndim == 2
     if merge and (n_views != 2 or ch != 3):
         raise ValueError("merge needs two 3-channel views")
-    outs = [_result_empty((h, w * (1 if merge else n_views), ch)) for _ in range(n_frames)]
+    if merge and dtype != np.uint8:
+        raise ValueError("merge (the anaglyph) takes uint8 images")
+    outs = [_result_empty((h, w * (1 if merge else n_views), ch), dtype) for _ in range(n_frames)]
 
     job = N.HostJob()
     job.n_views, job.n_frames = n_views, n_frames
@@ -381,8 +413,6 @@ def warp_host(
         job.src_frame_stride[v] = pitch * rows
     job.out_w, job.out_h = w, h
     job.interpolation, job.border_mode = interpolation, border_mode
-    for i, b in enumerate(_border_bytes(border_value, ch)):
-        job.border_value[i] = b
     dptrs = (C.c_void_p * n_frames)(*[o.ctypes.data for o in outs])
     keep.append(dptrs)
     job.dst = dptrs[0]
@@ -396,7 +426,7 @@ def warp_host(
         job.threshold = float(threshold)
         trans = np.empty((n_frames, n_views, 2), dtype=np.int32)
         job.transitions_out = trans.ctypes.data
-    N.check(lib.vr180_ctx_run(_ctx(), C.byref(job)), "vr180_ctx_run")
+    _run_job(job, dtype, border_value)
     del keep
     if trans is not None and (trans < 0).any():
         raise IndexError("index 0 is out of bounds for axis 0 with size 0")  # get_radius found no transition
@@ -444,7 +474,10 @@ def apply(
     images = [_imread(p) if isinstance(p, (str, Path)) else p for p in in_list]
     radius_ = get_radius_smart(radius, images)
     size_in = (images[0].shape[0], images[0].shape[1])
-    same = [i for i, img in enumerate(images) if np.asarray(img).shape == np.asarray(images[0]).shape]
+    # one job for the images of images[0]'s shape and dtype; cv.remap takes every image on its own, in its own dtype
+    first = np.asarray(images[0])
+    same = [i for i, img in enumerate(images)
+            if np.asarray(img).shape == first.shape and np.asarray(img).dtype == first.dtype]
     results: list[Any] = [None] * len(images)
     warped = warp_host([transformer], [[images[i] for i in same]], radii=[radius_], share_map=True,
                        size_output=size_output, interpolation=interpolation, border_mode=border_mode,
@@ -454,8 +487,9 @@ def apply(
     for i, img in enumerate(images):
         if results[i] is None:
             # the reference samples a differently-sized image with images[0]'s map; keep that behaviour
-            LOG.warning("image shape %s differs from the first image %s; using the first image's map",
-                        np.asarray(img).shape, size_in)
+            if np.asarray(img).shape != first.shape:
+                LOG.warning("image shape %s differs from the first image %s; using the first image's map",
+                            np.asarray(img).shape, size_in)
             results[i] = _warp_with_first_geometry(transformer, img, size_in, radius_, size_output, interpolation,
                                                    border_mode, boarder_value)
     if out_list is not None:
@@ -476,7 +510,7 @@ def _warp_with_first_geometry(transformer, img, size_in, radius_, size_output, i
 
 def remap_maps(img: NDArray, xmap: NDArray, ymap: NDArray, *, interpolation: int = INTER_LINEAR,
                border_mode: int = BORDER_CONSTANT, border_value: Any = 0) -> NDArray[np.uint8]:
-    """cv2.remap(img, xmap, ymap, interpolation, borderMode, borderValue) for uint8 images and float32 maps."""
+    """cv2.remap(img, xmap, ymap, interpolation, borderMode, borderValue) for uint8 / uint16 images and float32 maps."""
     interpolation, border_mode = _check_modes(interpolation, border_mode)
     xm = np.ascontiguousarray(xmap, dtype=np.float32)
     ym = np.ascontiguousarray(ymap, dtype=np.float32)
@@ -485,7 +519,7 @@ def remap_maps(img: NDArray, xmap: NDArray, ymap: NDArray, *, interpolation: int
     view = _as_image(img)
     rows, cols, ch = view.shape
     h, w = xm.shape
-    dst = _result_empty((h, w, ch))
+    dst = _result_empty((h, w, ch), view.dtype)
     job = N.HostJob()
     job.n_views = job.n_frames = 1
     job.src[0] = view.ctypes.data
@@ -496,10 +530,8 @@ def remap_maps(img: NDArray, xmap: NDArray, ymap: NDArray, *, interpolation: int
     job.xmap[0], job.ymap[0] = xm.ctypes.data, ym.ctypes.data
     job.out_w, job.out_h = w, h
     job.interpolation, job.border_mode = interpolation, border_mode
-    for i, b in enumerate(_border_bytes(border_value, ch)):
-        job.border_value[i] = b
     job.dst, job.dst_pitch, job.dst_frame_stride = dst.ctypes.data, dst.strides[0], dst.strides[0] * h
-    N.check(N.lib().vr180_ctx_run(_ctx(), C.byref(job)), "vr180_ctx_run")
+    _run_job(job, view.dtype, border_value)
     return dst[:, :, 0] if np.asarray(img).ndim == 2 else dst
 
 
@@ -614,8 +646,12 @@ def lr_frame(transformer, left, right, *, size_output=(2048, 2048), interpolatio
     interpolation, border_mode = _check_modes(interpolation, boarder_mode)
     left, right = _split_if_same_path(left, right)
     eyes = [_imread(p) if isinstance(p, (str, Path)) else p for p in (left, right)]
+    if merge and any(np.asarray(e).dtype != np.uint8 for e in eyes):
+        raise ValueError("merge (the anaglyph) takes uint8 images")
     kw = dict(size_output=size_output, interpolation=interpolation, border_mode=border_mode, border_value=boarder_value)
-    same_shape = np.asarray(eyes[0]).shape == np.asarray(eyes[1]).shape
+    # eyes of different dtypes are warped one by one, and np.concatenate promotes the halves as in the reference
+    same_shape = (np.asarray(eyes[0]).shape == np.asarray(eyes[1]).shape
+                  and np.asarray(eyes[0]).dtype == np.asarray(eyes[1]).dtype)
     fused_merge = merge and same_shape and np.asarray(eyes[0]).ndim == 3 and np.asarray(eyes[0]).shape[2] == 3
 
     def finish(halves):  # eyes that had to be warped separately
@@ -681,7 +717,7 @@ def lr_frames(transformer, lefts: Sequence[Any], rights: Sequence[Any], *, size_
         return []
     kw = dict(size_output=size_output, interpolation=interpolation, border_mode=border_mode, border_value=boarder_value)
     auto = isinstance(radius, str) and radius == "auto"
-    shapes = {np.asarray(im).shape for im in (*lefts, *rights)}
+    shapes = {(np.asarray(im).shape, np.asarray(im).dtype) for im in (*lefts, *rights)}
     per_eye = isinstance(transformer, tuple)
     lowerable = all(t.lower(shape=(int(size_output[1]), int(size_output[0]))) is not None
                     for t in (transformer if per_eye else (transformer,)))

@@ -26,8 +26,8 @@ from typing import Any, Literal, Sequence
 import numpy as np
 
 from . import _native as N
-from .remapper import (BORDER_CONSTANT, INTER_LINEAR, INTER_NEAREST, _border_bytes, _check_modes, host_maps,
-                       lower_full)
+from .remapper import (BORDER_CONSTANT, INTER_LINEAR, INTER_NEAREST, _border_bytes, _border_scalar, _check_modes,
+                       host_maps, lower_full)
 from .shard import shard_range  # noqa: F401  (re-exported)
 from .transformer import TransformerBase
 
@@ -60,6 +60,7 @@ class SbsWarper:
         self.w, self.h = int(size_output[0]), int(size_output[1])
         self.interpolation, self.border_mode = _check_modes(interpolation, boarder_mode)
         self.border_value = _border_bytes(boarder_value, channels)
+        self.border_scalar = _border_scalar(boarder_value)  # 16-bit frames: saturated by the library
         self.channels = channels
         self.threshold = float(threshold)
         if map_source not in ("auto", "analytic", "lut", "lut_fixed", "lut_packed"):
@@ -148,11 +149,12 @@ class SbsWarper:
     # (frame, eye) rectangles per tile up to which vr180_remap streams the tiles (csrc/tiled.cu: 20 with a shared map)
     _STREAM_ITEMS = {True: 20, False: 16}
 
-    def _source_for(self, n_frames: int) -> str:
-        """The coordinate source of one call: the plan's, or for "auto" the faster one for this batch size."""
+    def _source_for(self, n_frames: int, wide: bool = False) -> str:
+        """The coordinate source of one call: the plan's, or for "auto" the faster one for this batch size (`wide`:
+        16-bit frames, which the tile-streaming kernel does not take)."""
         if self.map_source != "auto":
             return self.map_source
-        has_tiled_lut = self.channels == 3
+        has_tiled_lut = self.channels == 3 and not wide
         if not self._lowerable:  # user-defined Python transformer: host maps, once
             return "lut_packed" if has_tiled_lut else "lut"
         if self.auto_radius or not has_tiled_lut:
@@ -163,10 +165,16 @@ class SbsWarper:
         return "lut_packed" if self._small_calls > 1 or self._packed is not None else "analytic"
 
     def _image(self, t) -> N.Image:
-        if t.dtype != self.torch.uint8 or t.dim() != 4 or t.shape[1] != self.rows or t.shape[2] != self.cols \
+        torch = self.torch
+        depths = {torch.uint8: N.DEPTH_8U, torch.uint16: N.DEPTH_16U}
+        if t.dtype not in depths:
+            raise TypeError(f"frames must be torch.uint8 or torch.uint16, got {t.dtype}")
+        if t.dim() != 4 or t.shape[1] != self.rows or t.shape[2] != self.cols \
                 or t.shape[3] != self.channels or t.stride(3) != 1 or t.stride(2) != self.channels:
-            raise ValueError(f"frames must be uint8 (F, {self.rows}, {self.cols}, {self.channels}) with contiguous pixels")
-        return N.Image(t.data_ptr(), self.rows, self.cols, self.channels, 0, t.stride(1), t.stride(0))
+            raise ValueError(f"frames must be (F, {self.rows}, {self.cols}, {self.channels}) with contiguous pixels")
+        e = t.element_size()  # torch strides count elements; the ABI's pitches are bytes
+        return N.Image(t.data_ptr(), self.rows, self.cols, self.channels, depths[t.dtype], t.stride(1) * e,
+                       t.stride(0) * e)
 
     def radius_per_frame(self, left, right):
         """k_get_radius over the batch: float64 radius per frame (max over both eyes) and the raw transitions."""
@@ -182,16 +190,20 @@ class SbsWarper:
         return self._radius_buf[:n], self._trans_buf[:n]
 
     def __call__(self, left, right, out=None, radius=None):
-        """left / right: uint8 CUDA tensors (F, rows, cols, C) -> out (F, H, 2W, C), eyes side by side.
+        """left / right: uint8 or uint16 CUDA tensors (F, rows, cols, C) -> out (F, H, 2W, C) of the same dtype, eyes
+        side by side.
 
         `radius` (plans built with radius="auto" only): float64 CUDA tensor (F,) of per-frame radii to use instead
         of running get_radius, e.g. radii estimated once and smoothed over a clip; NaN = "no transition found"."""
         torch = self.torch
         n = left.shape[0]
-        if right.shape != left.shape:
-            raise ValueError("left / right batches differ in shape")
+        if right.shape != left.shape or right.dtype != left.dtype:
+            raise ValueError("left / right batches differ in shape or dtype")
+        wide = left.dtype == torch.uint16
         if out is None:
-            out = torch.empty((n, self.h, 2 * self.w, self.channels), dtype=torch.uint8, device=self.device)
+            out = torch.empty((n, self.h, 2 * self.w, self.channels), dtype=left.dtype, device=self.device)
+        if out.dtype != left.dtype:
+            raise ValueError("out must have the dtype of the frames")
         p = N.RemapParams()
         p.n_views, p.n_frames = 2, n
         p.share_map = 1 if self.share_map else 0
@@ -199,7 +211,8 @@ class SbsWarper:
         p.interpolation, p.border_mode = self.interpolation, self.border_mode
         for i, b in enumerate(self.border_value):
             p.border_value[i] = b
-        p.dst, p.dst_pitch, p.dst_frame_stride = out.data_ptr(), out.stride(1), out.stride(0)
+        e = out.element_size()
+        p.dst, p.dst_pitch, p.dst_frame_stride = out.data_ptr(), out.stride(1) * e, out.stride(0) * e
         radius_dev = None
         if radius is not None:
             if not self.auto_radius:
@@ -209,7 +222,7 @@ class SbsWarper:
             radius_dev = radius
         elif self.auto_radius:
             radius_dev, _ = self.radius_per_frame(left, right)
-        source = self._source_for(n)
+        source = self._source_for(n, wide)
         for v, frames in enumerate((left, right)):
             vw = p.view[v]
             vw.src = self._image(frames)
@@ -233,5 +246,8 @@ class SbsWarper:
                 vw.map.kind = N.MAPSRC_FIXED
                 vw.map.fixed, vw.map.map_pitch = fixed[m].data_ptr(), self.w
         stream = torch.cuda.current_stream(self.device).cuda_stream
-        N.check(N.lib().vr180_remap(C.byref(p), stream), "vr180_remap")
+        if wide:
+            N.check(N.lib().vr180_remap_ex(C.byref(p), self.border_scalar, stream), "vr180_remap_ex")
+        else:
+            N.check(N.lib().vr180_remap(C.byref(p), stream), "vr180_remap")
         return out
