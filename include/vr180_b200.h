@@ -225,15 +225,18 @@ int vr180_pack_lut_tiles(const float* xmap_dev, const float* ymap_dev, int64_t m
  *      pitch and frame stride is a multiple of 16 bytes and every view's dst_x_offset * 3 is too (a TMA box must start at
  *      a 16-byte aligned global address).  With BORDER_CONSTANT and a zero colour, tiles that straddle the source edge
  *      are staged too (TMA's zero fill is the border); with any other border mode / colour only tiles whose footprint
- *      lies inside the source are staged and the (few) edge tiles are gathered per pixel inside the same kernel.  Any
- *      other request runs in the generic per-pixel kernel.
+ *      lies inside the source are staged and the (few) edge tiles are gathered per pixel inside the same kernel.
+ *      16-bit images (vr180_remap_ex) are tiled for 3 channels with NEAREST / LINEAR under the same conditions, with
+ *      6 bytes per pixel: every row pitch >= cols * 6 and every dst_x_offset * 6 a multiple of 16 (the right eye of an
+ *      SBS frame at column W: W a multiple of 8).  Any other request, including 16-bit CUBIC / LANCZOS4 and 16-bit
+ *      1 / 4 channels, runs in the generic per-pixel kernel.
  * ---------------------------------------------------------------------------------------------------- */
 int vr180_remap(const vr180_remap_params_t* params, void* stream);
 /* vr180_remap with the border colour given as the cv::Scalar the reference passes (borderValue): the library saturates
  * each entry to the depth of the images (round half to even, clamp), as cv2 does.  NULL = use params->border_value.
  * 16-bit images (src.depth = VR180_DEPTH_16U for every view; the destination has the same depth) follow cv::remap's
- * float-weight arithmetic for non-8-bit depths and are bit-exact to cv2.remap on uint16 images; they run in the generic
- * per-pixel kernel (base pointers, pitches and strides 2-byte aligned).  Any other depth, or views of different depths,
+ * float-weight arithmetic for non-8-bit depths and are bit-exact to cv2.remap on uint16 images (base pointers, pitches
+ * and strides 2-byte aligned); see the performance note of vr180_remap for which of them run in the TMA-tiled kernel.  Any other depth, or views of different depths,
  * is VR180_ERR_UNSUPPORTED. */
 int vr180_remap_ex(const vr180_remap_params_t* params, const double border_scalar[4], void* stream);
 

@@ -104,7 +104,7 @@ size_t packed_lut_bytes(int out_w, int out_h, int interp);  // tiled.cu; 0 = int
 int launch_pack_lut_tiles(const float* xmap, const float* ymap, int64_t map_pitch, int out_w, int out_h, int interp,
                           void* packed, cudaStream_t st);
 int launch_remap_tiled(const RemapArgs& a, int channels, int interp, const vr180_chain_t& c0, const vr180_chain_t& c1,
-                       const short* weight_tab, cudaStream_t st);  // tiled.cu; VR180_ERR_UNSUPPORTED = not eligible, use the generic kernel
+                       const short* weight_tab, const Remap16& x16, cudaStream_t st);  // tiled.cu; VR180_ERR_UNSUPPORTED = not eligible, use the generic kernel
 int launch_get_radius(const vr180_image_t* views, int n_views, int n_frames, double threshold, int32_t* transitions,
                       double* radius, cudaStream_t st);
 int validate_chain(const vr180_chain_t* c);

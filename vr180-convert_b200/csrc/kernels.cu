@@ -357,7 +357,7 @@ int launch_remap(const vr180_remap_params_t* p, const double* border_scalar, cud
         const short* weight_tab = nullptr;
         if (interp == VR180_INTER_CUBIC) VR180_CUDA(cudaGetSymbolAddress((void**)&weight_tab, g_tab_cubic));
         if (interp == VR180_INTER_LANCZOS4) VR180_CUDA(cudaGetSymbolAddress((void**)&weight_tab, g_tab_lanczos));
-        const int rc = launch_remap_tiled(a, C, interp, *chains[0], *chains[1], weight_tab, st);
+        const int rc = launch_remap_tiled(a, C, interp, *chains[0], *chains[1], weight_tab, x16, st);
         if (rc != VR180_ERR_UNSUPPORTED) return rc;
     }
 

@@ -240,6 +240,19 @@ __device__ __forceinline__ void sample16_nearest(const Src& s, float mx, float m
     for (int c = 0; c < C; ++c) out[c] = __ldg(q + c);
 }
 
+// INTER_NEAREST on the integer coordinate (ix, iy) = (sat16(cvRound(x)), sat16(cvRound(y))): the pixel or the border.
+template <int C>
+__device__ __forceinline__ void nearest16(const Src& s, int ix, int iy, int border_mode, const float* cval, int* out) {
+    if (border_mode == VR180_BORDER_CONSTANT && !((unsigned)ix < (unsigned)s.cols && (unsigned)iy < (unsigned)s.rows)) {
+#pragma unroll
+        for (int c = 0; c < C; ++c) out[c] = (int)cval[c];
+        return;
+    }
+    const uint16_t* q = px16<C>(s, border_index(ix, s.cols, border_mode), border_index(iy, s.rows, border_mode));
+#pragma unroll
+    for (int c = 0; c < C; ++c) out[c] = __ldg(q + c);
+}
+
 // One bilinear tap as float: the pixel, or under BORDER_CONSTANT the border colour outside the source.
 template <int C>
 __device__ __forceinline__ void tap16(const Src& s, int x, int y, int border_mode, const float* cval, float* v) {

@@ -354,6 +354,7 @@ static int launch_stream_mode(const RemapArgs& a, const short* tab, cudaStream_t
 // of this interpolation, no per-frame radius).
 int launch_remap_stream(const RemapArgs& a, int interp, const short* weight_tab, cudaStream_t st) {
     using namespace tiled;
+    if (a.depth != VR180_DEPTH_8U) return VR180_ERR_UNSUPPORTED;  // tile headers hold 8-bit box geometry
     if (interp == VR180_INTER_NEAREST) return launch_stream_mode<Nearest>(a, nullptr, st);
     if (interp == VR180_INTER_LINEAR) return launch_stream_mode<LinearP>(a, nullptr, st);
     if (interp == VR180_INTER_CUBIC) return launch_stream_mode<Cubic>(a, weight_tab, st);

@@ -1,5 +1,5 @@
-// tiled.cu -- the tiled fast path of the fused warp: uint8 x 3 channels, INTER_LINEAR or INTER_CUBIC,
-// BORDER_CONSTANT (0).
+// tiled.cu -- the tiled fast path of the fused warp: uint8 x 3 channels with every interpolation, uint16 x 3 channels
+// with INTER_NEAREST / INTER_LINEAR (modes Linear16 / Nearest16, tiled.cuh); every border mode.
 //
 // Replaces cv.remap per eye + np.concatenate (/root/reference/src/vr180_convert/remapper.py:388-398, :518) and,
 // for MAPSRC_ANALYTIC, get_map (remapper.py:23-59) for a batch of frames that share their maps (the reference's
@@ -86,7 +86,7 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
                                            const double (&nx)[M::kPx], const double (&ny)[M::kPx], const short* tab) {
     static_assert(FR == 1 || !DYN, "a per-frame radius gives every frame its own rectangle");
     static_assert(M::kOutTiles / FR >= 2, "at least two out buffers of one item each");
-    constexpr int kOutTileBytes = M::kTileH * kTileW * 3;
+    constexpr int kOutTileBytes = M::kTileH * kTileW * M::kBpp;
     constexpr int kOutItemBytes = FR * kOutTileBytes;
     constexpr int OB = M::kOutTiles / FR < kOutBufs ? M::kOutTiles / FR : kOutBufs;  // out buffers of one item each
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -112,9 +112,9 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
 
     if (warp == kSamplers / 32) {  // ---- producer ----
         if (lane != 0) return;
-        const CUtensorMap* const map0 = &tm.src[v_begin][(pitch - kPitchMin) / kPitchStep][tg.rsel];
-        const int dst_x0 = (a.view[v_begin].dst_x_offset + tg.x0) * 3;
-        const int dst_x1 = (a.view[v_begin + NV - 1].dst_x_offset + tg.x0) * 3;
+        const CUtensorMap* const map0 = &tm.src[v_begin][(pitch - M::kPitchMin) / M::kPitchStep][tg.rsel];
+        const int dst_x0 = (a.view[v_begin].dst_x_offset + tg.x0) * M::kBpp;
+        const int dst_x1 = (a.view[v_begin + NV - 1].dst_x_offset + tg.x0) * M::kBpp;
         int p_item = 0, p_stage = 0;  // next item to fetch and its stage
         auto load = [&]() {
             const uint32_t bar = s_full + p_stage * 8;
@@ -140,9 +140,9 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
 #pragma unroll
                 for (int fr = 0; fr < FR; ++fr)  // a frame past the batch is all zero fill, and still rect_bytes on the barrier
                     tma_load_3d(s_stage + p_stage * stage_stride + fr * frame_pitch,
-                                map0 + (VPAIR ? fr : v) * (kWidths * kRowSizes), bx0, ry0, VPAIR ? f : f + fr, bar);
+                                map0 + (VPAIR ? fr : v) * (kWidths * kRowSizes), bx0 / M::kElem, ry0, VPAIR ? f : f + fr, bar);
             } else {
-                tma_load_3d(s_stage + p_stage * stage_stride, map0 + v * (kWidths * kRowSizes), bx0, ry0, f, bar);
+                tma_load_3d(s_stage + p_stage * stage_stride, map0 + v * (kWidths * kRowSizes), bx0 / M::kElem, ry0, f, bar);
             }
             ++p_item;
             if (++p_stage == S) p_stage = 0;
@@ -173,92 +173,154 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
     }
 
     // ---- sampling warps ----
-    // The 3-byte results [c0 c1 c2 .] of a warp step are re-packed into words of the dense out tile with ONE
-    // shuffle: every lane fetches the pixel of lane + 1; lanes 4 m + i, i < 3, then hold word 3 m + i of the row
-    // segment (12 bytes of 4 pixels = 3 words): [c0 c1 c2 c0'], [c1 c2 c0' c1'], [c2 c0' c1' c2'].
-    const int sub = lane & 3;
-    const uint32_t out_sel = sub == 0 ? 0x4210u : (sub == 1 ? 0x5421u : 0x6542u);
-    const bool writer = sub != 3;
-    // this lane's word of step k inside the dense out tile
-    //   row patch: row 4 band + k, word 3 (lane >> 2) + sub
-    //   8 x 4 patch: row 4 band + (lane >> 3), byte 24 (kPx cg + k), word 3 ((lane & 7) >> 2) + sub
-    constexpr int kOutStep = M::kRowPatch ? kTileW * 3 : 24;
-    const int sw = band * (4 / M::kPx) + cg;  // sampling warp index; with row patches it owns rows kPx sw .. kPx sw + kPx - 1
-    uint32_t outp = s_out + (M::kRowPatch ? (M::kPx * sw) * (kTileW * 3) + (3 * (lane >> 2) + sub) * 4
-                                          : (4 * band + (lane >> 3)) * (kTileW * 3) + M::kPx * cg * 24 +
-                                                (3 * ((lane & 7) >> 2) + sub) * 4);
-    uint32_t flags = (writer ? 1u : 0u) | (lane == 0 ? 2u : 0u);
-    // opaque to the compiler: otherwise it re-derives them from S2R SR_TID.X inside the frame loop
-    asm volatile("" : "+r"(outp), "+r"(flags));
-
-    int st = 0;
-    uint32_t ph = 0;
-    typename M::Pixel cur[M::kPx];  // DYN: constants of the current radius
-    double cur_rad = CUDART_NAN;
-    bool cur_have = false;
+    if constexpr (M::kBpp == 6) {
+        // 16-bit modes, one-frame items.  The 6-byte results (.x = [c0 c1], .y = [c2 .]) of a warp step are re-packed
+        // with ONE shuffle: lanes 2 m and 2 m + 1 hold the 12 bytes = words 3 m .. 3 m + 2 of the row segment; lane
+        // 2 m + 1 sends its [c0' c1'] to lane 2 m, which stores [c0 c1] and [c2 c0'], and lane 2 m + 1 stores [c1' c2'].
+        static_assert(FR == 1 && !VPAIR, "a 16-bit item is one frame");
+        constexpr int kRowBytes = kTileW * M::kBpp;  // 192: one row of the out tile
+        const bool odd = (lane & 1) != 0;
+        const uint32_t sel_a = odd ? 0x5432u : 0x3210u;
+        const int sw = band * (4 / M::kPx) + cg;  // the warp owns rows kPx sw .. kPx sw + kPx - 1 of the tile
+        uint32_t outp = s_out + (M::kPx * sw) * kRowBytes + 12 * (lane >> 1) + (odd ? 8 : 0);
+        uint32_t flags = (odd ? 0u : 1u) | (lane == 0 ? 2u : 0u);
+        asm volatile("" : "+r"(outp), "+r"(flags));
+        int st = 0;
+        uint32_t ph = 0;
+        typename M::Pixel cur[M::kPx];  // DYN: constants of the current radius
+        double cur_rad = CUDART_NAN;
+        bool cur_have = false;
 #pragma unroll
-    for (int k = 0; k < M::kPx; ++k) cur[k] = pc[k];
-    for (int n = 0; n < n_items; ++n) {
-        mbar_wait(s_full + st * 8, ph);
-        const uint32_t buf = s_stage + st * stage_stride;
-        uint32_t res[FR][M::kPx];
-        if (DYN) {
-            // The per-pixel constants depend on the frame only through its radius: they are rebuilt when the radius
-            // changes (a static rig gives runs of equal radii; both eyes of a frame always share it).
-            const int f = f0 + ((NV == 2) ? (n >> 1) : n);  // FR == 1
-            const double rad = __ldg(dr.radius + f);
-            if (!(rad == cur_rad)) {
-                const int2 org = s_org[st];
-                cur_have = rad == rad;
+        for (int k = 0; k < M::kPx; ++k) cur[k] = pc[k];
+        for (int n = 0; n < n_items; ++n) {
+            mbar_wait(s_full + st * 8, ph);
+            const uint32_t buf = s_stage + st * stage_stride;
+            if (DYN) {  // constants rebuilt when the radius changes, as for 8 bits
+                const int f = f0 + ((NV == 2) ? (n >> 1) : n);
+                const double rad = __ldg(dr.radius + f);
+                if (!(rad == cur_rad)) {
+                    const int2 org = s_org[st];
+                    cur_have = rad == rad;
 #pragma unroll
-                for (int k = 0; k < M::kPx; ++k) {
-                    const int qx = denorm_q<M>(nx[k], rad, dr.cx), qy = denorm_q<M>(ny[k], rad, dr.cy);
-                    const int off = ((qy >> M::kShift) - M::kLo - org.y) * pitch + 3 * ((qx >> M::kShift) - M::kLo) - org.x;
-                    M::set_offset(cur[k], off, cur_have);
-                    M::weights(cur[k], qx & 31, qy & 31, tab);
+                    for (int k = 0; k < M::kPx; ++k) {
+                        const int qx = denorm_q<M>(nx[k], rad, dr.cx), qy = denorm_q<M>(ny[k], rad, dr.cy);
+                        const int off = ((qy >> M::kShift) - M::kLo - org.y) * pitch + M::kBpp * ((qx >> M::kShift) - M::kLo) - org.x;
+                        M::set_offset(cur[k], off, cur_have);
+                        M::weights(cur[k], qx & 31, qy & 31, tab);
+                    }
+                    cur_rad = rad;
                 }
-                cur_rad = rad;
             }
+            uint32_t w0[M::kPx], w1[M::kPx];
 #pragma unroll
             for (int k = 0; k < M::kPx; ++k) {
-                const uint32_t r = M::sample(buf, cur[k], (uint32_t)pitch);
-                res[0][k] = cur_have ? r : 0u;  // NaN radius (no transition found): border colour
+                uint2 r = M::sample(buf, DYN ? cur[k] : pc[k], (uint32_t)pitch);
+                if (DYN && !cur_have) r = make_uint2(0u, 0u);  // NaN radius (no transition found): border colour 0
+                const uint32_t next = __shfl_down_sync(0xffffffffu, r.x, 1);
+                w0[k] = __byte_perm(r.x, r.y, sel_a);
+                w1[k] = __byte_perm(r.y, next, 0x5410);
             }
-        }
-        uint32_t word[FR][M::kPx];
-        if (!DYN && M::kInterp == VR180_INTER_LANCZOS4) {  // a tap row's weights serve every frame of the item
-#pragma unroll
-            for (int k = 0; k < M::kPx; ++k) {
-                uint32_t r[FR];
-                sample_item<M, FR>(buf, (uint32_t)frame_pitch, pc[k], (uint32_t)pitch, r);
-#pragma unroll
-                for (int fr = 0; fr < FR; ++fr) res[fr][k] = r[fr];
-            }
-        }
-#pragma unroll
-        for (int fr = 0; fr < FR; ++fr) {
-            if (!DYN && M::kInterp != VR180_INTER_LANCZOS4) {
-#pragma unroll
-                for (int k = 0; k < M::kPx; ++k) res[fr][k] = M::sample(buf + fr * frame_pitch, pc[k], (uint32_t)pitch);
-            }
-            // re-pack frame fr right away: its shuffles are in flight while the next frame is sampled
-#pragma unroll
-            for (int k = 0; k < M::kPx; ++k)
-                word[fr][k] = __byte_perm(res[fr][k], __shfl_down_sync(0xffffffffu, res[fr][k], 1), out_sel);
-        }
-        const int o = n & (OB - 1);
-        if (n >= OB) mbar_wait(s_oempty + o * 8, (uint32_t)(n / OB + 1) & 1u);  // store n - OB has read out[o]
-        if (flags & 1u) {
+            const int o = n & (OB - 1);
+            if (n >= OB) mbar_wait(s_oempty + o * 8, (uint32_t)(n / OB + 1) & 1u);  // store n - OB has read out[o]
             const uint32_t ob = outp + o * kOutItemBytes;
 #pragma unroll
-            for (int fr = 0; fr < FR; ++fr)
-#pragma unroll
-                for (int k = 0; k < M::kPx; ++k) sts32(ob + fr * kOutTileBytes + k * kOutStep, word[fr][k]);
+            for (int k = 0; k < M::kPx; ++k) {
+                sts32(ob + k * kRowBytes, w0[k]);
+                if (flags & 1u) sts32(ob + k * kRowBytes + 4, w1[k]);
+            }
+            fence_proxy_async();
+            __syncwarp();
+            if (flags & 2u) mbar_arrive(s_ofull + o * 8);
+            if (++st == S) { st = 0; ph ^= 1u; }
         }
-        fence_proxy_async();
-        __syncwarp();
-        if (flags & 2u) mbar_arrive(s_ofull + o * 8);  // this warp's rows of item n are in out[o]; it has left stage st
-        if (++st == S) { st = 0; ph ^= 1u; }
+    } else {
+        // The 3-byte results [c0 c1 c2 .] of a warp step are re-packed into words of the dense out tile with ONE
+        // shuffle: every lane fetches the pixel of lane + 1; lanes 4 m + i, i < 3, then hold word 3 m + i of the row
+        // segment (12 bytes of 4 pixels = 3 words): [c0 c1 c2 c0'], [c1 c2 c0' c1'], [c2 c0' c1' c2'].
+        const int sub = lane & 3;
+        const uint32_t out_sel = sub == 0 ? 0x4210u : (sub == 1 ? 0x5421u : 0x6542u);
+        const bool writer = sub != 3;
+        // this lane's word of step k inside the dense out tile
+        //   row patch: row 4 band + k, word 3 (lane >> 2) + sub
+        //   8 x 4 patch: row 4 band + (lane >> 3), byte 24 (kPx cg + k), word 3 ((lane & 7) >> 2) + sub
+        constexpr int kOutStep = M::kRowPatch ? kTileW * 3 : 24;
+        const int sw = band * (4 / M::kPx) + cg;  // sampling warp index; with row patches it owns rows kPx sw .. kPx sw + kPx - 1
+        uint32_t outp = s_out + (M::kRowPatch ? (M::kPx * sw) * (kTileW * 3) + (3 * (lane >> 2) + sub) * 4
+                                              : (4 * band + (lane >> 3)) * (kTileW * 3) + M::kPx * cg * 24 +
+                                                    (3 * ((lane & 7) >> 2) + sub) * 4);
+        uint32_t flags = (writer ? 1u : 0u) | (lane == 0 ? 2u : 0u);
+        // opaque to the compiler: otherwise it re-derives them from S2R SR_TID.X inside the frame loop
+        asm volatile("" : "+r"(outp), "+r"(flags));
+
+        int st = 0;
+        uint32_t ph = 0;
+        typename M::Pixel cur[M::kPx];  // DYN: constants of the current radius
+        double cur_rad = CUDART_NAN;
+        bool cur_have = false;
+    #pragma unroll
+        for (int k = 0; k < M::kPx; ++k) cur[k] = pc[k];
+        for (int n = 0; n < n_items; ++n) {
+            mbar_wait(s_full + st * 8, ph);
+            const uint32_t buf = s_stage + st * stage_stride;
+            uint32_t res[FR][M::kPx];
+            if (DYN) {
+                // The per-pixel constants depend on the frame only through its radius: they are rebuilt when the radius
+                // changes (a static rig gives runs of equal radii; both eyes of a frame always share it).
+                const int f = f0 + ((NV == 2) ? (n >> 1) : n);  // FR == 1
+                const double rad = __ldg(dr.radius + f);
+                if (!(rad == cur_rad)) {
+                    const int2 org = s_org[st];
+                    cur_have = rad == rad;
+    #pragma unroll
+                    for (int k = 0; k < M::kPx; ++k) {
+                        const int qx = denorm_q<M>(nx[k], rad, dr.cx), qy = denorm_q<M>(ny[k], rad, dr.cy);
+                        const int off = ((qy >> M::kShift) - M::kLo - org.y) * pitch + M::kBpp * ((qx >> M::kShift) - M::kLo) - org.x;
+                        M::set_offset(cur[k], off, cur_have);
+                        M::weights(cur[k], qx & 31, qy & 31, tab);
+                    }
+                    cur_rad = rad;
+                }
+    #pragma unroll
+                for (int k = 0; k < M::kPx; ++k) {
+                    const uint32_t r = M::sample(buf, cur[k], (uint32_t)pitch);
+                    res[0][k] = cur_have ? r : 0u;  // NaN radius (no transition found): border colour
+                }
+            }
+            uint32_t word[FR][M::kPx];
+            if (!DYN && M::kInterp == VR180_INTER_LANCZOS4) {  // a tap row's weights serve every frame of the item
+    #pragma unroll
+                for (int k = 0; k < M::kPx; ++k) {
+                    uint32_t r[FR];
+                    sample_item<M, FR>(buf, (uint32_t)frame_pitch, pc[k], (uint32_t)pitch, r);
+    #pragma unroll
+                    for (int fr = 0; fr < FR; ++fr) res[fr][k] = r[fr];
+                }
+            }
+    #pragma unroll
+            for (int fr = 0; fr < FR; ++fr) {
+                if (!DYN && M::kInterp != VR180_INTER_LANCZOS4) {
+    #pragma unroll
+                    for (int k = 0; k < M::kPx; ++k) res[fr][k] = M::sample(buf + fr * frame_pitch, pc[k], (uint32_t)pitch);
+                }
+                // re-pack frame fr right away: its shuffles are in flight while the next frame is sampled
+    #pragma unroll
+                for (int k = 0; k < M::kPx; ++k)
+                    word[fr][k] = __byte_perm(res[fr][k], __shfl_down_sync(0xffffffffu, res[fr][k], 1), out_sel);
+            }
+            const int o = n & (OB - 1);
+            if (n >= OB) mbar_wait(s_oempty + o * 8, (uint32_t)(n / OB + 1) & 1u);  // store n - OB has read out[o]
+            if (flags & 1u) {
+                const uint32_t ob = outp + o * kOutItemBytes;
+    #pragma unroll
+                for (int fr = 0; fr < FR; ++fr)
+    #pragma unroll
+                    for (int k = 0; k < M::kPx; ++k) sts32(ob + fr * kOutTileBytes + k * kOutStep, word[fr][k]);
+            }
+            fence_proxy_async();
+            __syncwarp();
+            if (flags & 2u) mbar_arrive(s_ofull + o * 8);  // this warp's rows of item n are in out[o]; it has left stage st
+            if (++st == S) { st = 0; ph ^= 1u; }
+        }
     }
 }
 
@@ -268,7 +330,7 @@ template <class M, bool DYN, int FR>
 __global__ void __launch_bounds__(kThreads, 4)
 k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_chain_t chain0,
              const __grid_constant__ vr180_chain_t chain1, const __grid_constant__ TiledParams tp,
-             const __grid_constant__ TmaMaps tm) {
+             const __grid_constant__ TmaMaps tm, const __grid_constant__ Remap16 x16) {
     constexpr int kPx = M::kPx;
     constexpr int kChainUnroll = (FR == 1 && !DYN) ? kPx : 1;  // pixels of a thread whose chains are interleaved
     constexpr int kWarpsPerBand = 4 / kPx;  // a band = 4 output rows x 32 columns = 4 / kPx warps of 8 kPx columns
@@ -522,7 +584,8 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
     // ... and tiles whose item (FR frames x box rows x pitch) does not fit the staging area
     // (a chunk with varying radii runs one-frame items; FR-frame items of a DYN launch are FR one-frame boxes, each 128-byte aligned)
     // (a launch that gives its CTAs single frames pairs the two eyes of a shared map in one item: see VPAIR)
-    const bool vpair = !DYN && FR == 1 && nv == 2;
+    constexpr bool kPairItems = M::kOutTiles >= 4;  // two out tiles per item: the 16-bit modes keep one-frame items
+    const bool vpair = kPairItems && !DYN && FR == 1 && nv == 2;
     const int fr_item = dynr ? 1 : (vpair ? 2 : FR);
     auto stage_fits = [&](int box_rows, int pitch_bytes) {
         const int rect = box_rows * pitch_bytes;
@@ -534,8 +597,8 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
     auto inside_src = [&](int x_lo, int x_hi, int y_lo, int y_hi) {  // extreme integer coordinates of the tile
         return x_lo - M::kLo >= 0 && x_hi + M::kHi <= src_cols - 1 && y_lo - M::kLo >= 0 && y_hi + M::kHi <= src_rows - 1;
     };
-    bool fast = full_tile && rc.wbytes <= kPitchMax && rc.rsel < kRowSizes && mnx > -32768 && mny > -32768 &&
-                mxx < 32767 && mxy < 32767 && stage_fits(rc.box_rows, max(rc.wbytes, kPitchMin)) &&
+    bool fast = full_tile && rc.wbytes <= M::kPitchMax && rc.rsel < kRowSizes && mnx > -32768 && mny > -32768 &&
+                mxx < 32767 && mxy < 32767 && stage_fits(rc.box_rows, tight_pitch<M>(rc.wbytes)) &&
                 (tp.zero_border || inside_src(mnx, mxx, mny, mxy));
     int dyn_wbytes = 0, dyn_nrows = 0;  // the largest rectangle over the frames of the chunk
     if (dynr) {
@@ -574,8 +637,8 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
         dyn_wbytes = __reduce_max_sync(0xffffffffu, dyn_wbytes);
         dyn_nrows = __reduce_max_sync(0xffffffffu, dyn_nrows);
         ok = __all_sync(0xffffffffu, ok);
-        fast = full_tile && ok && !nan_px && dyn_wbytes <= kPitchMax && box_rsel<M>(dyn_nrows) < kRowSizes &&
-               stage_fits(M::kRowsMin + box_rsel<M>(dyn_nrows) * kRowsStep, max(dyn_wbytes, kPitchMin));
+        fast = full_tile && ok && !nan_px && dyn_wbytes <= M::kPitchMax && box_rsel<M>(dyn_nrows) < kRowSizes &&
+               stage_fits(M::kRowsMin + box_rsel<M>(dyn_nrows) * kRowsStep, tight_pitch<M>(dyn_wbytes));
     }
 
     if (!fast) {  // per-pixel gather from global memory with full border handling (rare tiles)
@@ -591,7 +654,7 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
                             qx = denorm_q<M>(nx[k], rad, dr.cx);
                             qy = denorm_q<M>(ny[k], rad, dr.cy);
                         }
-                        gather_pixel<M>(a, f, i, j, v_begin, v_end, qx, qy, tp.tab);
+                        gather_pixel<M>(a, f, i, j, v_begin, v_end, qx, qy, tp.tab, x16.cval);
                     }
                 }
             }
@@ -601,12 +664,12 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
 
     // ---- row pitch of the stages = TMA box width: the kPitchCands smallest multiples of 16 bytes that hold the
     // rectangle compete (pitch_costs) ----------------------------------------------------------------------------
-    int pitch = max(dynr ? dyn_wbytes : rc.wbytes, kPitchMin);
+    int pitch = tight_pitch<M>(dynr ? dyn_wbytes : rc.wbytes);
     // (not worth ~100 instructions per thread when the tile serves only a few frames: tightest box then)
     if (!dynr && (f1 - f0) * nv >= 8) {
         if (sampler) pitch_costs<M>(sx[0], sy[0], rc, pitch, lane, s_cost);
         __syncthreads();
-        pitch = pick_pitch(s_cost, pitch, rc.box_rows, [&](int pe) { return stage_fits(rc.box_rows, pe); });
+        pitch = pick_pitch<M::kPitchStep, M::kPitchMax>(s_cost, pitch, rc.box_rows, [&](int pe) { return stage_fits(rc.box_rows, pe); });
     }
 
     // ---- per-pixel constants of the frame loop ------------------------------------------------------------
@@ -614,7 +677,7 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
 #pragma unroll
     for (int k = 0; k < kPx; ++k) {
         const int ix = sx[k] >> M::kShift, iy = sy[k] >> M::kShift;
-        const int off = (iy - M::kLo - rc.ry0) * pitch + 3 * (ix - M::kLo) - rc.bx0;
+        const int off = (iy - M::kLo - rc.ry0) * pitch + M::kBpp * (ix - M::kLo) - rc.bx0;
         M::set_offset(pc[k], off, true);
         if (sampler && !dynr) M::weights(pc[k], sx[k] & 31, sy[k] & 31, tp.tab);
     }
@@ -640,7 +703,7 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
         else         frame_loop<M, 1, DYN, 1>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, band, cg, dr, nx, ny, tp.tab);
     } else {
         // (a DYN launch has one-frame boxes: its equal-radii chunks run FR-frame items as FR boxes each)
-        if constexpr (!DYN && FR == 1) {
+        if constexpr (!DYN && FR == 1 && kPairItems) {
             if (nv == 2) frame_loop<M, 2, false, 2, true, true>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, band, cg, dr, nx, ny, tp.tab);
             else         frame_loop<M, 1, false, 1, false>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, band, cg, dr, nx, ny, tp.tab);
         } else {
@@ -711,7 +774,7 @@ __global__ void __launch_bounds__(kSamplers) k_pack_tiles(const float* __restric
 
 }  // namespace tiled
 
-static int tile_height_of(int interp) {
+static int tile_height_of(int interp) {  // (the 16-bit modes: as LinearP / Nearest)
     return interp == VR180_INTER_LINEAR || interp == VR180_INTER_NEAREST ? tiled::LinearP::kTileH
            : interp == VR180_INTER_CUBIC                                  ? tiled::Cubic::kTileH
            : interp == VR180_INTER_LANCZOS4                               ? tiled::Lanczos4::kTileH
@@ -804,18 +867,19 @@ static EncodeTiledFn encode_tiled_fn() {
     return fn;
 }
 
-// uint8 tensor (row_bytes, rows, frames) with byte strides (pitch, frame_stride); box (box_w, box_h, 1).
-// Out-of-bounds box elements are filled with zeros on loads and dropped on stores.
-static bool encode_u8_3d(CUtensorMap* out, const void* base, long long row_bytes, long long rows, long long frames,
-                         long long pitch, long long frame_stride, int box_w, int box_h, int box_d) {
+// uint8 (elem = 1) or uint16 (elem = 2) tensor (row_bytes / elem, rows, frames) with byte strides (pitch, frame_stride);
+// box (box_w_bytes / elem, box_h, box_d).  Out-of-bounds box elements are filled with zeros on loads and dropped on stores.
+static bool encode_3d(CUtensorMap* out, int elem, const void* base, long long row_bytes, long long rows, long long frames,
+                      long long pitch, long long frame_stride, int box_w_bytes, int box_h, int box_d) {
     EncodeTiledFn fn = encode_tiled_fn();
     if (!fn) return false;
     if (frames <= 1 || frame_stride < pitch * rows) frame_stride = ((pitch * rows + 15) / 16) * 16;  // unused when frames == 1
-    const cuuint64_t dims[3] = {(cuuint64_t)row_bytes, (cuuint64_t)rows, (cuuint64_t)(frames < 1 ? 1 : frames)};
+    const cuuint64_t dims[3] = {(cuuint64_t)(row_bytes / elem), (cuuint64_t)rows, (cuuint64_t)(frames < 1 ? 1 : frames)};
     const cuuint64_t strides[2] = {(cuuint64_t)pitch, (cuuint64_t)frame_stride};
-    const cuuint32_t box[3] = {(cuuint32_t)box_w, (cuuint32_t)box_h, (cuuint32_t)box_d};
+    const cuuint32_t box[3] = {(cuuint32_t)(box_w_bytes / elem), (cuuint32_t)box_h, (cuuint32_t)box_d};
     const cuuint32_t estr[3] = {1u, 1u, 1u};
-    return fn(out, CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(base), dims, strides, box, estr,
+    return fn(out, elem == 2 ? CU_TENSOR_MAP_DATA_TYPE_UINT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8, 3, const_cast<void*>(base), dims,
+              strides, box, estr,
               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
@@ -847,13 +911,15 @@ static int frames_per_cta(long long tiles, int n_frames, int views_per_cta = 1) 
 // TMA descriptors of a launch.  They depend only on the buffers' geometry: video loops call with the same buffers again
 // and again, so the last few sets are kept per host thread (a ring of batches cycles through a handful of buffers, and
 // 199 cuTensorMapEncodeTiled calls cost about as much host time as a single-pair launch takes on the GPU).
-// `fr`: frames per box (depth of the load and store boxes).  nullptr = a descriptor could not be encoded.
-const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int interp, int rows_min, int tile_h, int fr) {
+// `fr`: frames per box (depth of the load and store boxes); `bpp`: the mode's bytes per pixel -- part of the key, since
+// one allocation can be warped as uint8 and as uint16 with equal pointers, sizes and pitches.  nullptr = a descriptor could
+// not be encoded.
+const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int interp, int rows_min, int tile_h, int fr, int bpp) {
     using namespace tiled;
     struct Key {
         const void* src[2];
         long long pitch[2], fs[2];
-        int rows, cols, n_views, n_frames, H, mode, fr, pad;
+        int rows, cols, n_views, n_frames, H, mode, fr, bpp;
         const void* dst;
         long long dst_pitch, dst_fs;
     };
@@ -871,6 +937,7 @@ const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int interp, int rows_min
     key.H = a0.H;
     key.mode = interp;
     key.fr = fr;
+    key.bpp = bpp;
     key.dst = a0.dst;
     key.dst_pitch = a0.dst_pitch;
     key.dst_fs = a0.dst_frame_stride;
@@ -897,17 +964,19 @@ const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int interp, int rows_min
         memset(&hit->key, 0xff, sizeof(hit->key));  // invalid until every descriptor is encoded
         TmaMaps& t = hit->tm;
         memset(&t, 0, sizeof(t));
+        const int elem = bpp / 3;  // uint16 views for the 16-bit modes
+        const int pitch_min = elem == 2 ? Bpp6::kPitchMin : Bpp3::kPitchMin, pitch_step = elem == 2 ? Bpp6::kPitchStep : Bpp3::kPitchStep;
         for (int v = 0; v < a0.n_views; ++v) {
             const ViewArgs& vw = a0.view[v];
             for (int w = 0; w < kWidths; ++w)
                 for (int r = 0; r < kRowSizes; ++r)
-                    if (!encode_u8_3d(&t.src[v][w][r], vw.src, (long long)vw.cols * 3, vw.rows, a0.n_frames, vw.pitch,
-                                      vw.frame_stride, kPitchMin + w * kPitchStep, rows_min + r * kRowsStep, fr))
+                    if (!encode_3d(&t.src[v][w][r], elem, vw.src, (long long)vw.cols * bpp, vw.rows, a0.n_frames, vw.pitch,
+                                   vw.frame_stride, pitch_min + w * pitch_step, rows_min + r * kRowsStep, fr))
                         return nullptr;
         }
         if (a0.n_views == 1) memcpy(&t.src[1], &t.src[0], sizeof(t.src[0]));
-        if (!encode_u8_3d(&t.dst, a0.dst, a0.dst_pitch, a0.H, a0.n_frames, a0.dst_pitch, a0.dst_frame_stride, kTileW * 3,
-                          tile_h, fr))
+        if (!encode_3d(&t.dst, 1, a0.dst, a0.dst_pitch, a0.H, a0.n_frames, a0.dst_pitch, a0.dst_frame_stride, kTileW * bpp,
+                       tile_h, fr))
             return nullptr;
         hit->key = key;
     }
@@ -917,10 +986,10 @@ const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int interp, int rows_min
 
 template <class M, bool DYN, int FR>
 static int launch_mode(const RemapArgs& a0, const vr180_chain_t& c0, const vr180_chain_t& c1, const short* tab,
-                       cudaStream_t st) {
+                       const Remap16& x16, cudaStream_t st) {
     using namespace tiled;
     const int n_groups = a0.share_map ? 1 : a0.n_views;
-    const TmaMaps* tmp = tma_maps_for(a0, M::kInterp, M::kRowsMin, M::kTileH, DYN ? 1 : FR);
+    const TmaMaps* tmp = tma_maps_for(a0, M::kInterp, M::kRowsMin, M::kTileH, DYN ? 1 : FR, M::kBpp);
     if (!tmp) return VR180_ERR_UNSUPPORTED;
     const TmaMaps& tm = *tmp;
 
@@ -935,7 +1004,7 @@ static int launch_mode(const RemapArgs& a0, const vr180_chain_t& c0, const vr180
     tp.tiles_x = tiles_x;
     tp.n_tiles = tiles_x * tiles_y;
     tp.tab = tab;
-    tp.zero_border = zero_border(a);
+    tp.zero_border = zero_border(a, x16);
     tp.debug = tiled_debug_flags();
     const long long tiles = (long long)tiles_x * tiles_y * n_groups;
     int fpc = frames_per_cta(tiles, a.n_frames, a.share_map ? a.n_views : 1);
@@ -955,32 +1024,39 @@ static int launch_mode(const RemapArgs& a0, const vr180_chain_t& c0, const vr180
         match_std_chain(c, tp.std[a.view[g].chain_idx ? 1 : 0]);
     }
     dim3 grid((unsigned)tiles_x, (unsigned)tiles_y, (unsigned)(n_groups * chunks));  // z = chunk * n_groups + map group
-    k_warp_tiled<M, DYN, FR><<<grid, kThreads, Lay<M>::kSmemBytes, st>>>(a, c0, c1, tp, tm);
+    k_warp_tiled<M, DYN, FR><<<grid, kThreads, Lay<M>::kSmemBytes, st>>>(a, c0, c1, tp, tm, x16);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     VR180_CUDA(cudaGetLastError());
     return VR180_OK;
 }
 
-// FR = frames per pipeline item for `fpc` frames per CTA: 2 from two frames on, bicubic 4 from eight on
+// FR = frames per pipeline item for `fpc` frames per CTA: 2 from two frames on, bicubic 4 from eight on; the 16-bit
+// modes 1 (two out tiles of 6 KB per item would cost the fourth CTA per SM)
 template <class M>
-static int launch_tiled(const RemapArgs& a0, const vr180_chain_t& c0, const vr180_chain_t& c1, const short* tab, bool dyn,
-                        int fpc, cudaStream_t st) {
+static int launch_tiled(const RemapArgs& a0, const vr180_chain_t& c0, const vr180_chain_t& c1, const short* tab,
+                        const Remap16& x16, bool dyn, int fpc, cudaStream_t st) {
     if constexpr (M::kInterp == VR180_INTER_CUBIC) {
-        if (fpc >= 8) return dyn ? launch_mode<M, true, 4>(a0, c0, c1, tab, st) : launch_mode<M, false, 4>(a0, c0, c1, tab, st);
+        if (fpc >= 8) return dyn ? launch_mode<M, true, 4>(a0, c0, c1, tab, x16, st) : launch_mode<M, false, 4>(a0, c0, c1, tab, x16, st);
     }
-    if (fpc >= 2) return dyn ? launch_mode<M, true, 2>(a0, c0, c1, tab, st) : launch_mode<M, false, 2>(a0, c0, c1, tab, st);
-    return dyn ? launch_mode<M, true, 1>(a0, c0, c1, tab, st) : launch_mode<M, false, 1>(a0, c0, c1, tab, st);
+    if constexpr (M::kBpp == 3) {
+        if (fpc >= 2) return dyn ? launch_mode<M, true, 2>(a0, c0, c1, tab, x16, st) : launch_mode<M, false, 2>(a0, c0, c1, tab, x16, st);
+    }
+    return dyn ? launch_mode<M, true, 1>(a0, c0, c1, tab, x16, st) : launch_mode<M, false, 1>(a0, c0, c1, tab, x16, st);
 }
 
 // Host-side eligibility + launch.  Returns VR180_ERR_UNSUPPORTED when the request is outside the fast path (the
 // caller then launches the generic k_remap); any other value is final.  `weight_tab`: device copy of the weight table of
-// the requested interpolation (1024 x 16 bicubic, 1024 x 64 Lanczos4; unused otherwise).
+// the requested interpolation (1024 x 16 bicubic, 1024 x 64 Lanczos4; unused otherwise).  uint16: NEAREST and LINEAR
+// only (`x16.cval`: the border colour); CUBIC / LANCZOS4 keep the generic kernel.
 int launch_remap_tiled(const RemapArgs& a0, int channels, int interp, const vr180_chain_t& c0, const vr180_chain_t& c1,
-                       const short* weight_tab, cudaStream_t st) {
-    if (channels != 3 || a0.depth != VR180_DEPTH_8U) return VR180_ERR_UNSUPPORTED;
+                       const short* weight_tab, const Remap16& x16, cudaStream_t st) {
+    if (channels != 3 || (a0.depth != VR180_DEPTH_8U && a0.depth != VR180_DEPTH_16U)) return VR180_ERR_UNSUPPORTED;
     if (interp != VR180_INTER_NEAREST && interp != VR180_INTER_LINEAR && interp != VR180_INTER_CUBIC &&
         interp != VR180_INTER_LANCZOS4)
         return VR180_ERR_UNSUPPORTED;
+    const bool u16 = a0.depth == VR180_DEPTH_16U;
+    if (u16 && interp != VR180_INTER_NEAREST && interp != VR180_INTER_LINEAR) return VR180_ERR_UNSUPPORTED;
+    const long long bpp = u16 ? 6 : 3;
     if (interp == VR180_INTER_NEAREST)  // the fixed-point LUT is a 1/32-pixel grid; NEAREST rounds the float coordinate itself
         for (int v = 0; v < a0.n_views; ++v)
             if (a0.view[v].map_kind == VR180_MAPSRC_FIXED) return VR180_ERR_UNSUPPORTED;
@@ -988,14 +1064,14 @@ int launch_remap_tiled(const RemapArgs& a0, int channels, int interp, const vr18
     for (int v = 0; v < a0.n_views; ++v) {
         const ViewArgs& vw = a0.view[v];
         // TMA: 16-byte aligned base and strides
-        if (((uintptr_t)vw.src & 15) || (vw.pitch & 15) || (vw.frame_stride & 15) || vw.pitch < (long long)vw.cols * 3)
+        if (((uintptr_t)vw.src & 15) || (vw.pitch & 15) || (vw.frame_stride & 15) || vw.pitch < (long long)vw.cols * bpp)
             return VR180_ERR_UNSUPPORTED;
         if (a0.n_frames > 1 && vw.frame_stride < vw.pitch * vw.rows) return VR180_ERR_UNSUPPORTED;
         if (vw.rows != a0.view[0].rows || vw.cols != a0.view[0].cols) return VR180_ERR_UNSUPPORTED;
         // a TMA box must start at a 16-byte aligned global address: tile columns are multiples of 32 pixels (96
-        // bytes), so the eye's column offset inside the SBS frame has to be one too (an unaligned start traps
-        // with "illegal instruction" on B200, for loads and stores alike)
-        if ((vw.dst_x_offset * 3) & 15) return VR180_ERR_UNSUPPORTED;
+        // bytes; 192 at 16 bits), so the eye's column offset inside the SBS frame has to be one too (an unaligned start
+        // traps with "illegal instruction" on B200, for loads and stores alike).  uint16: a multiple of 8 pixels.
+        if ((vw.dst_x_offset * bpp) & 15) return VR180_ERR_UNSUPPORTED;
     }
     if (((uintptr_t)a0.dst & 15) || (a0.dst_pitch & 15) || (a0.dst_frame_stride & 15)) return VR180_ERR_UNSUPPORTED;
     if (a0.n_frames > 1 && a0.dst_frame_stride < a0.dst_pitch * a0.H) return VR180_ERR_UNSUPPORTED;
@@ -1012,7 +1088,7 @@ int launch_remap_tiled(const RemapArgs& a0, int channels, int interp, const vr18
     // 1206 us vs 217 / 245 / 310 / 548 / 690 / 827 / 1125 us.  VR180_TILED_DEBUG bit 1: whenever eligible; bit 2: never.
     const int kStreamMaxItems = a0.share_map ? 20 : 16;  // (frame, eye) rectangles per tile
     {
-        bool all_packed = !dyn;
+        bool all_packed = !dyn && !u16;  // (the streaming kernel's tile headers hold 8-bit box geometry)
         for (int g = 0; g < n_groups; ++g) all_packed = all_packed && a0.view[g].packed != nullptr;
         const int dbg = tiled_debug_flags();
         const int items = a0.n_frames * (a0.share_map ? a0.n_views : 1);
@@ -1028,11 +1104,15 @@ int launch_remap_tiled(const RemapArgs& a0, int channels, int interp, const vr18
     const int tile_h = tile_height_of(interp);
     const long long tiles = (long long)((a0.W + tiled::kTileW - 1) / tiled::kTileW) * ((a0.H + tile_h - 1) / tile_h) * n_groups;
     const int fpc = frames_per_cta(tiles, a0.n_frames, a0.share_map ? a0.n_views : 1);
-    if (interp == VR180_INTER_NEAREST) return launch_tiled<tiled::Nearest>(a0, c0, c1, nullptr, dyn, fpc, st);
-    if (interp == VR180_INTER_LINEAR) return launch_tiled<tiled::LinearP>(a0, c0, c1, nullptr, dyn, fpc, st);
+    if (u16) {
+        if (interp == VR180_INTER_NEAREST) return launch_tiled<tiled::Nearest16>(a0, c0, c1, nullptr, x16, dyn, fpc, st);
+        return launch_tiled<tiled::Linear16>(a0, c0, c1, nullptr, x16, dyn, fpc, st);
+    }
+    if (interp == VR180_INTER_NEAREST) return launch_tiled<tiled::Nearest>(a0, c0, c1, nullptr, x16, dyn, fpc, st);
+    if (interp == VR180_INTER_LINEAR) return launch_tiled<tiled::LinearP>(a0, c0, c1, nullptr, x16, dyn, fpc, st);
     if (!weight_tab) return VR180_ERR_UNSUPPORTED;
-    if (interp == VR180_INTER_LANCZOS4) return launch_tiled<tiled::Lanczos4>(a0, c0, c1, weight_tab, dyn, fpc, st);
-    return launch_tiled<tiled::Cubic>(a0, c0, c1, weight_tab, dyn, fpc, st);
+    if (interp == VR180_INTER_LANCZOS4) return launch_tiled<tiled::Lanczos4>(a0, c0, c1, weight_tab, x16, dyn, fpc, st);
+    return launch_tiled<tiled::Cubic>(a0, c0, c1, weight_tab, x16, dyn, fpc, st);
 }
 
 }  // namespace vr180

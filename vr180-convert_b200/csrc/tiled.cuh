@@ -27,6 +27,7 @@ constexpr int kRowsStep = 4, kRowSizes = 9;  // TMA load box heights: Mode::kRow
 // Staged row pitch = TMA box width (bytes), a multiple of 16 picked PER TILE: the smallest kPitchCands widths that
 // hold the tile's source rectangle are compared by the bank conflicts of the tile's own tap addresses (counted with
 // match.any in the prologue) plus the shared-memory wavefronts of the TMA write of the box itself.
+// (the 8-bit modes; the 16-bit modes have their own range, see Bpp6 -- every mode has kWidths widths)
 constexpr int kPitchMin = 96, kPitchMax = 256, kPitchStep = 16;
 constexpr int kWidths = (kPitchMax - kPitchMin) / kPitchStep + 1;  // 11 box widths
 constexpr int kPitchCands = 4;
@@ -36,7 +37,7 @@ constexpr int kOutBufs = 4;        // ofull / oempty barrier slots; out buffers 
 template <class M>
 struct Lay {
     static constexpr int kStageArea = M::kStageArea;
-    static constexpr int kOutArea = M::kOutTiles * M::kTileH * kTileW * 3;
+    static constexpr int kOutArea = M::kOutTiles * M::kTileH * kTileW * M::kBpp;
     static constexpr int kOffOut = kStageArea;
     static constexpr int kOffTrig = kOffOut + kOutArea;
     static constexpr int kOffRed = kOffTrig + 7 * 32 * 8;  // double[4][32] sincos of the tile's columns / rows, or chain_fast.cuh's tables [4 + 3][32]
@@ -77,8 +78,10 @@ struct TiledParams {
 
 // TMA descriptors of one launch (kernel parameter; the TMA unit reads them from the parameter bank).
 struct alignas(64) TmaMaps {
-    CUtensorMap src[2][kWidths][kRowSizes];  // [view][box bytes kPitchMin + 16 w][box rows kRowsMin + 8 r]: uint8 (cols * 3, rows, frames)
-    CUtensorMap dst;                   // uint8 (dst_pitch, H, frames), box (96, tile height, 1)
+    // [view][box bytes M::kPitchMin + M::kPitchStep w][box rows kRowsMin + 4 r]: uint8 (cols * 3, rows, frames), or for
+    // the 16-bit modes uint16 (cols * 3, rows, frames) -- a box is at most 256 elements wide, i.e. 512 bytes at 16 bits
+    CUtensorMap src[2][kWidths][kRowSizes];
+    CUtensorMap dst;  // uint8 (dst_pitch, H, frames), box (32 M::kBpp bytes, tile height, 1)
 };
 
 // ---- tile-packed LUT (include/vr180_b200.h, vr180_pack_lut_tiles) -----------------------------------------------
@@ -198,6 +201,17 @@ __device__ __forceinline__ uint32_t dp2a_hi_su(uint32_t w, uint32_t px, uint32_t
 }
 
 // ---- interpolation modes -------------------------------------------------------------------------------------
+// Bytes per pixel and staged row pitches of a mode.  kElem: bytes per element of the source's TMA view (box starts are
+// given to the TMA unit in elements).
+struct Bpp3 {  // uint8 x 3 channels
+    static constexpr int kBpp = 3, kElem = 1;
+    static constexpr int kPitchMin = tiled::kPitchMin, kPitchMax = tiled::kPitchMax, kPitchStep = tiled::kPitchStep;
+};
+struct Bpp6 {  // uint16 x 3 channels: a 32-pixel tile row's footprint is twice as wide, so are the boxes (192 .. 512 B)
+    static constexpr int kBpp = 6, kElem = 2;
+    static constexpr int kPitchMin = 192, kPitchMax = 512, kPitchStep = 32;
+};
+static_assert((Bpp6::kPitchMax - Bpp6::kPitchMin) / Bpp6::kPitchStep + 1 == kWidths, "TmaMaps holds kWidths box widths");
 // A mode fixes: pixels per thread (the per-pixel constants must stay in registers across the frames of the batch),
 // the tile height, the tap footprint (taps start kLo pixels / rows before the integer coordinate and end kHi after
 // it), the per-pixel constants and the sampling of one pixel from the staged rectangle.
@@ -210,7 +224,7 @@ __device__ __forceinline__ uint32_t dp2a_hi_su(uint32_t w, uint32_t px, uint32_t
 //        [a1.0 a1.3 a1.1 a0.0]
 // i.e. 5 PRMT per pixel instead of 4 SHF + 3 PRMT.  selA shares a register with the window offset (PRMT reads only
 // the low 16 bits of its selector; the address is one LEA.HI).
-struct LinearP {
+struct LinearP : Bpp3 {
     static constexpr int kPx = 4, kTileH = 32, kLo = 0, kHi = 1, kRowsMin = 32, kInterp = VR180_INTER_LINEAR;
     static constexpr int kShift = kInterBits;  // coordinates are 1/32-pixel fixed point: sx = cvRound(x * 32)
     __device__ static __forceinline__ int quant(float m) { return quantise(m); }
@@ -264,7 +278,7 @@ struct LinearP {
 };
 
 // INTER_NEAREST: ix = saturate_int16(cvRound(x)) (no sub-pixel grid), out = src[iy, ix].
-struct Nearest {
+struct Nearest : Bpp3 {
     static constexpr int kPx = 4, kTileH = 32, kLo = 0, kHi = 0, kRowsMin = 32, kInterp = VR180_INTER_NEAREST;
     static constexpr int kShift = 0;
     __device__ static __forceinline__ int quant(float m) { return cv_round(m); }
@@ -286,7 +300,7 @@ struct Nearest {
     }
 };
 
-struct Cubic {
+struct Cubic : Bpp3 {
     static constexpr int kPx = 2, kTileH = 16, kLo = 1, kHi = 2, kRowsMin = 16, kInterp = VR180_INTER_CUBIC;
     static constexpr int kShift = kInterBits;  // coordinates are 1/32-pixel fixed point: sx = cvRound(x * 32)
     __device__ static __forceinline__ int quant(float m) { return quantise(m); }
@@ -339,7 +353,7 @@ struct Cubic {
 // that a warp reads 512 contiguous bytes per tap row (straight from the table every lane would touch its own cache
 // line: 32 tag look-ups per load).  The 8 tap rows are 28-byte windows of the staged rectangle.  ~300 instructions
 // and ~120 shared-memory wavefronts per pixel step.
-struct Lanczos4 {
+struct Lanczos4 : Bpp3 {
     static constexpr int kPx = 1, kTileH = 8, kLo = 3, kHi = 4, kRowsMin = 16, kInterp = VR180_INTER_LANCZOS4;
     static constexpr bool kRowPatch = true;  // a warp = one output row of the tile
     static constexpr int kShift = kInterBits;  // coordinates are 1/32-pixel fixed point: sx = cvRound(x * 32)
@@ -409,6 +423,111 @@ struct Lanczos4 {
         uint32_t out[1];
         sample_frames<1>(sbuf, 0u, p, pitch, out);
         return out[0];
+    }
+};
+
+// ---- 16-bit modes (uint16 x 3 channels, 6 bytes per pixel) ------------------------------------------------------
+// cv::remap's float arithmetic for depths other than 8 bits, as sample16_linear / sample16_nearest (sampler.cuh) do it
+// on global memory.  Same tile shape, thread <-> pixel order and packed-LUT entries as LinearP / Nearest; one frame per
+// item and two 6 KB out buffers, so the 40 KB stage ring + 12 KB of out tiles take the bytes of the 8-bit layout (4 CTAs
+// per SM).  A pixel's row window (6 bytes nearest, 12 bytes bilinear) starts at a 2-byte aligned offset: its words are
+// read with LDS.32 and aligned with one PRMT per word pair, selector 0x3210 (window 4-byte aligned) or 0x5432 (window
+// at byte 2 of a word), which travels in the low 16 bits of the offset register (PRMT reads only those).
+__device__ __forceinline__ uint32_t osel16(int off, bool valid) {
+    return ((valid ? (uint32_t)off & ~3u : 0u) << 16) | ((off & 2) ? 0x5432u : 0x3210u);
+}
+__device__ __forceinline__ uint32_t prmt_osel(uint32_t a, uint32_t b, uint32_t osel) {  // PRMT with an offset | selector register
+    uint32_t d;
+    asm("prmt.b32 %0, %1, %2, %3;" : "=r"(d) : "r"(a), "r"(b), "r"(osel));
+    return d;
+}
+// u16 -> float as the bits 2^23 + v (one LOP3 / PRMT instead of I2F): lo / hi halfword of a word
+__device__ __forceinline__ float magic_lo(uint32_t t) { return __uint_as_float((t & 0xffffu) | 0x4B000000u); }
+__device__ __forceinline__ float magic_hi(uint32_t t) { return __uint_as_float(__byte_perm(t, 0x4B00u, 0x5432)); }
+
+// INTER_LINEAR: s = ((v00 w00 + v01 w01) + v10 w10) + v11 w11, every product and sum one rounded float32 operation, then
+// saturate(cvRound(s)).  Weights (32-ax or ax)(32-ay or ay) / 1024 are exact floats.  Two exact shortcuts:
+//   * v w == fma(2^23 + v, w, -2^23 w): the exact value of the right side is v w, and an FMA rounds once, so the product
+//     is __fmul_rn(v, w) without converting v (2^23 w = k 2^13 is exact);
+//   * cvRound(s) == the low 16 bits of fl(s + 2^23) for 0 <= s < 2^22 (the add rounds to an integer, half to even).
+//     0 <= s < 65535.5 holds: the taps are >= 0 and s exceeds max(v) <= 65535 by at most a few float ulps, so no
+//     saturation is needed either.
+struct Linear16 : Bpp6 {
+    static constexpr int kPx = 4, kTileH = 32, kLo = 0, kHi = 1, kRowsMin = 32, kInterp = VR180_INTER_LINEAR;
+    static constexpr int kShift = kInterBits;
+    __device__ static __forceinline__ int quant(float m) { return quantise(m); }
+    static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 2;
+    static constexpr bool kRowPatch = true;
+    struct Pixel {
+        uint32_t osel;  // window byte offset (4-aligned) << 16 | alignment selector
+        float w[4];     // w00 w01 w10 w11
+    };
+    __device__ static __forceinline__ void set_offset(Pixel& p, int off, bool valid) { p.osel = osel16(off, valid); }
+    __device__ static __forceinline__ void weights(Pixel& p, int ax, int ay, const short*) {
+        p.w[0] = (float)((32 - ax) * (32 - ay)) * (1.0f / 1024.0f);
+        p.w[1] = (float)(ax * (32 - ay)) * (1.0f / 1024.0f);
+        p.w[2] = (float)((32 - ax) * ay) * (1.0f / 1024.0f);
+        p.w[3] = (float)(ax * ay) * (1.0f / 1024.0f);
+    }
+    // One output pixel: .x = [c0 c1], low half of .y = c2.  Row window = words t0 t1 t2 = [c0 c1] [c2 c0'] [c1' c2']
+    // (after alignment); the fourth word is loaded only for a window at byte 2, into a0's register (a0 is dead once t0
+    // exists), and selector 0x3210 ignores it otherwise.
+    __device__ static __forceinline__ uint2 sample(uint32_t sbuf, const Pixel& p, uint32_t pitch) {
+        const uint32_t row0 = sbuf + (p.osel >> 16);
+        uint32_t t0, t1, t2, u0, u1, u2;
+        asm volatile(
+            "{\n\t.reg .pred p;\n\t.reg .b32 a0, a1, a2, b0, b1, b2, m;\n\t"
+            "and.b32 m, %8, 2;\n\t"
+            "setp.ne.u32 p, m, 0;\n\t"
+            "ld.shared.u32 a0, [%6];\n\t"
+            "ld.shared.u32 a1, [%6+4];\n\t"
+            "ld.shared.u32 a2, [%6+8];\n\t"
+            "ld.shared.u32 b0, [%7];\n\t"
+            "ld.shared.u32 b1, [%7+4];\n\t"
+            "ld.shared.u32 b2, [%7+8];\n\t"
+            "prmt.b32 %0, a0, a1, %8;\n\t"
+            "prmt.b32 %3, b0, b1, %8;\n\t"
+            "@p ld.shared.u32 a0, [%6+12];\n\t"
+            "@p ld.shared.u32 b0, [%7+12];\n\t"
+            "prmt.b32 %1, a1, a2, %8;\n\t"
+            "prmt.b32 %4, b1, b2, %8;\n\t"
+            "prmt.b32 %2, a2, a0, %8;\n\t"
+            "prmt.b32 %5, b2, b0, %8;\n\t}"
+            : "=&r"(t0), "=&r"(t1), "=&r"(t2), "=&r"(u0), "=&r"(u1), "=&r"(u2)
+            : "r"(row0), "r"(row0 + pitch), "r"(p.osel));
+        float c[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) c[i] = __fmul_rn(p.w[i], -8388608.0f);
+        auto px = [&](float v00, float v01, float v10, float v11) {
+            float s = __fadd_rn(__fmaf_rn(v00, p.w[0], c[0]), __fmaf_rn(v01, p.w[1], c[1]));
+            s = __fadd_rn(s, __fmaf_rn(v10, p.w[2], c[2]));
+            s = __fadd_rn(s, __fmaf_rn(v11, p.w[3], c[3]));
+            return __float_as_uint(__fadd_rn(s, 8388608.0f));  // cvRound(s) in the low 16 bits
+        };
+        const uint32_t r0 = px(magic_lo(t0), magic_hi(t1), magic_lo(u0), magic_hi(u1));
+        const uint32_t r1 = px(magic_hi(t0), magic_lo(t2), magic_hi(u0), magic_lo(u2));
+        const uint32_t r2 = px(magic_lo(t1), magic_hi(t2), magic_lo(u1), magic_hi(u2));
+        return make_uint2(__byte_perm(r0, r1, 0x5410), r2);
+    }
+};
+
+// INTER_NEAREST: out = src[iy, ix], a copy of the pixel's 6 bytes = [c0 c1] [c2 .] after alignment
+struct Nearest16 : Bpp6 {
+    static constexpr int kPx = 4, kTileH = 32, kLo = 0, kHi = 0, kRowsMin = 32, kInterp = VR180_INTER_NEAREST;
+    static constexpr int kShift = 0;
+    __device__ static __forceinline__ int quant(float m) { return cv_round(m); }
+    static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 2;
+    static constexpr bool kRowPatch = true;
+    struct Pixel {
+        uint32_t osel;
+    };
+    __device__ static __forceinline__ void set_offset(Pixel& p, int off, bool valid) { p.osel = osel16(off, valid); }
+    __device__ static __forceinline__ void weights(Pixel&, int, int, const short*) {}
+    __device__ static __forceinline__ uint2 sample(uint32_t sbuf, const Pixel& p, uint32_t) {
+        uint32_t a0, a1;
+        asm volatile("ld.shared.u32 %0, [%2];\n\tld.shared.u32 %1, [%2+4];" : "=r"(a0), "=r"(a1) : "r"(sbuf + (p.osel >> 16)));
+        // c2 = a1.lo (selector 0x3210) or a1.hi (0x5432): the same selector on (a1, a1)
+        return make_uint2(prmt_osel(a0, a1, p.osel), prmt_osel(a1, a1, p.osel));
     }
 };
 
@@ -482,8 +601,8 @@ struct TileRect {
 template <class M>
 __device__ __forceinline__ TileRect tile_rect(int mnx, int mxx, int mny, int mxy) {
     TileRect r;
-    r.bx0 = (3 * (mnx - M::kLo)) & ~15;
-    r.wbytes = ((3 * (mxx + M::kHi + 1) + 15) & ~15) - r.bx0;
+    r.bx0 = (M::kBpp * (mnx - M::kLo)) & ~15;
+    r.wbytes = ((M::kBpp * (mxx + M::kHi + 1) + 15) & ~15) - r.bx0;
     r.ry0 = mny - M::kLo;
     r.nrows = mxy + M::kHi + 1 - r.ry0;
     r.rsel = box_rsel<M>(r.nrows);
@@ -499,11 +618,11 @@ __device__ __forceinline__ TileRect tile_rect(int mnx, int mxx, int mny, int mxy
 // caller); pick_pitch, after a barrier: the cheapest candidate that is <= kPitchMax and that `fits` admits.
 template <class M>
 __device__ __forceinline__ void pitch_costs(int sx0, int sy0, const TileRect& rc, int pitch0, int lane, int* s_cost) {
-    const int row = (sy0 >> M::kShift) - M::kLo - rc.ry0, col = 3 * ((sx0 >> M::kShift) - M::kLo) - rc.bx0;
+    const int row = (sy0 >> M::kShift) - M::kLo - rc.ry0, col = M::kBpp * ((sx0 >> M::kShift) - M::kLo) - rc.bx0;
     int cost = 0;
 #pragma unroll
     for (int e = 0; e < kPitchCands; ++e) {
-        const int w = (row * (pitch0 + kPitchStep * e) + col) >> 2;
+        const int w = (row * (pitch0 + M::kPitchStep * e) + col) >> 2;
         const unsigned same = __match_any_sync(0xffffffffu, w);
         const bool leader = (__ffs(same) - 1) == lane;  // one lane per distinct word
         const unsigned lm = __ballot_sync(0xffffffffu, leader);
@@ -517,28 +636,45 @@ __device__ __forceinline__ void pitch_costs(int sx0, int sy0, const TileRect& rc
                          : M::kInterp == VR180_INTER_CUBIC ? 16 : 56;
     if (lane < kPitchCands) atomicAdd(&s_cost[lane], cost * (kStepsPerWarp * kLoads));
 }
-template <class Fits>
+template <int Step = kPitchStep, int Max = kPitchMax, class Fits>  // (a mode's M::kPitchStep, M::kPitchMax)
 __device__ __forceinline__ int pick_pitch(const int* s_cost, int pitch0, int box_rows, Fits fits) {
     int best = 0, best_cost = INT_MAX;
 #pragma unroll
     for (int e = 0; e < kPitchCands; ++e) {
-        const int pe = pitch0 + kPitchStep * e;
+        const int pe = pitch0 + Step * e;
         const int c = s_cost[e] + box_rows * pe / 64;
-        if (pe <= kPitchMax && fits(pe) && c < best_cost) { best_cost = c; best = e; }
+        if (pe <= Max && fits(pe) && c < best_cost) { best_cost = c; best = e; }
     }
-    return pitch0 + kPitchStep * best;
+    return pitch0 + Step * best;
+}
+// the tightest admissible pitch of a rectangle `wbytes` wide (a multiple of 16): >= M::kPitchMin, a multiple of M::kPitchStep
+template <class M>
+__device__ __forceinline__ int tight_pitch(int wbytes) {
+    const int p = max(wbytes, M::kPitchMin);
+    if constexpr (M::kPitchStep == 16) return p;
+    else return (p + M::kPitchStep - 1) & -M::kPitchStep;
 }
 
 // Per-pixel gather from global memory with full border handling (the tiles that are not staged): one output pixel
 // (i, j) of frame f for the views v_begin .. v_end - 1, which share the quantised coordinates (qx, qy).
+// 16-bit modes: sample16_linear / nearest16 with the border colour `cval` (Remap16::cval).
 template <class M>
 __device__ __forceinline__ void gather_pixel(const RemapArgs& a, int f, int i, int j, int v_begin, int v_end, int qx, int qy,
-                                             const short* tab) {
+                                             const short* tab, const float* cval = nullptr) {
     uint8_t* drow = a.dst + (long long)f * a.dst_frame_stride + (long long)j * a.dst_pitch;
     for (int v = v_begin; v < v_end; ++v) {
         const ViewArgs& vw = a.view[v];
         Src s{vw.src + (long long)f * vw.frame_stride, vw.rows, vw.cols, vw.pitch};
         int px[3];
+        if constexpr (M::kBpp == 6) {
+            if (M::kInterp == VR180_INTER_NEAREST) nearest16<3>(s, sat16(qx), sat16(qy), a.border_mode, cval, px);
+            else sample16_linear<3>(s, qx, qy, a.border_mode, cval, px);
+            uint16_t* o = reinterpret_cast<uint16_t*>(drow) + (long long)(vw.dst_x_offset + i) * 3;
+            o[0] = (uint16_t)px[0];
+            o[1] = (uint16_t)px[1];
+            o[2] = (uint16_t)px[2];
+            continue;
+        }
         if (M::kInterp == VR180_INTER_NEAREST)
             fetch_tap<3>(s, sat16(qx), sat16(qy), a.border_mode, a.bv, px);
         else if (M::kInterp == VR180_INTER_LINEAR)
@@ -567,9 +703,14 @@ __device__ __forceinline__ void sample_item(uint32_t sbuf, uint32_t frame_bytes,
 }
 
 // ---- host ----------------------------------------------------------------------------------------------------
-// BORDER_CONSTANT with a zero colour: TMA's out-of-bounds zero fill is the border
+// BORDER_CONSTANT with a zero colour: TMA's out-of-bounds zero fill is the border.  16-bit requests: the colour
+// saturated to 16 bits (x16.cval).
 inline int zero_border(const RemapArgs& a) {
     return (a.border_mode == VR180_BORDER_CONSTANT && !(a.bv[0] | a.bv[1] | a.bv[2])) ? 1 : 0;
+}
+inline int zero_border(const RemapArgs& a, const Remap16& x16) {
+    if (a.depth != VR180_DEPTH_16U) return zero_border(a);
+    return (a.border_mode == VR180_BORDER_CONSTANT && x16.cval[0] == 0.f && x16.cval[1] == 0.f && x16.cval[2] == 0.f) ? 1 : 0;
 }
 // The kernel's dynamic shared-memory limit, raised once per device; `dev` = the current device
 template <auto Kernel>
@@ -587,7 +728,8 @@ int max_dyn_smem_once(int bytes, int& dev) {
 }  // namespace tiled
 
 // tiled.cu
-const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int interp, int rows_min, int tile_h, int fr);
+// bpp: bytes per pixel of the mode (3: uint8 views, 6: uint16 views with the 16-bit modes' box widths)
+const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int interp, int rows_min, int tile_h, int fr, int bpp = 3);
 int tiled_debug_flags();
 // stream.cu: tiles streamed through persistent CTAs (tile-packed LUT, a few frames per launch);
 // VR180_ERR_UNSUPPORTED = not eligible
