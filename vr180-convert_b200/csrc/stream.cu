@@ -72,7 +72,7 @@ __device__ __forceinline__ UnitGeom unit_geom(const int4& raw, int zero_border, 
     g.bx0 = rc.bx0;
     g.org = 3 * (h.mnx - M::kLo) - rc.bx0;  // byte offset of the tile's first tap column in the box
     g.ry0 = rc.ry0;
-    g.pitch = kPitchMin + kPitchStep * ((h.flags >> 8) & 15);
+    g.pitch = M::kPitchMin + M::kPitchStep * ((h.flags >> 8) & 15);
     g.rsel = (h.flags >> 12) & 15;
     g.rect_bytes = (M::kRowsMin + g.rsel * kRowsStep) * g.pitch;
     g.eye_pitch = (g.rect_bytes + 127) & ~127;
@@ -118,6 +118,7 @@ template <class M>
 __global__ void __launch_bounds__(kThreads, kStreamCtas)
 k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ StreamParams sp,
               const __grid_constant__ TmaMaps tm) {
+    static_assert(M::kBpp == 3, "tile headers hold 8-bit box geometry");
     constexpr int kPx = M::kPx;
     constexpr int kOB = SLay<M>::kOB, kOutTileBytes = SLay<M>::kOutTileBytes, kSlotBytes = SLay<M>::kSlotBytes;
     constexpr int kOutItemBytes = SLay<M>::kOutItemBytes;
@@ -171,7 +172,7 @@ k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ Strea
             const UnitGeom g = unit_geom<M>(hdr, sp.zero_border, src_cols, src_rows);
             if (!g.fast) continue;
             const int ty = tile / sp.tiles_x, tx = tile - ty * sp.tiles_x;
-            const CUtensorMap* const map0 = &tm.src[grp][(g.pitch - kPitchMin) / kPitchStep][g.rsel];
+            const CUtensorMap* const map0 = &tm.src[grp][(g.pitch - M::kPitchMin) / M::kPitchStep][g.rsel];
             // The tile's rectangles (frame-major, eye-minor: they all share the tile's coordinates) travel two per item when
             // two fit one slot: two box loads on one barrier, one hand-shake with the sampling warps, two tile stores.
             const int n_rects = a.n_frames * nv, per_item = 2 * g.eye_pitch <= kSlotBytes ? 2 : 1;
@@ -199,10 +200,9 @@ k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ Strea
 
     // ---- sampling warps ----
     const int sw = warp;  // owns rows kPx sw .. kPx sw + kPx - 1 of a tile, column = lane
-    const int sub = lane & 3;
-    const uint32_t out_sel = sub == 0 ? 0x4210u : (sub == 1 ? 0x5421u : 0x6542u);
-    uint32_t outp = s_out + (kPx * sw) * (kTileW * 3) + (3 * (lane >> 2) + sub) * 4;
-    uint32_t flags = (sub != 3 ? 1u : 0u) | (lane == 0 ? 2u : 0u);
+    const uint32_t out_sel = M::out_sel(lane);
+    uint32_t outp = s_out + (kPx * sw) * (kTileW * 3) + M::out_offset(lane);
+    uint32_t flags = (M::writer(lane) ? 1u : 0u) | (lane == 0 ? 2u : 0u);
     asm volatile("" : "+r"(outp), "+r"(flags));
 
     // Tiles that are not staged are only noted (s_slow) while the CTA streams; they are gathered per pixel afterwards,
@@ -272,18 +272,12 @@ k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ Strea
                 const uint32_t ob = outp + o * kOutItemBytes;
 #pragma unroll
                 for (int v = 0; v < EYES; ++v) {
-                    uint32_t word[kPx];
+                    uint32_t word[kPx][M::kOutWords];
 #pragma unroll
-                    for (int k = 0; k < kPx; ++k) {
-                        const uint32_t r = M::sample(buf + v * g.eye_pitch, pc[k], (uint32_t)g.pitch);
-                        word[k] = __byte_perm(r, __shfl_down_sync(0xffffffffu, r, 1), out_sel);
-                    }
+                    for (int k = 0; k < kPx; ++k) M::repack(M::sample(buf + v * g.eye_pitch, pc[k], (uint32_t)g.pitch), out_sel, word[k]);
                     // (after the first rectangle's sampling, which does not need the out buffer yet)
                     if (v == 0 && n >= kOB) mbar_wait(s_oempty + o * 8, (uint32_t)(n / kOB + 1) & 1u);  // store n - kOB has read out[o]
-                    if (flags & 1u) {
-#pragma unroll
-                        for (int k = 0; k < kPx; ++k) sts32(ob + v * kOutTileBytes + k * (kTileW * 3), word[k]);
-                    }
+                    M::store(ob + v * kOutTileBytes, kTileW * 3, word, flags & 1u);
                 }
                 fence_proxy_async();
                 __syncwarp();

@@ -30,11 +30,9 @@
 //              6 LDS.32 per pixel (2 rows x 12 bytes, the third word only for a byte offset of 3), funnel shifts
 //              to byte-align, PRMT to pair the taps, 2 x dp2a (16-bit weight x 8-bit pixel) per channel:
 //              (sum_t w_t p_t + 512) >> 10  ==  (sum_t 64 w_t p_t + 32768) >> 16, i.e. byte 2 of the dp2a chain.
-//              Bicubic: a warp step = an 8 x 4 patch; 4 rows x 16-byte windows, the pixel's 16 int16 table
-//              weights (OpenCV's 1024 x 16 table, tables.cuh) live in 8 registers, 2 x dp2a (s16 x u8) per
-//              channel and row, clip((acc + 16384) >> 15).
-//   store      the 3-byte results of a step are re-packed with ONE shuffle (every lane fetches the pixel of
-//              lane + 1; lanes 4 m + i, i < 3, then hold word 3 m + i of the row segment) into a dense output
+//              Bicubic: 4 rows x 16-byte windows, the pixel's 16 int16 table weights (OpenCV's 1024 x 16 table,
+//              tables.cuh) live in 8 registers, 2 x dp2a (s16 x u8) per channel and row, clip((acc + 16384) >> 15).
+//   store      the results of a step are re-packed with ONE shuffle (tiled.cuh: Bpp3 / Bpp6) into a dense output
 //              tile in shared memory; the producer writes the item's tiles into the eye's half of the SBS frames
 //              with one TMA store (full 32-byte sectors, no STG) and hands the buffer back once it has been read.
 // Tiles whose footprint is unbounded (NaN / huge coordinates) or exceeds the staging buffer, and partial edge
@@ -82,7 +80,7 @@ struct TileGeom {
 template <class M, int NV, bool DYN, int FR, bool SPLIT = false, bool VPAIR = false>  // FR: frames per item (2: one box load / tile store / barrier round per 2 frames)
 __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm, int v_begin, int f0, int f1,
                                            const typename M::Pixel (&pc)[M::kPx], const TileGeom& tg, const int pitch,
-                                           uint8_t* smem, int band, int cg, const DynRadius& dr,
+                                           uint8_t* smem, int sw, const DynRadius& dr,
                                            const double (&nx)[M::kPx], const double (&ny)[M::kPx], const short* tab) {
     static_assert(FR == 1 || !DYN, "a per-frame radius gives every frame its own rectangle");
     static_assert(M::kOutTiles / FR >= 2, "at least two out buffers of one item each");
@@ -93,7 +91,7 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
     uint32_t s_stage = smem_u32(smem);
     asm volatile("" : "+r"(s_stage));  // opaque: otherwise the window base is re-derived (S2R SR_CgaCtaId + MOV + LEA) in every item
     const uint32_t s_full = s_stage + Lay<M>::kOffBar;
-    const uint32_t s_ofull = s_full + 2 * kMaxStages * 8, s_oempty = s_ofull + kOutBufs * 8, s_out = s_stage + Lay<M>::kOffOut;
+    const uint32_t s_ofull = s_full + kMaxStages * 8, s_oempty = s_ofull + kOutBufs * 8, s_out = s_stage + Lay<M>::kOffOut;
 
     int2* const s_org = reinterpret_cast<int2*>(smem + Lay<M>::kOffOrg);
     // item n = FR consecutive frames of one view; a chunk with an odd frame count ends with a phantom frame: the
@@ -173,154 +171,74 @@ __device__ __forceinline__ void frame_loop(const RemapArgs& a, const TmaMaps& tm
     }
 
     // ---- sampling warps ----
-    if constexpr (M::kBpp == 6) {
-        // 16-bit modes, one-frame items.  The 6-byte results (.x = [c0 c1], .y = [c2 .]) of a warp step are re-packed
-        // with ONE shuffle: lanes 2 m and 2 m + 1 hold the 12 bytes = words 3 m .. 3 m + 2 of the row segment; lane
-        // 2 m + 1 sends its [c0' c1'] to lane 2 m, which stores [c0 c1] and [c2 c0'], and lane 2 m + 1 stores [c1' c2'].
-        static_assert(FR == 1 && !VPAIR, "a 16-bit item is one frame");
-        constexpr int kRowBytes = kTileW * M::kBpp;  // 192: one row of the out tile
-        const bool odd = (lane & 1) != 0;
-        const uint32_t sel_a = odd ? 0x5432u : 0x3210u;
-        const int sw = band * (4 / M::kPx) + cg;  // the warp owns rows kPx sw .. kPx sw + kPx - 1 of the tile
-        uint32_t outp = s_out + (M::kPx * sw) * kRowBytes + 12 * (lane >> 1) + (odd ? 8 : 0);
-        uint32_t flags = (odd ? 0u : 1u) | (lane == 0 ? 2u : 0u);
-        asm volatile("" : "+r"(outp), "+r"(flags));
-        int st = 0;
-        uint32_t ph = 0;
-        typename M::Pixel cur[M::kPx];  // DYN: constants of the current radius
-        double cur_rad = CUDART_NAN;
-        bool cur_have = false;
-#pragma unroll
-        for (int k = 0; k < M::kPx; ++k) cur[k] = pc[k];
-        for (int n = 0; n < n_items; ++n) {
-            mbar_wait(s_full + st * 8, ph);
-            const uint32_t buf = s_stage + st * stage_stride;
-            if (DYN) {  // constants rebuilt when the radius changes, as for 8 bits
-                const int f = f0 + ((NV == 2) ? (n >> 1) : n);
-                const double rad = __ldg(dr.radius + f);
-                if (!(rad == cur_rad)) {
-                    const int2 org = s_org[st];
-                    cur_have = rad == rad;
-#pragma unroll
-                    for (int k = 0; k < M::kPx; ++k) {
-                        const int qx = denorm_q<M>(nx[k], rad, dr.cx), qy = denorm_q<M>(ny[k], rad, dr.cy);
-                        const int off = ((qy >> M::kShift) - M::kLo - org.y) * pitch + M::kBpp * ((qx >> M::kShift) - M::kLo) - org.x;
-                        M::set_offset(cur[k], off, cur_have);
-                        M::weights(cur[k], qx & 31, qy & 31, tab);
-                    }
-                    cur_rad = rad;
-                }
-            }
-            uint32_t w0[M::kPx], w1[M::kPx];
-#pragma unroll
-            for (int k = 0; k < M::kPx; ++k) {
-                uint2 r = M::sample(buf, DYN ? cur[k] : pc[k], (uint32_t)pitch);
-                if (DYN && !cur_have) r = make_uint2(0u, 0u);  // NaN radius (no transition found): border colour 0
-                const uint32_t next = __shfl_down_sync(0xffffffffu, r.x, 1);
-                w0[k] = __byte_perm(r.x, r.y, sel_a);
-                w1[k] = __byte_perm(r.y, next, 0x5410);
-            }
-            const int o = n & (OB - 1);
-            if (n >= OB) mbar_wait(s_oempty + o * 8, (uint32_t)(n / OB + 1) & 1u);  // store n - OB has read out[o]
-            const uint32_t ob = outp + o * kOutItemBytes;
-#pragma unroll
-            for (int k = 0; k < M::kPx; ++k) {
-                sts32(ob + k * kRowBytes, w0[k]);
-                if (flags & 1u) sts32(ob + k * kRowBytes + 4, w1[k]);
-            }
-            fence_proxy_async();
-            __syncwarp();
-            if (flags & 2u) mbar_arrive(s_ofull + o * 8);
-            if (++st == S) { st = 0; ph ^= 1u; }
-        }
-    } else {
-        // The 3-byte results [c0 c1 c2 .] of a warp step are re-packed into words of the dense out tile with ONE
-        // shuffle: every lane fetches the pixel of lane + 1; lanes 4 m + i, i < 3, then hold word 3 m + i of the row
-        // segment (12 bytes of 4 pixels = 3 words): [c0 c1 c2 c0'], [c1 c2 c0' c1'], [c2 c0' c1' c2'].
-        const int sub = lane & 3;
-        const uint32_t out_sel = sub == 0 ? 0x4210u : (sub == 1 ? 0x5421u : 0x6542u);
-        const bool writer = sub != 3;
-        // this lane's word of step k inside the dense out tile
-        //   row patch: row 4 band + k, word 3 (lane >> 2) + sub
-        //   8 x 4 patch: row 4 band + (lane >> 3), byte 24 (kPx cg + k), word 3 ((lane & 7) >> 2) + sub
-        constexpr int kOutStep = M::kRowPatch ? kTileW * 3 : 24;
-        const int sw = band * (4 / M::kPx) + cg;  // sampling warp index; with row patches it owns rows kPx sw .. kPx sw + kPx - 1
-        uint32_t outp = s_out + (M::kRowPatch ? (M::kPx * sw) * (kTileW * 3) + (3 * (lane >> 2) + sub) * 4
-                                              : (4 * band + (lane >> 3)) * (kTileW * 3) + M::kPx * cg * 24 +
-                                                    (3 * ((lane & 7) >> 2) + sub) * 4);
-        uint32_t flags = (writer ? 1u : 0u) | (lane == 0 ? 2u : 0u);
-        // opaque to the compiler: otherwise it re-derives them from S2R SR_TID.X inside the frame loop
-        asm volatile("" : "+r"(outp), "+r"(flags));
+    // Pixel k of a thread is column `lane`, row kPx sw + k of the tile.  Each frame is re-packed (M::sample_repack) right
+    // after it is sampled: its shuffles are in flight while the next frame is sampled.
+    static_assert(M::kBpp == 3 || (FR == 1 && !VPAIR), "a 16-bit item is one frame");
+    using Px = typename M::Px;
+    constexpr int kRowBytes = kTileW * M::kBpp;  // one row of the out tile
+    const uint32_t out_sel = M::out_sel(lane);
+    const bool writer = M::writer(lane);
+    uint32_t outp = s_out + (M::kPx * sw) * kRowBytes + M::out_offset(lane);
+    uint32_t flags = (writer ? 1u : 0u) | (lane == 0 ? 2u : 0u);
+    // opaque to the compiler: otherwise it re-derives them from S2R SR_TID.X inside the frame loop
+    asm volatile("" : "+r"(outp), "+r"(flags));
 
-        int st = 0;
-        uint32_t ph = 0;
-        typename M::Pixel cur[M::kPx];  // DYN: constants of the current radius
-        double cur_rad = CUDART_NAN;
-        bool cur_have = false;
-    #pragma unroll
-        for (int k = 0; k < M::kPx; ++k) cur[k] = pc[k];
-        for (int n = 0; n < n_items; ++n) {
-            mbar_wait(s_full + st * 8, ph);
-            const uint32_t buf = s_stage + st * stage_stride;
-            uint32_t res[FR][M::kPx];
-            if (DYN) {
-                // The per-pixel constants depend on the frame only through its radius: they are rebuilt when the radius
-                // changes (a static rig gives runs of equal radii; both eyes of a frame always share it).
-                const int f = f0 + ((NV == 2) ? (n >> 1) : n);  // FR == 1
-                const double rad = __ldg(dr.radius + f);
-                if (!(rad == cur_rad)) {
-                    const int2 org = s_org[st];
-                    cur_have = rad == rad;
-    #pragma unroll
-                    for (int k = 0; k < M::kPx; ++k) {
-                        const int qx = denorm_q<M>(nx[k], rad, dr.cx), qy = denorm_q<M>(ny[k], rad, dr.cy);
-                        const int off = ((qy >> M::kShift) - M::kLo - org.y) * pitch + M::kBpp * ((qx >> M::kShift) - M::kLo) - org.x;
-                        M::set_offset(cur[k], off, cur_have);
-                        M::weights(cur[k], qx & 31, qy & 31, tab);
-                    }
-                    cur_rad = rad;
-                }
-    #pragma unroll
+    int st = 0;
+    uint32_t ph = 0;
+    typename M::Pixel cur[M::kPx];  // DYN: constants of the current radius
+    double cur_rad = CUDART_NAN;
+    bool cur_have = false;
+#pragma unroll
+    for (int k = 0; k < M::kPx; ++k) cur[k] = pc[k];
+    for (int n = 0; n < n_items; ++n) {
+        mbar_wait(s_full + st * 8, ph);
+        const uint32_t buf = s_stage + st * stage_stride;
+        Px res[FR][M::kPx];  // fixed-radius Lanczos4: the item's frames, sampled together
+        if (DYN) {
+            // The per-pixel constants depend on the frame only through its radius: they are rebuilt when the radius
+            // changes (a static rig gives runs of equal radii; both eyes of a frame always share it).
+            const int f = f0 + ((NV == 2) ? (n >> 1) : n);  // FR == 1
+            const double rad = __ldg(dr.radius + f);
+            if (!(rad == cur_rad)) {
+                const int2 org = s_org[st];
+                cur_have = rad == rad;
+#pragma unroll
                 for (int k = 0; k < M::kPx; ++k) {
-                    const uint32_t r = M::sample(buf, cur[k], (uint32_t)pitch);
-                    res[0][k] = cur_have ? r : 0u;  // NaN radius (no transition found): border colour
+                    const int qx = denorm_q<M>(nx[k], rad, dr.cx), qy = denorm_q<M>(ny[k], rad, dr.cy);
+                    stage_pixel<M>(cur[k], qx, qy, org.x, org.y, pitch, cur_have, true, tab);
                 }
+                cur_rad = rad;
             }
-            uint32_t word[FR][M::kPx];
-            if (!DYN && M::kInterp == VR180_INTER_LANCZOS4) {  // a tap row's weights serve every frame of the item
-    #pragma unroll
-                for (int k = 0; k < M::kPx; ++k) {
-                    uint32_t r[FR];
-                    sample_item<M, FR>(buf, (uint32_t)frame_pitch, pc[k], (uint32_t)pitch, r);
-    #pragma unroll
-                    for (int fr = 0; fr < FR; ++fr) res[fr][k] = r[fr];
-                }
+        } else if constexpr (M::kInterp == VR180_INTER_LANCZOS4) {  // a tap row's weights serve every frame of the item
+#pragma unroll
+            for (int k = 0; k < M::kPx; ++k) {
+                uint32_t r[FR];
+                M::template sample_frames<FR>(buf, (uint32_t)frame_pitch, pc[k], (uint32_t)pitch, r);
+#pragma unroll
+                for (int fr = 0; fr < FR; ++fr) res[fr][k] = r[fr];
             }
-    #pragma unroll
-            for (int fr = 0; fr < FR; ++fr) {
-                if (!DYN && M::kInterp != VR180_INTER_LANCZOS4) {
-    #pragma unroll
-                    for (int k = 0; k < M::kPx; ++k) res[fr][k] = M::sample(buf + fr * frame_pitch, pc[k], (uint32_t)pitch);
-                }
-                // re-pack frame fr right away: its shuffles are in flight while the next frame is sampled
-    #pragma unroll
-                for (int k = 0; k < M::kPx; ++k)
-                    word[fr][k] = __byte_perm(res[fr][k], __shfl_down_sync(0xffffffffu, res[fr][k], 1), out_sel);
-            }
-            const int o = n & (OB - 1);
-            if (n >= OB) mbar_wait(s_oempty + o * 8, (uint32_t)(n / OB + 1) & 1u);  // store n - OB has read out[o]
-            if (flags & 1u) {
-                const uint32_t ob = outp + o * kOutItemBytes;
-    #pragma unroll
-                for (int fr = 0; fr < FR; ++fr)
-    #pragma unroll
-                    for (int k = 0; k < M::kPx; ++k) sts32(ob + fr * kOutTileBytes + k * kOutStep, word[fr][k]);
-            }
-            fence_proxy_async();
-            __syncwarp();
-            if (flags & 2u) mbar_arrive(s_ofull + o * 8);  // this warp's rows of item n are in out[o]; it has left stage st
-            if (++st == S) { st = 0; ph ^= 1u; }
         }
+        uint32_t word[FR][M::kPx][M::kOutWords];
+#pragma unroll
+        for (int fr = 0; fr < FR; ++fr) {
+            M::template sample_repack<M::kPx>([&](int k) -> Px {
+                if (DYN) {
+                    const Px r = M::sample(buf, cur[k], (uint32_t)pitch);
+                    return cur_have ? r : Px{};  // NaN radius (no transition found): border colour
+                }
+                if (M::kInterp == VR180_INTER_LANCZOS4) return res[fr][k];
+                return M::sample(buf + fr * frame_pitch, pc[k], (uint32_t)pitch);
+            }, out_sel, word[fr]);
+        }
+        const int o = n & (OB - 1);
+        if (n >= OB) mbar_wait(s_oempty + o * 8, (uint32_t)(n / OB + 1) & 1u);  // store n - OB has read out[o]
+        const uint32_t ob = outp + o * kOutItemBytes;
+#pragma unroll
+        for (int fr = 0; fr < FR; ++fr) M::store(ob + fr * kOutTileBytes, kRowBytes, word[fr], flags & 1u);
+        fence_proxy_async();
+        __syncwarp();
+        if (flags & 2u) mbar_arrive(s_ofull + o * 8);  // this warp's rows of item n are in out[o]; it has left stage st
+        if (++st == S) { st = 0; ph ^= 1u; }
     }
 }
 
@@ -333,17 +251,16 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
              const __grid_constant__ TmaMaps tm, const __grid_constant__ Remap16 x16) {
     constexpr int kPx = M::kPx;
     constexpr int kChainUnroll = (FR == 1 && !DYN) ? kPx : 1;  // pixels of a thread whose chains are interleaved
-    constexpr int kWarpsPerBand = 4 / kPx;  // a band = 4 output rows x 32 columns = 4 / kPx warps of 8 kPx columns
     extern __shared__ __align__(1024) uint8_t smem[];
     double* s_trig = reinterpret_cast<double*>(smem + Lay<M>::kOffTrig);  // [4][32]
     int4* s_red = reinterpret_cast<int4*>(smem + Lay<M>::kOffRed);        // [8]: box of each sampling warp
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    if (tid < 2 * kMaxStages + 2 * kOutBufs) {  // one barrier per thread: a single-frame launch is latency bound, and one
-        const uint32_t bars = smem_u32(smem + Lay<M>::kOffBar);  // thread initialising all 24 kept the whole CTA waiting
-        // layout: full[kMaxStages] (1: the producer + tx bytes), empty[kMaxStages] (one arrive per sampling warp),
-        //         ofull[kOutBufs] (one arrive per sampling warp), oempty[kOutBufs] (1: the producer)
-        const bool by_warps = (tid >= kMaxStages && tid < 2 * kMaxStages + kOutBufs);
+    if (tid < kMaxStages + 2 * kOutBufs) {  // one barrier per thread: a single-frame launch is latency bound, and one
+        const uint32_t bars = smem_u32(smem + Lay<M>::kOffBar);  // thread initialising all 16 kept the whole CTA waiting
+        // layout: full[kMaxStages] (1: the producer + tx bytes), ofull[kOutBufs] (one arrive per sampling warp),
+        //         oempty[kOutBufs] (1: the producer)
+        const bool by_warps = (tid >= kMaxStages && tid < kMaxStages + kOutBufs);
         mbar_init(bars + tid * 8, by_warps ? kSamplers / 32 : 1);
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");  // visible to the async proxy (TMA)
     }
@@ -360,11 +277,8 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
     const int v_begin = g, v_end = a.share_map ? a.n_views : g + 1, nv = v_end - v_begin;
     const int f0 = chunk * a.frames_per_cta, f1 = min(a.n_frames, f0 + a.frames_per_cta);
     const bool sampler = warp < kSamplers / 32;  // the last warp = TMA producer: no pixels of its own
-    const int sw = warp & (kSamplers / 32 - 1), band = sw / kWarpsPerBand, cg = sw % kWarpsPerBand;
-    // pixel k of this thread (tile-local): 8 x 4 patches: column lx + 8 k, row ly; row patches: column lane, row 4 band + k
-    const int lx = M::kRowPatch ? lane : 8 * kPx * cg + (lane & 7), ly = M::kRowPatch ? kPx * sw : 4 * band + (lane >> 3);
-    auto pcol = [&](int k) { return M::kRowPatch ? lx : lx + 8 * k; };
-    auto prow = [&](int k) { return M::kRowPatch ? ly + k : ly; };
+    const int sw = warp & (kSamplers / 32 - 1);
+    const int py = kPx * sw;  // pixel k of this thread (tile-local): column lane, row py + k
     const bool full_tile = (x0 + kTileW <= a.W) && (y0 + M::kTileH <= a.H);
 
     // tile-packed LUT: the tile's header (every thread: the producer warp needs the rectangle too)
@@ -406,8 +320,8 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
             __syncthreads();
             const bool lat_is_y = ch.ops[1].iparam != 0;
             auto seed = [&](int k, ChainState& s) {
-                const double s_row = s_trig[64 + prow(k)], c_row = s_trig[96 + prow(k)];
-                const double s_col = s_trig[pcol(k)], c_col = s_trig[32 + pcol(k)];
+                const double s_row = s_trig[64 + (py + k)], c_row = s_trig[96 + (py + k)];
+                const double s_col = s_trig[lane], c_col = s_trig[32 + lane];
                 s.mode = MODE_VEC3;
                 s.x = s.y = s.r = s.ux = s.uy = 0.0;
                 if (lat_is_y) {  // lat from the row, lon from the column
@@ -426,16 +340,14 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
                 // constant-bank operands (no indexed LDC, no register copies); one pixel at a time, not unrolled: a CTA
                 // that serves one frame runs this exactly once, and instruction fetch is what such a launch waits for
                 auto std_eval = [&](const StdChain& c) {
-                    // v = scale A + B (chain_fast.cuh).  A thread's pixels share their column (row patches) or their row
-                    // (8 x 4 patches): that side of the table is read once, the other per pixel -- these are 8-byte
-                    // loads on the pipe that bounds the kernel
-                    const bool x_fixed = M::kRowPatch ? !c.lat_is_y : (c.lat_is_y != 0);  // side X = rows iff lat_is_y
-                    const int fi = M::kRowPatch ? lx : ly;
-                    const double* const ft = s_trig + (x_fixed ? 0 : 128) + fi;
+                    // v = scale A + B (chain_fast.cuh).  A thread's pixels share their column: that side of the table is
+                    // read once, the other per pixel -- these are 8-byte loads on the pipe that bounds the kernel
+                    const bool x_fixed = !c.lat_is_y;  // side X = rows iff lat_is_y
+                    const double* const ft = s_trig + (x_fixed ? 0 : 128) + lane;
                     const double f0 = ft[0], f1 = ft[32], f2 = ft[64], f3 = x_fixed ? ft[96] : 0.0;
 #pragma unroll(kChainUnroll)
                     for (int k = 0; k < kPx; ++k) {
-                        const int vi = M::kRowPatch ? prow(k) : pcol(k);
+                        const int vi = py + k;
                         double vx, vy, vz;
                         if (x_fixed) {  // (uniform)
                             vx = fma(f0, s_trig[128 + vi], f1); vy = fma(f0, s_trig[160 + vi], f2); vz = fma(f0, s_trig[192 + vi], f3);
@@ -476,8 +388,8 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
 #pragma unroll 1
             for (int k = 0; k < kPx; ++k) {
                 double xs, ys;
-                if (dyn) eval_chain_normalised(ch, x0 + pcol(k), y0 + prow(k), xs, ys);
-                else eval_chain(ch, x0 + pcol(k), y0 + prow(k), xs, ys);
+                if (dyn) eval_chain_normalised(ch, x0 + lane, y0 + (py + k), xs, ys);
+                else eval_chain(ch, x0 + lane, y0 + (py + k), xs, ys);
                 const int qx = M::quant(__double2float_rn(xs)), qy = M::quant(__double2float_rn(ys));
 #pragma unroll
                 for (int kk = 0; kk < kPx; ++kk)
@@ -503,7 +415,7 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
 #pragma unroll
         for (int k = 0; k < kPx; ++k) {
             if (unpacked) break;
-            const int i = x0 + pcol(k), j = y0 + prow(k);
+            const int i = x0 + lane, j = y0 + (py + k);
             sx[k] = sy[k] = (int)0x80000000;
             if (i < a.W && j < a.H) {
                 if (mv.map_kind == VR180_MAPSRC_FLOAT2) {
@@ -645,7 +557,7 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
         if (sampler) {
 #pragma unroll
             for (int k = 0; k < kPx; ++k) {
-                const int i = x0 + pcol(k), j = y0 + prow(k);
+                const int i = x0 + lane, j = y0 + (py + k);
                 if (i < a.W && j < a.H) {
                     for (int f = f0; f < f1; ++f) {
                         int qx = sx[k], qy = sy[k];
@@ -669,18 +581,13 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
     if (!dynr && (f1 - f0) * nv >= 8) {
         if (sampler) pitch_costs<M>(sx[0], sy[0], rc, pitch, lane, s_cost);
         __syncthreads();
-        pitch = pick_pitch<M::kPitchStep, M::kPitchMax>(s_cost, pitch, rc.box_rows, [&](int pe) { return stage_fits(rc.box_rows, pe); });
+        pitch = pick_pitch<M>(s_cost, pitch, rc.box_rows, [&](int pe) { return stage_fits(rc.box_rows, pe); });
     }
 
     // ---- per-pixel constants of the frame loop ------------------------------------------------------------
     typename M::Pixel pc[kPx];
 #pragma unroll
-    for (int k = 0; k < kPx; ++k) {
-        const int ix = sx[k] >> M::kShift, iy = sy[k] >> M::kShift;
-        const int off = (iy - M::kLo - rc.ry0) * pitch + M::kBpp * (ix - M::kLo) - rc.bx0;
-        M::set_offset(pc[k], off, true);
-        if (sampler && !dynr) M::weights(pc[k], sx[k] & 31, sy[k] & 31, tp.tab);
-    }
+    for (int k = 0; k < kPx; ++k) stage_pixel<M>(pc[k], sx[k], sy[k], rc.bx0, rc.ry0, pitch, true, sampler && !dynr, tp.tab);
     if constexpr (M::kWeightSmem != 0) {
         // fixed radius: the pixel's weights do not change from frame to frame -> private copy in shared memory
         // (written and read by this thread only: no barrier)
@@ -699,16 +606,16 @@ k_warp_tiled(const __grid_constant__ RemapArgs a, const __grid_constant__ vr180_
     tg.x0 = x0;
     tg.y0 = y0;
     if (DYN && dynr) {
-        if (nv == 2) frame_loop<M, 2, DYN, 1>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, band, cg, dr, nx, ny, tp.tab);
-        else         frame_loop<M, 1, DYN, 1>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, band, cg, dr, nx, ny, tp.tab);
+        if (nv == 2) frame_loop<M, 2, DYN, 1>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, sw, dr, nx, ny, tp.tab);
+        else         frame_loop<M, 1, DYN, 1>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, sw, dr, nx, ny, tp.tab);
     } else {
         // (a DYN launch has one-frame boxes: its equal-radii chunks run FR-frame items as FR boxes each)
         if constexpr (!DYN && FR == 1 && kPairItems) {
-            if (nv == 2) frame_loop<M, 2, false, 2, true, true>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, band, cg, dr, nx, ny, tp.tab);
-            else         frame_loop<M, 1, false, 1, false>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, band, cg, dr, nx, ny, tp.tab);
+            if (nv == 2) frame_loop<M, 2, false, 2, true, true>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, sw, dr, nx, ny, tp.tab);
+            else         frame_loop<M, 1, false, 1, false>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, sw, dr, nx, ny, tp.tab);
         } else {
-            if (nv == 2) frame_loop<M, 2, false, FR, DYN>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, band, cg, dr, nx, ny, tp.tab);
-            else         frame_loop<M, 1, false, FR, DYN>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, band, cg, dr, nx, ny, tp.tab);
+            if (nv == 2) frame_loop<M, 2, false, FR, DYN>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, sw, dr, nx, ny, tp.tab);
+            else         frame_loop<M, 1, false, FR, DYN>(a, tm, v_begin, f0, f1, pc, tg, pitch, smem, sw, dr, nx, ny, tp.tab);
         }
     }
 }
@@ -745,14 +652,14 @@ __global__ void __launch_bounds__(kSamplers) k_pack_tiles(const float* __restric
     // Geometry of the tile's source rectangle for the tile-streaming kernel (stream.cu), which has no time to derive it
     // per launch: box rows, and the row pitch (= TMA box width) that k_warp_tiled's choice gives a stage slot.
     const TileRect rc = tile_rect<M>(mnx, mxx, mny, mxy);
-    const bool stageable = ok && rc.wbytes <= kPitchMax && rc.rsel < kRowSizes;
-    const int pitch0 = max(rc.wbytes, kPitchMin);
+    const bool stageable = ok && rc.wbytes <= M::kPitchMax && rc.rsel < kRowSizes;
+    const int pitch0 = max(rc.wbytes, M::kPitchMin);
     if (stageable) pitch_costs<M>(sx[0], sy[0], rc, pitch0, lane, s_cost);  // (CTA-uniform)
     __syncthreads();
-    const int pitch = !stageable ? kPitchMin : pick_pitch(s_cost, pitch0, rc.box_rows, [&](int pe) {
+    const int pitch = !stageable ? M::kPitchMin : pick_pitch<M>(s_cost, pitch0, rc.box_rows, [&](int pe) {
         return pe == pitch0 || rc.box_rows * pe <= kStreamSlotBytes<M>;
     });
-    const int widx = (pitch - kPitchMin) / kPitchStep;
+    const int widx = (pitch - M::kPitchMin) / M::kPitchStep;
     if (tid == 0) {
         int4 h;
         h.x = (mnx & 0xffff) | (mxx << 16);

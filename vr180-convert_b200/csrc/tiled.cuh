@@ -17,19 +17,17 @@
 namespace vr180 {
 namespace tiled {
 
-constexpr int kTileW = 32;      // output tile width.  Per step a warp covers 32 pixels: one output row (bilinear: the
+constexpr int kTileW = 32;      // output tile width.  Per step a warp covers 32 pixels of one output row (bilinear: the
                                 // taps of a row are ~26 consecutive source pixels = ~20 consecutive words, one
-                                // wavefront per load while the row stays in one source row) or an 8 x 4 patch (bicubic)
+                                // wavefront per load while the row stays in one source row)
 constexpr int kSamplers = 256;  // 8 sampling warps
 constexpr int kThreads = kSamplers + 32;  // + the TMA producer warp
 constexpr int kMaxStages = 8;   // ring depth is chosen per tile: kStageArea / (bytes of the tile's source rectangle)
 constexpr int kRowsStep = 4, kRowSizes = 9;  // TMA load box heights: Mode::kRowsMin + 4 r, r < 9
-// Staged row pitch = TMA box width (bytes), a multiple of 16 picked PER TILE: the smallest kPitchCands widths that
-// hold the tile's source rectangle are compared by the bank conflicts of the tile's own tap addresses (counted with
-// match.any in the prologue) plus the shared-memory wavefronts of the TMA write of the box itself.
-// (the 8-bit modes; the 16-bit modes have their own range, see Bpp6 -- every mode has kWidths widths)
-constexpr int kPitchMin = 96, kPitchMax = 256, kPitchStep = 16;
-constexpr int kWidths = (kPitchMax - kPitchMin) / kPitchStep + 1;  // 11 box widths
+// Staged row pitch = TMA box width (bytes), a multiple of 16 picked PER TILE among the mode's widths (M::kPitchMin ..
+// M::kPitchMax, see Bpp3 / Bpp6): the smallest kPitchCands widths that hold the tile's source rectangle are compared by
+// the bank conflicts of the tile's own tap addresses (counted with match.any in the prologue) plus the shared-memory
+// wavefronts of the TMA write of the box itself.
 constexpr int kPitchCands = 4;
 constexpr int kStageAreaDefault = 40960;  // >= 1 two-frame stage of the largest admissible rectangle (64 rows x 256 B)
 constexpr int kOutBufs = 4;        // ofull / oempty barrier slots; out buffers in use: M::kOutTiles / FR (a power of two <= 4)
@@ -41,8 +39,8 @@ struct Lay {
     static constexpr int kOffOut = kStageArea;
     static constexpr int kOffTrig = kOffOut + kOutArea;
     static constexpr int kOffRed = kOffTrig + 7 * 32 * 8;  // double[4][32] sincos of the tile's columns / rows, or chain_fast.cuh's tables [4 + 3][32]
-    static constexpr int kOffBar = kOffRed + 8 * 4 * 4;  // full[kMaxStages], empty[kMaxStages], ofull[kOutBufs], oempty[kOutBufs]
-    static constexpr int kOffOrg = kOffBar + (2 * kMaxStages + 2 * kOutBufs) * 8;  // int2 origin of the rectangle in each stage
+    static constexpr int kOffBar = kOffRed + 8 * 4 * 4;  // full[kMaxStages], ofull[kOutBufs], oempty[kOutBufs]
+    static constexpr int kOffOrg = kOffBar + (kMaxStages + 2 * kOutBufs) * 8;  // int2 origin of the rectangle in each stage
     static constexpr int kOffExt = kOffOrg + kMaxStages * 8;                         // double[8][4] per-warp normalised extremes
     static constexpr int kOffCost = kOffExt + 8 * 4 * 8;                             // int[kPitchCands] candidate pitch costs
     static constexpr int kOffW = (kOffCost + 16 + 15) & ~15;  // M::kWeightSmem bytes of per-pixel weights (Lanczos4)
@@ -76,14 +74,6 @@ struct TiledParams {
     StdChain std[2];
 };
 
-// TMA descriptors of one launch (kernel parameter; the TMA unit reads them from the parameter bank).
-struct alignas(64) TmaMaps {
-    // [view][box bytes M::kPitchMin + M::kPitchStep w][box rows kRowsMin + 4 r]: uint8 (cols * 3, rows, frames), or for
-    // the 16-bit modes uint16 (cols * 3, rows, frames) -- a box is at most 256 elements wide, i.e. 512 bytes at 16 bits
-    CUtensorMap src[2][kWidths][kRowSizes];
-    CUtensorMap dst;  // uint8 (dst_pitch, H, frames), box (32 M::kBpp bytes, tile height, 1)
-};
-
 // ---- tile-packed LUT (include/vr180_b200.h, vr180_pack_lut_tiles) -----------------------------------------------
 // buffer = [n_tiles x PackedHdr][pad to 256 bytes][n_tiles x (256 threads x kPx) uint32, thread-major]
 // entry  = (ix - mnx) | (iy - mny) << 8 | ax << 16 | ay << 21     (ax = ay = 0 for INTER_NEAREST)
@@ -93,9 +83,9 @@ struct PackedHdr {
     int pad;
 };
 constexpr int kHdrPackable = 1;   // full tile, finite unsaturated coordinates, extents <= 255: the entries are valid
-constexpr int kHdrStageable = 2;  // the source rectangle fits a TMA box of this mode (width <= kPitchMax, rows <= the largest box)
+constexpr int kHdrStageable = 2;  // the source rectangle fits a TMA box of this mode (width <= M::kPitchMax, rows <= the largest box)
 constexpr int kHdrFitsSlot = 4;   // ... and one stage slot of the tile-streaming kernel
-// bits 8-11: (row pitch - kPitchMin) / kPitchStep chosen for the tile; bits 12-15: box rows = kRowsMin + kRowsStep * r
+// bits 8-11: (row pitch - M::kPitchMin) / M::kPitchStep chosen for the tile; bits 12-15: box rows = kRowsMin + kRowsStep * r
 static_assert(sizeof(PackedHdr) == 16, "PackedHdr is one 128-bit load");
 __host__ __device__ inline size_t packed_entries_offset(long long n_tiles) { return ((size_t)n_tiles * 16 + 255) & ~(size_t)255; }
 // the header as loaded (the streaming kernel keeps the prefetched next header in this form: three live registers)
@@ -201,17 +191,87 @@ __device__ __forceinline__ uint32_t dp2a_hi_su(uint32_t w, uint32_t px, uint32_t
 }
 
 // ---- interpolation modes -------------------------------------------------------------------------------------
-// Bytes per pixel and staged row pitches of a mode.  kElem: bytes per element of the source's TMA view (box starts are
-// given to the TMA unit in elements).
+// Bytes per pixel, staged row pitches and out-tile re-pack of a mode.  kElem: bytes per element of the source's TMA view
+// (box starts are given to the TMA unit in elements).
+// A warp step samples one pixel (Px) per lane of a 32-pixel output row.  repack turns it into the lane's kOutWords words
+// of the dense out tile with ONE shuffle (selector out_sel(lane)); sample_repack does that for a lane's N pixels of a
+// frame, in the order that measured fastest for the depth; store writes the words the lane owns for N pixels `step`
+// bytes apart, from byte out_offset(lane) of the row on (`writer` = writer(lane)).
 struct Bpp3 {  // uint8 x 3 channels
     static constexpr int kBpp = 3, kElem = 1;
-    static constexpr int kPitchMin = tiled::kPitchMin, kPitchMax = tiled::kPitchMax, kPitchStep = tiled::kPitchStep;
+    static constexpr int kPitchMin = 96, kPitchMax = 256, kPitchStep = 16;
+    // [c0 c1 c2 .]: every lane fetches the pixel of lane + 1; lanes 4 m + i, i < 3, then hold word 3 m + i of the row
+    // segment (12 bytes of 4 pixels = 3 words): [c0 c1 c2 c0'], [c1 c2 c0' c1'], [c2 c0' c1' c2'].  Lanes 4 m + 3 store nothing.
+    using Px = uint32_t;
+    static constexpr int kOutWords = 1;
+    __device__ static __forceinline__ uint32_t out_sel(int lane) {
+        const int sub = lane & 3;
+        return sub == 0 ? 0x4210u : (sub == 1 ? 0x5421u : 0x6542u);
+    }
+    __device__ static __forceinline__ int out_offset(int lane) { return (3 * (lane >> 2) + (lane & 3)) * 4; }
+    __device__ static __forceinline__ bool writer(int lane) { return (lane & 3) != 3; }
+    __device__ static __forceinline__ void repack(Px r, uint32_t sel, uint32_t (&w)[kOutWords]) {
+        w[0] = __byte_perm(r, __shfl_down_sync(0xffffffffu, r, 1), sel);
+    }
+    // N pixels `sample(k)`: all sampled first, then re-packed
+    template <int N, class Sample>
+    __device__ static __forceinline__ void sample_repack(Sample sample, uint32_t sel, uint32_t (&w)[N][kOutWords]) {
+        Px r[N];
+#pragma unroll
+        for (int k = 0; k < N; ++k) r[k] = sample(k);
+#pragma unroll
+        for (int k = 0; k < N; ++k) repack(r[k], sel, w[k]);
+    }
+    template <int N>
+    __device__ static __forceinline__ void store(uint32_t addr, uint32_t step, const uint32_t (&w)[N][kOutWords], bool writer) {
+        if (writer) {
+#pragma unroll
+            for (int k = 0; k < N; ++k) sts32(addr + k * step, w[k][0]);
+        }
+    }
 };
+constexpr int kWidths = (Bpp3::kPitchMax - Bpp3::kPitchMin) / Bpp3::kPitchStep + 1;  // 11 box widths
 struct Bpp6 {  // uint16 x 3 channels: a 32-pixel tile row's footprint is twice as wide, so are the boxes (192 .. 512 B)
     static constexpr int kBpp = 6, kElem = 2;
     static constexpr int kPitchMin = 192, kPitchMax = 512, kPitchStep = 32;
+    // .x = [c0 c1], .y = [c2 .]: lanes 2 m and 2 m + 1 hold the 12 bytes = words 3 m .. 3 m + 2 of the row segment; lane
+    // 2 m + 1 sends its [c0' c1'] to lane 2 m, which stores [c0 c1] and [c2 c0'], and lane 2 m + 1 stores [c1' c2'].
+    using Px = uint2;
+    static constexpr int kOutWords = 2;
+    __device__ static __forceinline__ uint32_t out_sel(int lane) { return (lane & 1) ? 0x5432u : 0x3210u; }
+    __device__ static __forceinline__ int out_offset(int lane) { return 12 * (lane >> 1) + ((lane & 1) ? 8 : 0); }
+    __device__ static __forceinline__ bool writer(int lane) { return (lane & 1) == 0; }
+    __device__ static __forceinline__ void repack(Px r, uint32_t sel, uint32_t (&w)[kOutWords]) {
+        const uint32_t next = __shfl_down_sync(0xffffffffu, r.x, 1);
+        w[0] = __byte_perm(r.x, r.y, sel);
+        w[1] = __byte_perm(r.y, next, 0x5410);
+    }
+    // N pixels `sample(k)`: each re-packed as soon as it is sampled (all sampled first measured up to 1 % slower on
+    // scripts/bench_u16.py, B200)
+    template <int N, class Sample>
+    __device__ static __forceinline__ void sample_repack(Sample sample, uint32_t sel, uint32_t (&w)[N][kOutWords]) {
+#pragma unroll
+        for (int k = 0; k < N; ++k) repack(sample(k), sel, w[k]);
+    }
+    template <int N>
+    __device__ static __forceinline__ void store(uint32_t addr, uint32_t step, const uint32_t (&w)[N][kOutWords], bool writer) {
+#pragma unroll
+        for (int k = 0; k < N; ++k) {
+            sts32(addr + k * step, w[k][0]);
+            if (writer) sts32(addr + k * step + 4, w[k][1]);
+        }
+    }
 };
 static_assert((Bpp6::kPitchMax - Bpp6::kPitchMin) / Bpp6::kPitchStep + 1 == kWidths, "TmaMaps holds kWidths box widths");
+
+// TMA descriptors of one launch (kernel parameter; the TMA unit reads them from the parameter bank).
+struct alignas(64) TmaMaps {
+    // [view][box bytes M::kPitchMin + M::kPitchStep w][box rows kRowsMin + 4 r]: uint8 (cols * 3, rows, frames), or for
+    // the 16-bit modes uint16 (cols * 3, rows, frames) -- a box is at most 256 elements wide, i.e. 512 bytes at 16 bits
+    CUtensorMap src[2][kWidths][kRowSizes];
+    CUtensorMap dst;  // uint8 (dst_pitch, H, frames), box (32 M::kBpp bytes, tile height, 1)
+};
+
 // A mode fixes: pixels per thread (the per-pixel constants must stay in registers across the frames of the batch),
 // the tile height, the tap footprint (taps start kLo pixels / rows before the integer coordinate and end kHi after
 // it), the per-pixel constants and the sampling of one pixel from the staged rectangle.
@@ -229,7 +289,6 @@ struct LinearP : Bpp3 {
     static constexpr int kShift = kInterBits;  // coordinates are 1/32-pixel fixed point: sx = cvRound(x * 32)
     __device__ static __forceinline__ int quant(float m) { return quantise(m); }
     static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 4;
-    static constexpr bool kRowPatch = true;  // a warp step = 32 pixels of one output row (pixel k of a thread: row 4 band + k)
     struct Pixel {  // constant over the frames of the batch
         uint32_t osel;     // window byte offset (4-aligned) << 16 | selA
         uint32_t selT;
@@ -283,7 +342,6 @@ struct Nearest : Bpp3 {
     static constexpr int kShift = 0;
     __device__ static __forceinline__ int quant(float m) { return cv_round(m); }
     static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 4;
-    static constexpr bool kRowPatch = true;
     struct Pixel {
         int boff;  // byte offset (4-aligned) of the 8-byte window that holds the pixel
         int sh;    // 8 * (byte offset & 3)
@@ -307,7 +365,6 @@ struct Cubic : Bpp3 {
     // a thread owns only 2 pixels (their 16 table weights take 16 registers), so an item is FOUR frames: the
     // per-item bookkeeping is paid once per 8 pixels of a thread, as for the bilinear mode
     static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 8;
-    static constexpr bool kRowPatch = true;  // a warp step = 32 pixels of one output row (pixel k of a thread: row 2 warp + k)
     struct Pixel {
         int boff;       // byte offset (4-aligned) of the 16-byte window of tap row 0 (iy - 1), first tap ix - 1
         int sh;
@@ -355,7 +412,6 @@ struct Cubic : Bpp3 {
 // and ~120 shared-memory wavefronts per pixel step.
 struct Lanczos4 : Bpp3 {
     static constexpr int kPx = 1, kTileH = 8, kLo = 3, kHi = 4, kRowsMin = 16, kInterp = VR180_INTER_LANCZOS4;
-    static constexpr bool kRowPatch = true;  // a warp = one output row of the tile
     static constexpr int kShift = kInterBits;  // coordinates are 1/32-pixel fixed point: sx = cvRound(x * 32)
     __device__ static __forceinline__ int quant(float m) { return quantise(m); }
     static constexpr int kStageArea = 16384, kWeightSmem = kSamplers * 128;  // 16 KB of stages + 32 KB of weights
@@ -457,7 +513,6 @@ struct Linear16 : Bpp6 {
     static constexpr int kShift = kInterBits;
     __device__ static __forceinline__ int quant(float m) { return quantise(m); }
     static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 2;
-    static constexpr bool kRowPatch = true;
     struct Pixel {
         uint32_t osel;  // window byte offset (4-aligned) << 16 | alignment selector
         float w[4];     // w00 w01 w10 w11
@@ -517,7 +572,6 @@ struct Nearest16 : Bpp6 {
     static constexpr int kShift = 0;
     __device__ static __forceinline__ int quant(float m) { return cv_round(m); }
     static constexpr int kStageArea = kStageAreaDefault, kWeightSmem = 0, kOutTiles = 2;
-    static constexpr bool kRowPatch = true;
     struct Pixel {
         uint32_t osel;
     };
@@ -609,13 +663,22 @@ __device__ __forceinline__ TileRect tile_rect(int mnx, int mxx, int mny, int mxy
     r.box_rows = M::kRowsMin + r.rsel * kRowsStep;
     return r;
 }
+// Sampling constants of a pixel with quantised coordinates (qx, qy) in a stage whose rectangle starts at source byte
+// column bx0, row ry0: the offset of its first tap (valid: the pixel is sampled) and, if `with_weights`, its weights
+template <class M>
+__device__ __forceinline__ void stage_pixel(typename M::Pixel& p, int qx, int qy, int bx0, int ry0, int pitch, bool valid,
+                                            bool with_weights, const short* tab) {
+    const int off = ((qy >> M::kShift) - M::kLo - ry0) * pitch + M::kBpp * ((qx >> M::kShift) - M::kLo) - bx0;
+    M::set_offset(p, off, valid);
+    if (with_weights) M::weights(p, qx & 31, qy & 31, tab);
+}
 
 // Row pitch of the staged rectangle (= TMA box width).  Candidates: the kPitchCands widths pitch0 + kPitchStep e.
 // Cost of a candidate in shared-memory wavefronts per (frame, eye) item: the tap loads (every sampling warp measures
 // the wavefronts = max distinct words per bank, counted with match.any, of the first tap load of its step k = 0; a
 // tile has kStepsPerWarp steps of kLoads loads with the same address pattern) + the TMA write of the box (64 bytes per
 // wavefront, measured).  pitch_costs: one sampling warp's share, added into s_cost[kPitchCands] (zeroed by the
-// caller); pick_pitch, after a barrier: the cheapest candidate that is <= kPitchMax and that `fits` admits.
+// caller); pick_pitch, after a barrier: the cheapest candidate that is <= M::kPitchMax and that `fits` admits.
 template <class M>
 __device__ __forceinline__ void pitch_costs(int sx0, int sy0, const TileRect& rc, int pitch0, int lane, int* s_cost) {
     const int row = (sy0 >> M::kShift) - M::kLo - rc.ry0, col = M::kBpp * ((sx0 >> M::kShift) - M::kLo) - rc.bx0;
@@ -636,16 +699,16 @@ __device__ __forceinline__ void pitch_costs(int sx0, int sy0, const TileRect& rc
                          : M::kInterp == VR180_INTER_CUBIC ? 16 : 56;
     if (lane < kPitchCands) atomicAdd(&s_cost[lane], cost * (kStepsPerWarp * kLoads));
 }
-template <int Step = kPitchStep, int Max = kPitchMax, class Fits>  // (a mode's M::kPitchStep, M::kPitchMax)
+template <class M, class Fits>
 __device__ __forceinline__ int pick_pitch(const int* s_cost, int pitch0, int box_rows, Fits fits) {
     int best = 0, best_cost = INT_MAX;
 #pragma unroll
     for (int e = 0; e < kPitchCands; ++e) {
-        const int pe = pitch0 + Step * e;
+        const int pe = pitch0 + M::kPitchStep * e;
         const int c = s_cost[e] + box_rows * pe / 64;
-        if (pe <= Max && fits(pe) && c < best_cost) { best_cost = c; best = e; }
+        if (pe <= M::kPitchMax && fits(pe) && c < best_cost) { best_cost = c; best = e; }
     }
-    return pitch0 + Step * best;
+    return pitch0 + M::kPitchStep * best;
 }
 // the tightest admissible pitch of a rectangle `wbytes` wide (a multiple of 16): >= M::kPitchMin, a multiple of M::kPitchStep
 template <class M>
@@ -687,18 +750,6 @@ __device__ __forceinline__ void gather_pixel(const RemapArgs& a, int f, int i, i
         o[0] = (uint8_t)px[0];
         o[1] = (uint8_t)px[1];
         o[2] = (uint8_t)px[2];
-    }
-}
-
-// the FR frames of an item for one pixel; only modes with per-row state worth sharing implement sample_frames
-template <class M, int FR>
-__device__ __forceinline__ void sample_item(uint32_t sbuf, uint32_t frame_bytes, const typename M::Pixel& p, uint32_t pitch,
-                                            uint32_t (&out)[FR]) {
-    if constexpr (M::kInterp == VR180_INTER_LANCZOS4) {
-        M::template sample_frames<FR>(sbuf, frame_bytes, p, pitch, out);
-    } else {
-#pragma unroll
-        for (int f = 0; f < FR; ++f) out[f] = M::sample(sbuf + f * frame_bytes, p, pitch);
     }
 }
 
