@@ -309,11 +309,13 @@ k_warp_stream(const __grid_constant__ RemapArgs a, const __grid_constant__ Strea
   }
 }
 
+// Eligibility is decided by the caller (launch_remap_tiled: 3 channels, aligned buffers, every map group with a packed LUT
+// of this interpolation, no per-frame radius, an 8-bit mode).
 template <class M>
-static int launch_stream_mode(const RemapArgs& a, const short* tab, cudaStream_t st) {
+int launch_stream_mode(const RemapArgs& a, const short* tab, const Remap16& x16, cudaStream_t st) {
     const int n_groups = a.share_map ? 1 : a.n_views;
     if (a.n_frames > 0x7fff) return VR180_ERR_UNSUPPORTED;  // an item's two frame indices travel in one int
-    const TmaMaps* tm = tma_maps_for(a, M::kInterp, M::kRowsMin, M::kTileH, 1);
+    const TmaMaps* tm = tma_maps_for<M>(a, 1);
     if (!tm) return VR180_ERR_UNSUPPORTED;
     int dev = 0;
     const int rc = max_dyn_smem_once<k_warp_stream<M>>(SLay<M>::kSmemBytes, dev);
@@ -331,7 +333,7 @@ static int launch_stream_mode(const RemapArgs& a, const short* tab, cudaStream_t
     if (tiles * n_groups > 0x7fffffffLL) return VR180_ERR_UNSUPPORTED;
     sp.n_tiles = (int)tiles;
     sp.n_units = (int)(tiles * n_groups);
-    sp.zero_border = zero_border(a);
+    sp.zero_border = zero_border(a, x16);
     sp.tab = tab;
     const int forced = g_debug_stream_grid.load(std::memory_order_relaxed);  // vr180_debug_set(3, n): tests
     int grid = forced > 0 ? forced : sms * kStreamCtas;
@@ -341,19 +343,11 @@ static int launch_stream_mode(const RemapArgs& a, const short* tab, cudaStream_t
     VR180_CUDA(cudaGetLastError());
     return VR180_OK;
 }
+// the 8-bit modes, for launch_remap_tiled (tiled.cu)
+template int launch_stream_mode<Nearest>(const RemapArgs&, const short*, const Remap16&, cudaStream_t);
+template int launch_stream_mode<LinearP>(const RemapArgs&, const short*, const Remap16&, cudaStream_t);
+template int launch_stream_mode<Cubic>(const RemapArgs&, const short*, const Remap16&, cudaStream_t);
+template int launch_stream_mode<Lanczos4>(const RemapArgs&, const short*, const Remap16&, cudaStream_t);
 
 }  // namespace tiled
-
-// Eligibility is decided by the caller (launch_remap_tiled: 3 channels, aligned buffers, every map group with a packed LUT
-// of this interpolation, no per-frame radius).
-int launch_remap_stream(const RemapArgs& a, int interp, const short* weight_tab, cudaStream_t st) {
-    using namespace tiled;
-    if (a.depth != VR180_DEPTH_8U) return VR180_ERR_UNSUPPORTED;  // tile headers hold 8-bit box geometry
-    if (interp == VR180_INTER_NEAREST) return launch_stream_mode<Nearest>(a, nullptr, st);
-    if (interp == VR180_INTER_LINEAR) return launch_stream_mode<LinearP>(a, nullptr, st);
-    if (interp == VR180_INTER_CUBIC) return launch_stream_mode<Cubic>(a, weight_tab, st);
-    if (interp == VR180_INTER_LANCZOS4) return launch_stream_mode<Lanczos4>(a, weight_tab, st);
-    return VR180_ERR_UNSUPPORTED;
-}
-
 }  // namespace vr180

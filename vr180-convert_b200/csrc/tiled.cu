@@ -681,40 +681,51 @@ __global__ void __launch_bounds__(kSamplers) k_pack_tiles(const float* __restric
 
 }  // namespace tiled
 
-static int tile_height_of(int interp) {  // (the 16-bit modes: as LinearP / Nearest)
-    return interp == VR180_INTER_LINEAR || interp == VR180_INTER_NEAREST ? tiled::LinearP::kTileH
-           : interp == VR180_INTER_CUBIC                                  ? tiled::Cubic::kTileH
-           : interp == VR180_INTER_LANCZOS4                               ? tiled::Lanczos4::kTileH
-                                                                          : 0;
+// The tiled mode of an interpolation at depth D: returns f(M{}) for its mode struct M, or VR180_ERR_UNSUPPORTED where
+// there is none (16-bit CUBIC / LANCZOS4).  f is instantiated for the modes of depth D only.
+template <int D, class F>
+static int with_mode(int interp, F&& f) {
+    using namespace tiled;
+    if constexpr (D == VR180_DEPTH_16U) {
+        if (interp == VR180_INTER_NEAREST) return f(Nearest16{});
+        if (interp == VR180_INTER_LINEAR) return f(Linear16{});
+    } else {
+        if (interp == VR180_INTER_NEAREST) return f(Nearest{});
+        if (interp == VR180_INTER_LINEAR) return f(LinearP{});
+        if (interp == VR180_INTER_CUBIC) return f(Cubic{});
+        if (interp == VR180_INTER_LANCZOS4) return f(Lanczos4{});
+    }
+    return VR180_ERR_UNSUPPORTED;
 }
 
+// A tile-packed LUT belongs to an interpolation, not to a depth: Linear16 / Nearest16 keep the 8-bit modes' tile shape and
+// thread order and read their packed entries as they are.  So the packed paths select the 8-bit mode.
 size_t packed_lut_bytes(int out_w, int out_h, int interp) {
-    const int th = tile_height_of(interp);
-    if (!th) return 0;
-    const long long n_tiles = (long long)((out_w + tiled::kTileW - 1) / tiled::kTileW) * ((out_h + th - 1) / th);
-    return tiled::packed_entries_offset(n_tiles) + (size_t)n_tiles * tiled::kTileW * th * 4;
+    using namespace tiled;
+    size_t bytes = 0;
+    with_mode<VR180_DEPTH_8U>(interp, [&](auto m) -> int {
+        using M = decltype(m);
+        const long long n_tiles = (long long)((out_w + kTileW - 1) / kTileW) * ((out_h + M::kTileH - 1) / M::kTileH);
+        bytes = packed_entries_offset(n_tiles) + (size_t)n_tiles * kTileW * M::kTileH * 4;
+        return VR180_OK;
+    });
+    return bytes;
 }
 
 int launch_pack_lut_tiles(const float* xmap, const float* ymap, int64_t map_pitch, int W, int H, int interp, void* packed,
                           cudaStream_t st) {
     using namespace tiled;
-    const int th = tile_height_of(interp);
-    if (!th) return VR180_ERR_UNSUPPORTED;
-    const int tiles_x = (W + kTileW - 1) / kTileW, tiles_y = (H + th - 1) / th;
-    const long long n_tiles = (long long)tiles_x * tiles_y;
-    if (n_tiles > 0x7fffffffLL) return VR180_ERR_UNSUPPORTED;
-    const dim3 grid((unsigned)n_tiles);
-    if (interp == VR180_INTER_NEAREST)
-        k_pack_tiles<Nearest><<<grid, kSamplers, 0, st>>>(xmap, ymap, (long long)map_pitch, W, H, tiles_x, (int)n_tiles, packed);
-    else if (interp == VR180_INTER_LINEAR)
-        k_pack_tiles<LinearP><<<grid, kSamplers, 0, st>>>(xmap, ymap, (long long)map_pitch, W, H, tiles_x, (int)n_tiles, packed);
-    else if (interp == VR180_INTER_CUBIC)
-        k_pack_tiles<Cubic><<<grid, kSamplers, 0, st>>>(xmap, ymap, (long long)map_pitch, W, H, tiles_x, (int)n_tiles, packed);
-    else
-        k_pack_tiles<Lanczos4><<<grid, kSamplers, 0, st>>>(xmap, ymap, (long long)map_pitch, W, H, tiles_x, (int)n_tiles, packed);
-    g_launches.fetch_add(1, std::memory_order_relaxed);
-    VR180_CUDA(cudaGetLastError());
-    return VR180_OK;
+    return with_mode<VR180_DEPTH_8U>(interp, [&](auto m) -> int {
+        using M = decltype(m);
+        const int tiles_x = (W + kTileW - 1) / kTileW, tiles_y = (H + M::kTileH - 1) / M::kTileH;
+        const long long n_tiles = (long long)tiles_x * tiles_y;
+        if (n_tiles > 0x7fffffffLL) return VR180_ERR_UNSUPPORTED;
+        k_pack_tiles<M><<<(unsigned)n_tiles, kSamplers, 0, st>>>(xmap, ymap, (long long)map_pitch, W, H, tiles_x,
+                                                                 (int)n_tiles, packed);
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        VR180_CUDA(cudaGetLastError());
+        return VR180_OK;
+    });
 }
 
 // Host: recognise the standard chain shape (see StdChain).
@@ -799,7 +810,7 @@ int tiled_debug_flags() {  // vr180_debug_set(1, flags), else $VR180_TILED_DEBUG
 
 constexpr int kMaxFramesPerCta = 64;
 // frames per CTA: the coordinates are evaluated once per CTA, so keep the chunk as large as the grid allows
-static int frames_per_cta(long long tiles, int n_frames, int views_per_cta = 1) {
+static int frames_per_cta(long long tiles, int n_frames, int views_per_cta) {
     const int forced = g_debug_frames_per_cta.load(std::memory_order_relaxed);  // vr180_debug_set(0, n): tests
     if (forced > 0) return forced < n_frames ? forced : n_frames;
     // A CTA streams through its frames one after the other and the CTAs of neighbouring tiles -- which share the halo
@@ -815,22 +826,30 @@ static int frames_per_cta(long long tiles, int n_frames, int views_per_cta = 1) 
     return fpc;
 }
 
-// TMA descriptors of a launch.  They depend only on the buffers' geometry: video loops call with the same buffers again
-// and again, so the last few sets are kept per host thread (a ring of batches cycles through a handful of buffers, and
-// 199 cuTensorMapEncodeTiled calls cost about as much host time as a single-pair launch takes on the GPU).
-// `fr`: frames per box (depth of the load and store boxes); `bpp`: the mode's bytes per pixel -- part of the key, since
-// one allocation can be warped as uint8 and as uint16 with equal pointers, sizes and pitches.  nullptr = a descriptor could
-// not be encoded.
-const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int interp, int rows_min, int tile_h, int fr, int bpp) {
+// TMA descriptors of a launch of mode M with `fr` frames per box (depth of the load and store boxes); nullptr = a
+// descriptor could not be encoded.  They depend only on the buffers' geometry: video loops call with the same buffers
+// again and again, so the last few sets are kept per host thread (a ring of batches cycles through a handful of buffers,
+// and 199 cuTensorMapEncodeTiled calls cost about as much host time as a single-pair launch takes on the GPU).  One cache
+// serves every mode: the key holds the mode's interpolation and bytes per pixel, since Nearest and Nearest16 share their
+// interpolation and one allocation can be warped as uint8 and as uint16 with equal pointers, sizes and pitches.
+struct TmaKey {
+    const void* src[2];
+    long long pitch[2], fs[2];
+    int rows, cols, n_views, n_frames, H, mode, fr, bpp;
+    const void* dst;
+    long long dst_pitch, dst_fs;
+};
+struct TmaEntry {
+    TmaKey key;
+    tiled::TmaMaps tm;
+    uint64_t stamp;
+};
+static thread_local std::vector<TmaEntry> t_tma_cache;
+static thread_local uint64_t t_tma_clock = 0;
+template <class M>
+const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int fr) {
     using namespace tiled;
-    struct Key {
-        const void* src[2];
-        long long pitch[2], fs[2];
-        int rows, cols, n_views, n_frames, H, mode, fr, bpp;
-        const void* dst;
-        long long dst_pitch, dst_fs;
-    };
-    Key key;
+    TmaKey key;
     memset(&key, 0, sizeof(key));
     for (int v = 0; v < a0.n_views; ++v) {
         key.src[v] = a0.view[v].src;
@@ -842,61 +861,57 @@ const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int interp, int rows_min
     key.n_views = a0.n_views;
     key.n_frames = a0.n_frames;
     key.H = a0.H;
-    key.mode = interp;
+    key.mode = M::kInterp;
     key.fr = fr;
-    key.bpp = bpp;
+    key.bpp = M::kBpp;
     key.dst = a0.dst;
     key.dst_pitch = a0.dst_pitch;
     key.dst_fs = a0.dst_frame_stride;
-    struct Entry {
-        Key key;
-        TmaMaps tm;
-        uint64_t stamp;
-    };
     constexpr size_t kCacheEntries = 8;
-    static thread_local std::vector<Entry> cache;
-    static thread_local uint64_t clock_ = 0;
-    Entry* hit = nullptr;
-    for (Entry& e : cache)
+    TmaEntry* hit = nullptr;
+    for (TmaEntry& e : t_tma_cache)
         if (memcmp(&key, &e.key, sizeof(key)) == 0) hit = &e;
     if (!hit) {
-        if (cache.size() < kCacheEntries) {
-            cache.emplace_back();
-            hit = &cache.back();
+        if (t_tma_cache.size() < kCacheEntries) {
+            t_tma_cache.emplace_back();
+            hit = &t_tma_cache.back();
         } else {
-            hit = &cache[0];
-            for (Entry& e : cache)
+            hit = &t_tma_cache[0];
+            for (TmaEntry& e : t_tma_cache)
                 if (e.stamp < hit->stamp) hit = &e;
         }
         memset(&hit->key, 0xff, sizeof(hit->key));  // invalid until every descriptor is encoded
         TmaMaps& t = hit->tm;
         memset(&t, 0, sizeof(t));
-        const int elem = bpp / 3;  // uint16 views for the 16-bit modes
-        const int pitch_min = elem == 2 ? Bpp6::kPitchMin : Bpp3::kPitchMin, pitch_step = elem == 2 ? Bpp6::kPitchStep : Bpp3::kPitchStep;
         for (int v = 0; v < a0.n_views; ++v) {
             const ViewArgs& vw = a0.view[v];
             for (int w = 0; w < kWidths; ++w)
                 for (int r = 0; r < kRowSizes; ++r)
-                    if (!encode_3d(&t.src[v][w][r], elem, vw.src, (long long)vw.cols * bpp, vw.rows, a0.n_frames, vw.pitch,
-                                   vw.frame_stride, pitch_min + w * pitch_step, rows_min + r * kRowsStep, fr))
+                    if (!encode_3d(&t.src[v][w][r], M::kElem, vw.src, (long long)vw.cols * M::kBpp, vw.rows, a0.n_frames,
+                                   vw.pitch, vw.frame_stride, M::kPitchMin + w * M::kPitchStep, M::kRowsMin + r * kRowsStep, fr))
                         return nullptr;
         }
         if (a0.n_views == 1) memcpy(&t.src[1], &t.src[0], sizeof(t.src[0]));
-        if (!encode_3d(&t.dst, 1, a0.dst, a0.dst_pitch, a0.H, a0.n_frames, a0.dst_pitch, a0.dst_frame_stride, kTileW * bpp,
-                       tile_h, fr))
+        if (!encode_3d(&t.dst, 1, a0.dst, a0.dst_pitch, a0.H, a0.n_frames, a0.dst_pitch, a0.dst_frame_stride,
+                       kTileW * M::kBpp, M::kTileH, fr))
             return nullptr;
         hit->key = key;
     }
-    hit->stamp = ++clock_;
+    hit->stamp = ++t_tma_clock;
     return &hit->tm;
 }
+// the 8-bit modes, for the tile-streaming kernel (stream.cu)
+template const tiled::TmaMaps* tma_maps_for<tiled::Nearest>(const RemapArgs&, int);
+template const tiled::TmaMaps* tma_maps_for<tiled::LinearP>(const RemapArgs&, int);
+template const tiled::TmaMaps* tma_maps_for<tiled::Cubic>(const RemapArgs&, int);
+template const tiled::TmaMaps* tma_maps_for<tiled::Lanczos4>(const RemapArgs&, int);
 
 template <class M, bool DYN, int FR>
 static int launch_mode(const RemapArgs& a0, const vr180_chain_t& c0, const vr180_chain_t& c1, const short* tab,
-                       const Remap16& x16, cudaStream_t st) {
+                       const Remap16& x16, int fpc, cudaStream_t st) {
     using namespace tiled;
     const int n_groups = a0.share_map ? 1 : a0.n_views;
-    const TmaMaps* tmp = tma_maps_for(a0, M::kInterp, M::kRowsMin, M::kTileH, DYN ? 1 : FR, M::kBpp);
+    const TmaMaps* tmp = tma_maps_for<M>(a0, DYN ? 1 : FR);
     if (!tmp) return VR180_ERR_UNSUPPORTED;
     const TmaMaps& tm = *tmp;
 
@@ -913,8 +928,6 @@ static int launch_mode(const RemapArgs& a0, const vr180_chain_t& c0, const vr180
     tp.tab = tab;
     tp.zero_border = zero_border(a, x16);
     tp.debug = tiled_debug_flags();
-    const long long tiles = (long long)tiles_x * tiles_y * n_groups;
-    int fpc = frames_per_cta(tiles, a.n_frames, a.share_map ? a.n_views : 1);
     fpc = (fpc + FR - 1) / FR * FR;  // chunks start at multiples of FR: phantom frames can only lie past the batch
     a.frames_per_cta = fpc;
     const int chunks = (a.n_frames + fpc - 1) / fpc;
@@ -943,30 +956,25 @@ template <class M>
 static int launch_tiled(const RemapArgs& a0, const vr180_chain_t& c0, const vr180_chain_t& c1, const short* tab,
                         const Remap16& x16, bool dyn, int fpc, cudaStream_t st) {
     if constexpr (M::kInterp == VR180_INTER_CUBIC) {
-        if (fpc >= 8) return dyn ? launch_mode<M, true, 4>(a0, c0, c1, tab, x16, st) : launch_mode<M, false, 4>(a0, c0, c1, tab, x16, st);
+        if (fpc >= 8)
+            return dyn ? launch_mode<M, true, 4>(a0, c0, c1, tab, x16, fpc, st) : launch_mode<M, false, 4>(a0, c0, c1, tab, x16, fpc, st);
     }
     if constexpr (M::kBpp == 3) {
-        if (fpc >= 2) return dyn ? launch_mode<M, true, 2>(a0, c0, c1, tab, x16, st) : launch_mode<M, false, 2>(a0, c0, c1, tab, x16, st);
+        if (fpc >= 2)
+            return dyn ? launch_mode<M, true, 2>(a0, c0, c1, tab, x16, fpc, st) : launch_mode<M, false, 2>(a0, c0, c1, tab, x16, fpc, st);
     }
-    return dyn ? launch_mode<M, true, 1>(a0, c0, c1, tab, x16, st) : launch_mode<M, false, 1>(a0, c0, c1, tab, x16, st);
+    return dyn ? launch_mode<M, true, 1>(a0, c0, c1, tab, x16, fpc, st) : launch_mode<M, false, 1>(a0, c0, c1, tab, x16, fpc, st);
 }
 
-// Host-side eligibility + launch.  Returns VR180_ERR_UNSUPPORTED when the request is outside the fast path (the
-// caller then launches the generic k_remap); any other value is final.  `weight_tab`: device copy of the weight table of
-// the requested interpolation (1024 x 16 bicubic, 1024 x 64 Lanczos4; unused otherwise).  uint16: NEAREST and LINEAR
-// only (`x16.cval`: the border colour); CUBIC / LANCZOS4 keep the generic kernel.
+// Host-side eligibility + launch of a request that launch_remap (kernels.cu) has validated.  Returns
+// VR180_ERR_UNSUPPORTED when the request is outside the fast path (the caller then launches the generic k_remap); any
+// other value is final.  16-bit CUBIC / LANCZOS4 have no tiled mode (with_mode) and keep the generic kernel.
+// `weight_tab`: device copy of the weight table of the requested interpolation (1024 x 16 bicubic, 1024 x 64 Lanczos4;
+// unused otherwise); `x16.cval`: the border colour of a 16-bit request.
 int launch_remap_tiled(const RemapArgs& a0, int channels, int interp, const vr180_chain_t& c0, const vr180_chain_t& c1,
                        const short* weight_tab, const Remap16& x16, cudaStream_t st) {
-    if (channels != 3 || (a0.depth != VR180_DEPTH_8U && a0.depth != VR180_DEPTH_16U)) return VR180_ERR_UNSUPPORTED;
-    if (interp != VR180_INTER_NEAREST && interp != VR180_INTER_LINEAR && interp != VR180_INTER_CUBIC &&
-        interp != VR180_INTER_LANCZOS4)
-        return VR180_ERR_UNSUPPORTED;
-    const bool u16 = a0.depth == VR180_DEPTH_16U;
-    if (u16 && interp != VR180_INTER_NEAREST && interp != VR180_INTER_LINEAR) return VR180_ERR_UNSUPPORTED;
-    const long long bpp = u16 ? 6 : 3;
-    if (interp == VR180_INTER_NEAREST)  // the fixed-point LUT is a 1/32-pixel grid; NEAREST rounds the float coordinate itself
-        for (int v = 0; v < a0.n_views; ++v)
-            if (a0.view[v].map_kind == VR180_MAPSRC_FIXED) return VR180_ERR_UNSUPPORTED;
+    if (channels != 3) return VR180_ERR_UNSUPPORTED;
+    const long long bpp = 3 * depth_bytes(a0.depth);
     const int n_groups = a0.share_map ? 1 : a0.n_views;
     for (int v = 0; v < a0.n_views; ++v) {
         const ViewArgs& vw = a0.view[v];
@@ -994,32 +1002,27 @@ int launch_remap_tiled(const RemapArgs& a0, int channels, int interp, const vr18
     // 78.5 / 116 / 155 / 196 us; 8K pairs with per-eye maps 1 / 2 / 4 / 8 / 12 / 16 / 24 pairs 110 / 151 / 240 / 431 / 618 / 806 /
     // 1206 us vs 217 / 245 / 310 / 548 / 690 / 827 / 1125 us.  VR180_TILED_DEBUG bit 1: whenever eligible; bit 2: never.
     const int kStreamMaxItems = a0.share_map ? 20 : 16;  // (frame, eye) rectangles per tile
-    {
-        bool all_packed = !dyn && !u16;  // (the streaming kernel's tile headers hold 8-bit box geometry)
-        for (int g = 0; g < n_groups; ++g) all_packed = all_packed && a0.view[g].packed != nullptr;
-        const int dbg = tiled_debug_flags();
-        const int items = a0.n_frames * (a0.share_map ? a0.n_views : 1);
-        const bool tab_ok = (interp != VR180_INTER_CUBIC && interp != VR180_INTER_LANCZOS4) || weight_tab != nullptr;
-        if (all_packed && tab_ok && !(dbg & 4) && ((dbg & 2) || items <= kStreamMaxItems) &&
-            g_debug_frames_per_cta.load(std::memory_order_relaxed) <= 0) {
-            const int rc = launch_remap_stream(a0, interp, weight_tab, st);
+    bool all_packed = !dyn;
+    for (int g = 0; g < n_groups; ++g) all_packed = all_packed && a0.view[g].packed != nullptr;
+    const int dbg = tiled_debug_flags();
+    const int items = a0.n_frames * (a0.share_map ? a0.n_views : 1);
+    const bool stream = all_packed && !(dbg & 4) && ((dbg & 2) || items <= kStreamMaxItems) &&
+                        g_debug_frames_per_cta.load(std::memory_order_relaxed) <= 0;
+    auto launch = [&](auto m) -> int {
+        using M = decltype(m);
+        if constexpr (M::kBpp == 3) {  // the streaming kernel's tile headers hold 8-bit box geometry
+            const int rc = stream ? tiled::launch_stream_mode<M>(a0, weight_tab, x16, st) : VR180_ERR_UNSUPPORTED;
             if (rc != VR180_ERR_UNSUPPORTED) return rc;
         }
-    }
-    // two frames per pipeline item when the frames share their rectangles (per-frame radii: the chunks whose frames all
-    // share one radius, a static rig) and every CTA gets at least two of them
-    const int tile_h = tile_height_of(interp);
-    const long long tiles = (long long)((a0.W + tiled::kTileW - 1) / tiled::kTileW) * ((a0.H + tile_h - 1) / tile_h) * n_groups;
-    const int fpc = frames_per_cta(tiles, a0.n_frames, a0.share_map ? a0.n_views : 1);
-    if (u16) {
-        if (interp == VR180_INTER_NEAREST) return launch_tiled<tiled::Nearest16>(a0, c0, c1, nullptr, x16, dyn, fpc, st);
-        return launch_tiled<tiled::Linear16>(a0, c0, c1, nullptr, x16, dyn, fpc, st);
-    }
-    if (interp == VR180_INTER_NEAREST) return launch_tiled<tiled::Nearest>(a0, c0, c1, nullptr, x16, dyn, fpc, st);
-    if (interp == VR180_INTER_LINEAR) return launch_tiled<tiled::LinearP>(a0, c0, c1, nullptr, x16, dyn, fpc, st);
-    if (!weight_tab) return VR180_ERR_UNSUPPORTED;
-    if (interp == VR180_INTER_LANCZOS4) return launch_tiled<tiled::Lanczos4>(a0, c0, c1, weight_tab, x16, dyn, fpc, st);
-    return launch_tiled<tiled::Cubic>(a0, c0, c1, weight_tab, x16, dyn, fpc, st);
+        // two frames per pipeline item when the frames share their rectangles (per-frame radii: the chunks whose frames
+        // all share one radius, a static rig) and every CTA gets at least two of them
+        const long long tiles =
+            (long long)((a0.W + tiled::kTileW - 1) / tiled::kTileW) * ((a0.H + M::kTileH - 1) / M::kTileH) * n_groups;
+        const int fpc = frames_per_cta(tiles, a0.n_frames, a0.share_map ? a0.n_views : 1);
+        return launch_tiled<M>(a0, c0, c1, weight_tab, x16, dyn, fpc, st);
+    };
+    if (a0.depth == VR180_DEPTH_16U) return with_mode<VR180_DEPTH_16U>(interp, launch);
+    return with_mode<VR180_DEPTH_8U>(interp, launch);
 }
 
 }  // namespace vr180

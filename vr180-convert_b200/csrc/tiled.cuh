@@ -756,12 +756,10 @@ __device__ __forceinline__ void gather_pixel(const RemapArgs& a, int f, int i, i
 // ---- host ----------------------------------------------------------------------------------------------------
 // BORDER_CONSTANT with a zero colour: TMA's out-of-bounds zero fill is the border.  16-bit requests: the colour
 // saturated to 16 bits (x16.cval).
-inline int zero_border(const RemapArgs& a) {
-    return (a.border_mode == VR180_BORDER_CONSTANT && !(a.bv[0] | a.bv[1] | a.bv[2])) ? 1 : 0;
-}
 inline int zero_border(const RemapArgs& a, const Remap16& x16) {
-    if (a.depth != VR180_DEPTH_16U) return zero_border(a);
-    return (a.border_mode == VR180_BORDER_CONSTANT && x16.cval[0] == 0.f && x16.cval[1] == 0.f && x16.cval[2] == 0.f) ? 1 : 0;
+    if (a.border_mode != VR180_BORDER_CONSTANT) return 0;
+    if (a.depth == VR180_DEPTH_16U) return x16.cval[0] == 0.f && x16.cval[1] == 0.f && x16.cval[2] == 0.f;
+    return !(a.bv[0] | a.bv[1] | a.bv[2]);
 }
 // The kernel's dynamic shared-memory limit, raised once per device; `dev` = the current device
 template <auto Kernel>
@@ -776,13 +774,15 @@ int max_dyn_smem_once(int bytes, int& dev) {
     return VR180_OK;
 }
 
+// stream.cu: tiles streamed through persistent CTAs (tile-packed LUT, a few frames per launch), for the 8-bit modes;
+// VR180_ERR_UNSUPPORTED = not eligible
+template <class M>
+int launch_stream_mode(const RemapArgs& a, const short* tab, const Remap16& x16, cudaStream_t st);
+
 }  // namespace tiled
 
 // tiled.cu
-// bpp: bytes per pixel of the mode (3: uint8 views, 6: uint16 views with the 16-bit modes' box widths)
-const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int interp, int rows_min, int tile_h, int fr, int bpp = 3);
+template <class M>
+const tiled::TmaMaps* tma_maps_for(const RemapArgs& a0, int fr);
 int tiled_debug_flags();
-// stream.cu: tiles streamed through persistent CTAs (tile-packed LUT, a few frames per launch);
-// VR180_ERR_UNSUPPORTED = not eligible
-int launch_remap_stream(const RemapArgs& a, int interp, const short* weight_tab, cudaStream_t st);
 }  // namespace vr180
